@@ -3,12 +3,17 @@
 bench.py -- manager env-steps/s of the fused B200 manager step, on synthetic physics state.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--config command_direction] [--num-envs 1048576] [--no-sweep]
+                    [--config command_direction] [--num-envs 1048576] [--no-sweep] [--dump-outputs DIR]
 
 One "step" = one full `env.step(actions)` of the drop-in ManagedEnvironment through its public API
 (gfb_action_step -> synthetic scene.step() -> gfb_post_physics -> report read-back -> host reset
 fan-out -> gfb_observe), on a pool of pre-generated synthetic state sets that is larger than L2.
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what each key means.
+Every timed loop (headline, per-kernel pass, e2e, sweep, configs, CPU baseline) runs K steps after W
+warm-up steps.  Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what each key means.
+
+--dump-outputs DIR writes what the last timed step of the headline run returned (rank 0) as
+DIR/<name>.npy, float32 / float64, at most 64 MB in all, plus DIR/outputs.json describing them; the
+inputs are seeded, so two builds run with the same arguments can be compared array for array.
 
   value      whole-job env-steps/s, inputs resident in HBM, device-timed (CUDA events), max over ranks
   roofline   the post-physics kernel: its algorithmic bytes / its CUDA-event time / measured HBM peak
@@ -28,8 +33,10 @@ import subprocess
 import sys
 import time
 
+import numpy as np
 import torch
 
+sys.dont_write_bytecode = True  # the tree may be read-only; nothing is cached in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -50,7 +57,9 @@ def parse_args():
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs 3 / 4 / 5 block")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
-    ap.add_argument("--cpu-envs", type=int, default=0, help="envs for the CPU baseline (0 = same as --num-envs)")
+    ap.add_argument("--cpu-envs", type=int, default=0,
+                    help="envs for the CPU baseline (0 = --num-envs, bounded to a few minutes of host work)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -182,8 +191,11 @@ def make_dropin_env(spec, num_envs, device, pool, seed):
     return env
 
 
-def time_dropin(env, actions, steps, warmup, dist_on):
-    """CUDA-event time of `steps` full env.step() calls; returns ms per step (max over ranks)."""
+def time_dropin(env, actions, steps, warmup, dist_on, keep_outputs=False):
+    """
+    CUDA-event time of `steps` full env.step() calls; returns ms per step (max over ranks).
+    keep_outputs: env.timed_outputs = step_outputs() of the last timed step.
+    """
     import torch.distributed as dist
 
     dev = env._fused.device
@@ -199,12 +211,14 @@ def time_dropin(env, actions, steps, warmup, dist_on):
     wall0 = time.time()
     start.record()
     for i in range(steps):
-        env.step(actions[i % len(actions)])
+        out = env.step(actions[i % len(actions)])
         n_reset += env._fused.report.n_reset
     end.record()
     torch.cuda.synchronize(dev)
     env.timed_window = (wall0, time.time())
     env.timed_launches = env._fused.launch_count() - launches0
+    if keep_outputs:  # before the next step overwrites the buffers
+        env.timed_outputs = step_outputs(out, env.extras_logging_key)
     if dist_on:
         dist.barrier()
     ms = start.elapsed_time(end) / steps
@@ -216,10 +230,52 @@ def time_dropin(env, actions, steps, warmup, dist_on):
     # around every launch -- kept out of the timed region above, where the ~10 extra event records per
     # step would cost host time
     env._fused.profile(True)
-    for i in range(min(steps, 20)):
+    for i in range(steps):
         env.step(actions[i % len(actions)])
     torch.cuda.synchronize(dev)
     return ms, n_reset / max(steps, 1)
+
+
+DUMP_BYTES = 64_000_000
+DUMP_SAMPLE_SEED = 2024
+
+
+def step_outputs(out, logging_key: str) -> dict:
+    """
+    What one env.step() returned, as float32 / float64 numpy arrays: every observation group, rewards,
+    terminated / truncated (0 / 1) and the logged scalars (float64, in the order of `logging_keys`).
+    When the per-env arrays together exceed DUMP_BYTES, all of them are cut to the same fixed, seeded
+    sample of env rows, stored as `env_index` (float64).
+    """
+    _, rewards, terminated, truncated, extras = out
+    per_env = {f"obs_{group}": t for group, t in extras["observations"].items()}
+    per_env.update(rewards=rewards, terminated=terminated, truncated=truncated)
+    n = rewards.shape[0]
+    row_bytes = sum(4 * (t.numel() // n) for t in per_env.values()) + 8  # + env_index
+    keep = min(n, (DUMP_BYTES - 1_000_000) // row_bytes)  # (1 MB left for the logged scalars and file headers)
+    arrays = {}
+    if keep < n:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(DUMP_SAMPLE_SEED))[:keep].sort().values
+        arrays["env_index"] = rows.double().numpy()
+        per_env = {name: t.index_select(0, rows.to(t.device)) for name, t in per_env.items()}
+    for name, t in per_env.items():
+        arrays[name] = t.float().cpu().numpy()
+    logging = extras.get(logging_key, {})
+    keys = sorted(logging)
+    arrays["logging"] = np.array([float(logging[k]) for k in keys], dtype=np.float64)
+    return {"arrays": arrays, "num_envs": n, "logging_keys": keys}
+
+
+def dump_outputs(directory: str, outputs: dict, meta: dict) -> None:
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs["arrays"].items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+    index = {
+        **meta, "num_envs": outputs["num_envs"], "logging_keys": outputs["logging_keys"],
+        "arrays": {name: {"shape": list(a.shape), "dtype": str(a.dtype)} for name, a in outputs["arrays"].items()},
+    }
+    with open(os.path.join(directory, "outputs.json"), "w") as f:
+        json.dump(index, f, indent=1)
 
 
 def pin_to_gpu_numa_node(index: int) -> dict:
@@ -512,12 +568,17 @@ def run_b200(args, rank, local_rank, world):
     actions = [a.to(dev) for a in actions_host]
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    ms, resets_per_step = time_dropin(env, actions, args.steps, args.warmup, dist_on)
+    dump = args.dump_outputs is not None and rank == 0
+    ms, resets_per_step = time_dropin(env, actions, args.steps, args.warmup, dist_on, keep_outputs=dump)
     prof = fused.profile_read()
     aux_prof = fused.profile_read_aux()
     fused.profile(False)
     launches = env.timed_launches
     clocks = sampler.stop(env.timed_window) if sampler else None
+    if dump:
+        dump_outputs(args.dump_outputs, env.timed_outputs,
+                     {"config": args.config, "num_envs_per_gpu": N, "n_gpus": world, "rank": rank, "seed": seed,
+                      "steps": args.steps, "warmup": args.warmup, "pool": args.pool})
 
     value = N * world / (ms / 1e3)
     peak, peak_src = peaks()
@@ -529,10 +590,9 @@ def run_b200(args, rank, local_rank, world):
 
     e2e = None
     if not args.no_e2e:
-        e2e_steps = max(3, min(args.steps, 10))
-        e2e_ms, h2d, d2h = time_e2e(env, actions_host, e2e_steps, 3, dist_on)
+        e2e_ms, h2d, d2h = time_e2e(env, actions_host, args.steps, args.warmup, dist_on)
         e2e = {"value": N * world / (e2e_ms / 1e3), "unit": UNIT, "h2d_bytes_per_step": h2d,
-               "d2h_bytes_per_step": d2h, "ms_per_step": e2e_ms, "steps": e2e_steps, "numa": numa,
+               "d2h_bytes_per_step": d2h, "ms_per_step": e2e_ms, "steps": args.steps, "numa": numa,
                "overlap": "observation read-back of step i on a copy stream, overlapping step i+1's H2D copies"}
 
     sweep = {}
@@ -540,7 +600,7 @@ def run_b200(args, rank, local_rank, world):
         for n_small in (4096, 65536):
             if n_small >= N:
                 continue
-            m = measure_config(args.config, n_small, dev, max(args.pool, 4), seed, max(args.steps, 100), max(args.warmup, 10), peak)
+            m = measure_config(args.config, n_small, dev, max(args.pool, 4), seed, args.steps, args.warmup, peak)
             sweep[str(n_small)] = {k: m[k] for k in ("value", "ms_per_step", "post_kernel_us", "action_kernel_us",
                                                        "step_roofline_frac", "l2")}
 
@@ -558,17 +618,15 @@ def run_b200(args, rank, local_rank, world):
                       "post_kernel_us": m["post_kernel_us"]}
     elif not args.no_configs:
         for name, n_cfg in EXTRA_CONFIGS:
-            k_steps = 100 if n_cfg <= 65536 else 20
-            configs[f"{name}:{n_cfg}"] = measure_config(name, n_cfg, dev, 4, seed, k_steps, 5, peak)
+            configs[f"{name}:{n_cfg}"] = measure_config(name, n_cfg, dev, 4, seed, args.steps, args.warmup, peak)
 
     cpu = None
     os.sched_setaffinity(0, all_cpus)  # the CPU baseline uses every core of the box
     if rank == 0 and not dist_on and not args.no_cpu:
-        n_cpu = args.cpu_envs or N
-        cpu_steps = 40  # a bounded sample: ~5-20 s of host work at 1M envs depending on the table
-        v, threads, cpu_ms, kind = time_cpu_reference(spec, n_cpu, args.pool, cpu_steps, 3, 1234)
+        n_cpu = args.cpu_envs or cpu_sample_envs(N, args.steps, args.warmup)
+        v, threads, cpu_ms, kind = time_cpu_reference(spec, n_cpu, args.pool, args.steps, args.warmup, 1234)
         cpu = {"value": v, "unit": UNIT, "cores": threads, "kind": kind, "ms_per_step": cpu_ms,
-               "sample": f"{cpu_steps} steps of {n_cpu} envs ({args.config} term table) on torch-CPU, {cpu_model()}; "
+               "sample": f"{args.steps} steps of {n_cpu} envs ({args.config} term table) on torch-CPU, {cpu_model()}; "
                          + ("the unmodified reference package" if kind == "reference" else "oracle port")}
 
     if rank == 0:

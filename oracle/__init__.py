@@ -17,5 +17,5 @@ ref_harness.py    builds the reference's own ManagedEnvironment + managers from 
 manager_port.py   the oracle proper: torch-CPU, op-for-op restatement of the reference managers,
                   driven by the same term-table spec; travels to the GPU box
 specs.py          the five BASELINE.json configs as term-table specs
-make_golden.py    regenerates tests/golden/*.pt from the unmodified reference
+make_golden.py    regenerates tests/golden/ from the unmodified reference; load() reads a trace
 """

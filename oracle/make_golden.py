@@ -1,5 +1,5 @@
 """
-TEST INFRASTRUCTURE (oracle).  Regenerates tests/golden/<config>.pt from the UNMODIFIED reference.
+TEST INFRASTRUCTURE (oracle).  Regenerates tests/golden/<config>.pt.xz from the UNMODIFIED reference.
 
     python -m oracle.make_golden            (needs /root/reference; run in the build container)
 
@@ -14,6 +14,8 @@ last-ulp behaviour of the CPU reference depends on ATen's dispatch level (SURVEY
 """
 from __future__ import annotations
 
+import io
+import lzma
 import os
 import sys
 
@@ -22,6 +24,31 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 NUM_ENVS, STEPS, SEED, NAN_STEP = 16, 48, 2024, 5
+
+
+def save(trace: dict, name: str) -> str:
+    """tests/golden/<name>.pt.xz: the torch.save of `trace`, xz-compressed (a trace with a few hundred
+    observation columns is 1.5 MB raw, 0.2 MB compressed); replaces an uncompressed <name>.pt."""
+    buf = io.BytesIO()
+    torch.save(trace, buf)
+    path = os.path.join(GOLDEN_DIR, f"{name}.pt.xz")
+    with open(path, "wb") as f:
+        f.write(lzma.compress(buf.getvalue(), preset=9 | lzma.PRESET_EXTREME))
+    stale = os.path.join(GOLDEN_DIR, f"{name}.pt")
+    if os.path.exists(stale):
+        os.remove(stale)
+    return path
+
+
+def load(name: str) -> dict:
+    """The golden trace `name`: tests/golden/<name>.pt.xz, or the uncompressed tests/golden/<name>.pt."""
+    path = os.path.join(GOLDEN_DIR, f"{name}.pt.xz")
+    if os.path.exists(path):
+        with open(path, "rb") as f:
+            return torch.load(io.BytesIO(lzma.decompress(f.read())), weights_only=False)
+    path = os.path.join(GOLDEN_DIR, f"{name}.pt")
+    assert os.path.exists(path), f"missing golden fixture {path} (python -m oracle.make_golden)"
+    return torch.load(path, weights_only=False)
 
 
 def state_checksum(scene) -> float:
@@ -72,8 +99,7 @@ def main(names=None):
         spec = specs.get(name)
         env = ref_harness.make_reference_env(spec, NUM_ENVS, seed=SEED)
         trace = trace_of(env, spec, NUM_ENVS, STEPS, SEED, NAN_STEP, compare.extras_to_cpu, compare.reference_snapshot)
-        path = os.path.join(GOLDEN_DIR, f"{name}.pt")
-        torch.save(trace, path)
+        path = save(trace, name)
         n_reset = sum(int(s["reset_idx"].numel()) for s in trace["step"])
         print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB, {n_reset} resets in {STEPS} steps")
     for stock_terms in (False, True):
@@ -93,8 +119,7 @@ def second_entity_trace(stock_terms: bool = False):
     env = second_entity.add_prop(ref_harness.make_reference_env(spec, NUM_ENVS, seed=SEED), reference_namespace())
     trace = trace_of(env, spec, NUM_ENVS, STEPS, SEED, None, compare.extras_to_cpu, lambda env: {},
                      extra_of=second_entity.prop_cache)
-    path = os.path.join(GOLDEN_DIR, f"{spec['name']}.pt")
-    torch.save(trace, path)
+    path = save(trace, spec["name"])
     n_reset = sum(int(s["reset_idx"].numel()) for s in trace["step"])
     print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB, {n_reset} resets in {STEPS} steps")
 

@@ -220,12 +220,10 @@ def test_cuda_path_reproduces_reference_golden_trace(name, cuda_device):
     in the build container by oracle/make_golden.py): same seeded inputs, the reference's random draws
     injected via the oracle port (which the CPU suite pins bit-exactly to the same traces).
     """
-    import os
-
-    from oracle.make_golden import GOLDEN_DIR
+    from oracle import make_golden
     from oracle.parity import ParityRun, _close
 
-    gold = torch.load(os.path.join(GOLDEN_DIR, f"{name}.pt"), weights_only=False)
+    gold = make_golden.load(name)
     run = ParityRun(name, num_envs=gold["num_envs"], device=cuda_device, seed=gold["seed"], sanitize=False)
     run.reset()
     for i, g in enumerate(gold["step"]):

@@ -10,8 +10,6 @@ genesis_forge/managed_env.py:200-220, :269-270, :294-296, :353-354).  Workload: 
     columns -- CPU, dry run;
   * the CUDA path reproduces the trace -- GPU.
 """
-import os
-
 import pytest
 import torch
 
@@ -21,17 +19,13 @@ from configs.env_builder import build_env, dropin_namespace
 from genesis_forge_b200 import _native as nat
 from genesis_forge_b200.fused import UnsupportedTermError
 from genesis_forge_b200.synthetic import ROBOT_MODELS, StateSource
-from oracle import geom
-from oracle.make_golden import GOLDEN_DIR
+from oracle import geom, make_golden
 from oracle.parity import _close
-
-GOLD = os.path.join(GOLDEN_DIR, "second_entity.pt")
-GOLD_TERMS = os.path.join(GOLDEN_DIR, "second_entity_terms.pt")
 
 
 def test_reference_trace_of_the_second_manager():
     """Pins the semantics the drop-in has to reproduce, on the reference's own output."""
-    gold = torch.load(GOLD, weights_only=False)
+    gold = make_golden.load("second_entity")
     n, spec = gold["num_envs"], second_entity.spec()
     source = StateSource(ROBOT_MODELS[spec["robot"]], n, 8, gold["seed"])
     gravity = torch.tensor([0.0, 0.0, -1.0]).expand(n, 3)
@@ -125,7 +119,7 @@ def test_body_acceleration_of_a_further_entity_is_refused(cpu_device):
 @pytest.mark.gpu
 @pytest.mark.parametrize("stock_terms", [False, True], ids=["getters", "stock_terms"])
 def test_cuda_path_reproduces_reference_trace_with_two_entity_managers(stock_terms, cuda_device):
-    gold = torch.load(GOLD_TERMS if stock_terms else GOLD, weights_only=False)
+    gold = make_golden.load("second_entity_terms" if stock_terms else "second_entity")
     n = gold["num_envs"]
     gfb.set_device(cuda_device)
     env = _dropin(n, cuda_device, stock_terms=stock_terms, seed=gold["seed"])
