@@ -172,6 +172,16 @@ void canonicalize(gfb_program_head& c) {
   }
 }
 
+bool uses_user_terms(const gfb_program_head& P, uint32_t phases) {
+  if (phases & GFB_PHASE_REWARD)
+    for (int r = 0; r < P.n_reward; ++r)
+      if (P.reward[r].op == GFB_R_USER && P.reward[r].weight != 0.0f) return true;
+  if (phases & GFB_PHASE_TERMINATION)
+    for (int t = 0; t < P.n_termination; ++t)
+      if (P.termination[t].op == GFB_T_USER) return true;
+  return false;
+}
+
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 int tile_index(int tile) { return tile == 32 ? 0 : (tile == 64 ? 1 : (tile == 128 ? 2 : 3)); }
@@ -992,6 +1002,11 @@ int gfb_post_physics(gfb_handle* h, const gfb_buffers* b, uint32_t phases, void*
         }
       }
     }
+    // user-defined terms lowered to device code exist only in the specialised kernel generated for them
+    if (c.spec_index < 0 && uses_user_terms(P, phases))
+      return fail(h, GFB_ERR_UNSUPPORTED,
+                  "the program has GFB_R_USER / GFB_T_USER terms and no specialised kernel generated for them is "
+                  "attached (the generic kernel does not evaluate them)");
     c.prog_epoch = h->prog_epoch;
     c.spec_gen = h->spec_gen;
     c.phases = phases;

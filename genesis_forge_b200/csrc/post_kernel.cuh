@@ -131,6 +131,35 @@ __device__ __forceinline__ void issue_slab_loads(const KParams& K, const Plan& p
   __syncwarp();
 }
 
+// What a user-defined term lowered to device code (genesis_forge_b200/expr.py) reads: the slab rows and
+// body-frame registers the plan already has (pos / quat / vel / ang, lin_b / ang_b / grav_b), otherwise its
+// env's rows of the engine / environment arrays in global memory; the owner thread's registers (episode
+// counters, this step's termination flags, the inverse base quaternion) and stash; its live params.
+struct UserCtx {
+  const gfb_buffers& b;
+  size_t e;
+  int ep_len, max_len;
+  bool terminated, truncated;
+  float iw;
+  V3 iq;
+  V3 lin_b, ang_b, grav_b;
+  const float* S;
+  int tid;
+  const float* st;
+  const Plan& plan;
+  const float* p;
+};
+
+#if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
+__device__ __forceinline__ float gfb_user_min(float a, float b) { return (a < b || a != a) ? a : b; }
+__device__ __forceinline__ float gfb_user_max(float a, float b) { return (a > b || a != a) ? a : b; }
+__device__ __forceinline__ int gfb_user_mod(int a, int b) {  // torch's remainder: the sign of the divisor
+  const int r = a % b;
+  return (r != 0 && ((r < 0) != (b < 0))) ? r + b : r;
+}
+GFB_SPEC_USER_TERMS
+#endif
+
 // Blocks per SM promised to the register allocator: the generic build assumes 768 threads per SM; a
 // specialised build knows its slab's shared memory and promises only what that admits (spec.py)
 #ifdef GFB_SPEC
@@ -592,6 +621,12 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
         case GFB_T_EXTERNAL:  // user-defined term evaluated on the host before this launch
           v = GFB_BUF(const float, GFB_B_EXT_VALUES)[(size_t)ts.i0 * N + e] != 0.0f;
           break;
+#if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
+        case GFB_T_USER:  // user-defined term lowered to device code (generated header)
+          v = user_termination(t, UserCtx{K.b, (size_t)e, ep_len, max_len, false, false, iw, iq, lin_b, ang_b, grav_b, S, tid,
+                                          st, plan, tt.p});
+          break;
+#endif
         default:
           break;
       }
@@ -817,6 +852,12 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
         case GFB_R_EXTERNAL:  // user-defined term evaluated on the host before this launch
           v = GFB_BUF(const float, GFB_B_EXT_VALUES)[(size_t)rs.ext_col * N + e];
           break;
+#if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
+        case GFB_R_USER:  // user-defined term lowered to device code (generated header)
+          v = user_reward(r, UserCtx{K.b, (size_t)e, ep_len, max_len, terminated, truncated, iw, iq, lin_b, ang_b, grav_b,
+                                     S, tid, st, plan, rt.p});
+          break;
+#endif
         default:
           break;
       }

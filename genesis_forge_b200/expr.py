@@ -1,0 +1,1012 @@
+"""
+User-defined reward / termination terms lowered into the specialised post-physics kernel.
+
+A user term is a plain Python function of the environment, e.g.
+
+    def speed(env):
+        return env.robot.get_vel()[:, 0].abs()
+
+`trace_term` runs it ONCE with symbolic stand-ins for the per-env state it may read (the primary
+entity's getters, the first EntityManager's cache and body-frame vectors, the action manager's
+getters, env.actions / last_actions / episode_length / max_episode_length, the `command` of
+kernel-resampled command managers, contact forces and air-time state, and -- rewards only --
+extras["terminations"] / ["time_outs"]).  Every operation on them is recorded as a node of a small
+expression IR (`Program`) with torch's shapes and type promotion.  Scalar entries of the term's
+params become LIVE slots (the term's p[4] in the packed table), so a curriculum that edits them keeps
+the same kernel binary; everything else the function captures is a compile-time constant.
+
+`device_code` turns a Program into one straight-line `__device__` function per term, in torch's
+operation order with the kernel's round-to-nearest helpers; reductions accumulate in index order.
+The generated functions go into the header of the specialised kernel (spec.py) and are called in the
+owner phase of post_kernel, in the GFB_R_USER / GFB_T_USER cases of the term switches.
+
+Anything outside this subset raises UnsupportedTermError naming the op or source; the term then
+stays a host callback (split execution), with exactly the results it had before.
+"""
+from __future__ import annotations
+
+import hashlib
+import math
+
+import numpy as np
+import torch
+
+from .managers.observation import UnsupportedTermError
+
+F32, I32, BOOL = "f32", "i32", "bool"
+_RANK = {BOOL: 0, I32: 1, F32: 2}
+MAX_CONST_VEC = 32  # GFB_MAX_DOFS: small constant vectors (per-joint limits, gains) are folded in
+MAX_LIVE_PARAMS = 4  # gfb_reward_term.p / gfb_termination_term.p
+
+
+class _ParamControlFlow(Exception):
+    """A live parameter reached Python control flow: trace again with params as constants."""
+
+
+def _f32(x) -> float:
+    return float(np.float32(x))
+
+
+# ------------------------------------------------------------------------------------------------
+# IR
+# ------------------------------------------------------------------------------------------------
+class Node:
+    __slots__ = ("op", "args", "attr", "shape", "dtype", "weak")
+
+    def __init__(self, op, args, attr, shape, dtype, weak=False):
+        self.op, self.args, self.attr = op, tuple(args), attr
+        self.shape, self.dtype, self.weak = tuple(shape), dtype, weak
+
+    def text(self, i: int) -> str:
+        return f"%{i} = {self.op}({', '.join('%' + str(a) for a in self.args)}; {self.attr!r}) : {self.dtype}{list(self.shape)}{' weak' if self.weak else ''}"
+
+
+class Program:
+    """The IR of one term: nodes in evaluation order, the result node, the live parameter names."""
+
+    def __init__(self, kind: str, nodes: list, out: int, params: list[str], param_types: list[str]):
+        self.kind, self.nodes, self.out = kind, nodes, out
+        self.params, self.param_types = params, param_types
+
+    def text(self) -> str:
+        head = f"{self.kind} params={self.params} types={self.param_types} out=%{self.out}\n"
+        return head + "\n".join(n.text(i) for i, n in enumerate(self.nodes))
+
+    def digest(self) -> int:
+        """31-bit identity of the expression (stored in the term's structural `i0` field)."""
+        return int.from_bytes(hashlib.sha1(self.text().encode()).digest()[:4], "little") & 0x7FFFFFFF
+
+    def sources(self) -> list[tuple]:
+        return [n.attr for n in self.nodes if n.op == "src"]
+
+
+# ------------------------------------------------------------------------------------------------
+# symbolic values
+# ------------------------------------------------------------------------------------------------
+def _promote(a: "Sym", b: "Sym") -> str:
+    """torch.result_type for two operands; `weak` operands are Python scalars (SURVEY appendix C)."""
+    if a.weak == b.weak:
+        return a.dtype_ if _RANK[a.dtype_] >= _RANK[b.dtype_] else b.dtype_
+    strong, weak = (b, a) if a.weak else (a, b)
+    return weak.dtype_ if _RANK[weak.dtype_] > _RANK[strong.dtype_] else strong.dtype_
+
+
+def _bshape(a: "Sym", b: "Sym", what: str) -> tuple:
+    if a.shape_ == b.shape_ or not b.shape_:
+        return a.shape_
+    if not a.shape_:
+        return b.shape_
+    raise UnsupportedTermError(f"user term: '{what}' of shapes (N, *{a.shape_}) and (N, *{b.shape_}) does not broadcast "
+                               "row by row")
+
+
+class Sym:
+    """A (N, *shape) tensor of the trace.  `weak`: a Python scalar (live param or constant)."""
+
+    __hash__ = object.__hash__
+
+    def __init__(self, tr: "Tracer", nid: int):
+        self._tr, self._id = tr, nid
+
+    @property
+    def _node(self) -> Node:
+        return self._tr.nodes[self._id]
+
+    shape_ = property(lambda self: self._node.shape)
+    dtype_ = property(lambda self: self._node.dtype)
+
+    @property
+    def weak(self):
+        return self._node.weak
+
+    @property
+    def dtype(self):
+        return {F32: torch.float32, I32: torch.int32, BOOL: torch.bool}[self._node.dtype]
+
+    @property
+    def shape(self):
+        if self.weak:
+            return torch.Size(())
+        return torch.Size((self._tr.N,) + self._node.shape)
+
+    @property
+    def device(self):
+        return self._tr.device
+
+    def size(self, dim=None):
+        return self.shape if dim is None else self.shape[dim]
+
+    def dim(self):
+        return len(self.shape)
+
+    ndim = property(dim)
+
+    # -- refusals -------------------------------------------------------------------------------
+    def _control(self, what):
+        if self.weak:
+            raise _ParamControlFlow(what)
+        raise UnsupportedTermError(f"user term: {what} of a per-env value (data-dependent Python control flow)")
+
+    def __bool__(self):
+        self._control("__bool__")
+
+    def __index__(self):
+        self._control("__index__")
+
+    def __int__(self):
+        self._control("__int__")
+
+    def __float__(self):
+        self._control("__float__")
+
+    def __len__(self):
+        return self.shape[0] if self.shape else self._control("len()")
+
+    def __iter__(self):
+        raise UnsupportedTermError("user term: iteration over a per-env value")
+
+    def __setitem__(self, key, value):
+        raise UnsupportedTermError("user term: in-place write (__setitem__)")
+
+    def __getattr__(self, name):
+        if name.startswith("__"):
+            raise AttributeError(name)
+        raise UnsupportedTermError(f"user term: tensor method '{name}' is not supported by the expression IR")
+
+    def _inplace(self, *a, **k):
+        raise UnsupportedTermError("user term: in-place arithmetic")
+
+    __iadd__ = __isub__ = __imul__ = __itruediv__ = __iand__ = __ior__ = __imod__ = __ipow__ = _inplace
+
+    # -- arithmetic ------------------------------------------------------------------------------
+    def __add__(self, o): return self._tr.binary("add", self, o)
+    def __radd__(self, o): return self._tr.binary("add", o, self)
+    def __sub__(self, o): return self._tr.binary("sub", self, o)
+    def __rsub__(self, o): return self._tr.binary("sub", o, self)
+    def __mul__(self, o): return self._tr.binary("mul", self, o)
+    def __rmul__(self, o): return self._tr.binary("mul", o, self)
+    def __truediv__(self, o): return self._tr.binary("div", self, o)
+    def __rtruediv__(self, o): return self._tr.binary("div", o, self)
+    def __mod__(self, o): return self._tr.binary("mod", self, o)
+    def __rmod__(self, o): return self._tr.binary("mod", o, self)
+    def __lt__(self, o): return self._tr.binary("lt", self, o)
+    def __le__(self, o): return self._tr.binary("le", self, o)
+    def __gt__(self, o): return self._tr.binary("gt", self, o)
+    def __ge__(self, o): return self._tr.binary("ge", self, o)
+    def __eq__(self, o): return self._tr.binary("eq", self, o)
+    def __ne__(self, o): return self._tr.binary("ne", self, o)
+    def __and__(self, o): return self._tr.binary("and", self, o)
+    def __rand__(self, o): return self._tr.binary("and", o, self)
+    def __or__(self, o): return self._tr.binary("or", self, o)
+    def __ror__(self, o): return self._tr.binary("or", o, self)
+    def __neg__(self): return self._tr.unary("neg", self)
+    def __invert__(self): return self._tr.unary("not", self)
+    def __abs__(self): return self._tr.unary("abs", self)
+
+    def __pow__(self, o):
+        if isinstance(o, (int, float)) and not isinstance(o, bool) and o == 2:
+            return self._tr.unary("square", self)
+        raise UnsupportedTermError(f"user term: '** {o!r}' (only ** 2 is supported)")
+
+    # -- methods ---------------------------------------------------------------------------------
+    def abs(self): return self._tr.unary("abs", self)
+    def square(self): return self._tr.unary("square", self)
+    def sqrt(self): return self._tr.unary("sqrt", self)
+    def exp(self): return self._tr.unary("exp", self)
+    def log(self): return self._tr.unary("log", self)
+    def sin(self): return self._tr.unary("sin", self)
+    def cos(self): return self._tr.unary("cos", self)
+    def tanh(self): return self._tr.unary("tanh", self)
+    def logical_not(self): return self._tr.unary("not", self)
+    def float(self): return self._tr.cast(self, F32)
+    def int(self): return self._tr.cast(self, I32)
+    def bool(self): return self._tr.cast(self, BOOL)
+    def detach(self): return self
+    def clone(self): return self
+    def contiguous(self): return self
+
+    def clamp(self, min=None, max=None): return self._tr.clamp(self, min, max)
+    clip = clamp
+
+    def sum(self, dim=None, keepdim=False): return self._tr.reduce("sum", self, dim, keepdim)
+    def mean(self, dim=None, keepdim=False): return self._tr.reduce("mean", self, dim, keepdim)
+    def any(self, dim=None, keepdim=False): return self._tr.reduce("any", self, dim, keepdim)
+    def all(self, dim=None, keepdim=False): return self._tr.reduce("all", self, dim, keepdim)
+    def amax(self, dim=None, keepdim=False): return self._tr.reduce("amax", self, dim, keepdim)
+    def amin(self, dim=None, keepdim=False): return self._tr.reduce("amin", self, dim, keepdim)
+
+    def norm(self, p=2, dim=None, keepdim=False):
+        if p != 2:
+            raise UnsupportedTermError(f"user term: norm(p={p!r}) (only the 2-norm is supported)")
+        return self._tr.reduce("norm", self, dim, keepdim)
+
+    def minimum(self, o): return self._tr.binary("minimum", self, o)
+    def maximum(self, o): return self._tr.binary("maximum", self, o)
+
+    def to(self, *args, **kwargs):
+        dtype = kwargs.get("dtype") or next((a for a in args if isinstance(a, torch.dtype)), None)
+        return self._tr.cast(self, _dtype_of(dtype)) if dtype is not None else self
+
+    def type(self, dtype):
+        return self._tr.cast(self, _dtype_of(dtype))
+
+    def __getitem__(self, key):
+        return self._tr.index(self, key)
+
+    def nonzero(self, *a, **k):
+        raise UnsupportedTermError("user term: nonzero() (data-dependent shape)")
+
+    # -- torch functions -------------------------------------------------------------------------
+    @classmethod
+    def __torch_function__(cls, func, types, args=(), kwargs=None):
+        kwargs = kwargs or {}
+        operands = list(args) + list(kwargs.values())
+        tr = next((a._tr for a in operands if isinstance(a, Sym)), None)
+        if tr is None:  # the symbolic values sit inside a sequence argument (torch.stack, torch.cat, ...)
+            name = getattr(func, "__name__", str(func))
+            raise UnsupportedTermError(f"user term: torch function '{name}' of a sequence of per-env values")
+        return tr.torch_function(func, args, kwargs)
+
+
+def _dtype_of(dtype) -> str:
+    if dtype in (torch.float32, torch.float):
+        return F32
+    if dtype in (torch.int32, torch.int64, torch.int):
+        return I32
+    if dtype is torch.bool:
+        return BOOL
+    raise UnsupportedTermError(f"user term: dtype {dtype} (float32, int32/int64 and bool are supported)")
+
+
+_UNARY_TORCH = {
+    "abs": "abs", "square": "square", "sqrt": "sqrt", "exp": "exp", "log": "log", "sin": "sin", "cos": "cos",
+    "tanh": "tanh", "neg": "neg", "negative": "neg", "logical_not": "not", "bitwise_not": "not",
+}
+_BINARY_TORCH = {
+    "add": "add", "sub": "sub", "subtract": "sub", "mul": "mul", "multiply": "mul", "div": "div", "divide": "div",
+    "true_divide": "div", "remainder": "mod", "lt": "lt", "less": "lt", "le": "le", "gt": "gt", "greater": "gt",
+    "ge": "ge", "eq": "eq", "ne": "ne", "logical_and": "and", "logical_or": "or", "bitwise_and": "and",
+    "bitwise_or": "or", "minimum": "minimum", "maximum": "maximum",
+}
+_REDUCE_TORCH = {"sum": "sum", "mean": "mean", "any": "any", "all": "all", "amax": "amax", "amin": "amin"}
+
+
+# ------------------------------------------------------------------------------------------------
+# tracer
+# ------------------------------------------------------------------------------------------------
+class Tracer:
+    def __init__(self, N: int, kind: str, device=torch.device("cpu")):
+        self.N, self.kind, self.device = N, kind, device
+        self.nodes: list[Node] = []
+        self._cse: dict = {}
+        self.params: list[str] = []
+        self.param_types: list[str] = []
+
+    def add(self, op, args, attr, shape, dtype, weak=False) -> Sym:
+        key = (op, tuple(args), repr(attr), tuple(shape), dtype, weak)
+        nid = self._cse.get(key)
+        if nid is None:
+            nid = len(self.nodes)
+            self.nodes.append(Node(op, args, attr, shape, dtype, weak))
+            self._cse[key] = nid
+        return Sym(self, nid)
+
+    def source(self, key: tuple, shape: tuple, dtype: str) -> Sym:
+        return self.add("src", (), key, shape, dtype)
+
+    def param(self, name: str, value) -> Sym:
+        dtype = I32 if isinstance(value, int) else F32
+        if len(self.params) >= MAX_LIVE_PARAMS:
+            raise UnsupportedTermError(f"user term: more than {MAX_LIVE_PARAMS} scalar params")
+        self.params.append(name)
+        self.param_types.append(dtype)
+        return self.add("param", (), len(self.params) - 1, (), dtype, weak=True)
+
+    # -- operands ----------------------------------------------------------------------------------
+    def lift(self, x) -> Sym:
+        if isinstance(x, Sym):
+            return x
+        if isinstance(x, bool):
+            return self.add("const", (), bool(x), (), BOOL, weak=True)
+        if isinstance(x, int):
+            if not -(1 << 31) <= x < (1 << 31):
+                raise UnsupportedTermError(f"user term: integer constant {x} does not fit int32")
+            return self.add("const", (), int(x), (), I32, weak=True)
+        if isinstance(x, float):
+            return self.add("const", (), float(x), (), F32, weak=True)
+        if isinstance(x, np.generic):
+            return self.lift(x.item())
+        if torch.is_tensor(x):
+            t = x.detach().cpu()
+            if t.dim() == 0:
+                v = t.item()
+                dtype = _dtype_of(t.dtype)
+                value = bool(v) if dtype == BOOL else (int(v) if dtype == I32 else _f32(v))
+                return self.add("const", (), value, (), dtype, weak=True)
+            if t.dim() == 1 and t.shape[0] <= MAX_CONST_VEC and t.shape[0] != self.N:
+                dtype = _dtype_of(t.dtype)
+                vals = tuple(bool(v) if dtype == BOOL else (int(v) if dtype == I32 else _f32(v)) for v in t.tolist())
+                return self.add("constvec", (), vals, (t.shape[0],), dtype)
+            raise UnsupportedTermError(
+                f"user term: a concrete tensor of shape {tuple(t.shape)} enters the expression (per-env state the "
+                "kernel does not hold: a captured buffer, a further entity, a user-level manager's state)")
+        raise UnsupportedTermError(f"user term: operand of type {type(x).__name__}")
+
+    # -- ops ---------------------------------------------------------------------------------------
+    def unary(self, op: str, a) -> Sym:
+        a = self.lift(a)
+        dt = a.dtype_
+        if op == "not":
+            if dt != BOOL:
+                raise UnsupportedTermError("user term: '~' on a non-bool value (bitwise not of integers)")
+            out = BOOL
+        elif op in ("neg", "abs", "square"):
+            if dt == BOOL:
+                raise UnsupportedTermError(f"user term: '{op}' of a bool value")
+            out = dt
+        else:  # transcendental / sqrt: integer inputs become float32
+            out = F32
+        if a.weak and op != "neg":
+            raise _ParamControlFlow(op)  # math on a Python scalar: evaluated in double by the function itself
+        x = a if out == dt or op in ("neg", "abs", "square", "not") else self.cast(a, F32)
+        return self.add(op, (x._id,), None, a.shape_, out, weak=a.weak)
+
+    def cast(self, a, dtype: str) -> Sym:
+        a = self.lift(a)
+        if a.dtype_ == dtype:
+            return a
+        return self.add("cast", (a._id,), dtype, a.shape_, dtype, weak=a.weak)
+
+    def binary(self, op: str, a, b) -> Sym:
+        a, b = self.lift(a), self.lift(b)
+        if a.weak and b.weak:
+            raise _ParamControlFlow(op)  # Python scalars combine in double precision
+        shape = _bshape(a, b, op)
+        dt = _promote(a, b)
+        if op in ("and", "or"):
+            if a.dtype_ != BOOL or b.dtype_ != BOOL:
+                raise UnsupportedTermError(f"user term: '{op}' of non-bool values (bitwise integer ops)")
+            return self.add(op, (a._id, b._id), None, shape, BOOL)
+        if op == "div":
+            dt = F32  # true division
+        if op == "mod" and dt != I32:
+            raise UnsupportedTermError("user term: '%' is supported for integers only")
+        if op in ("add", "sub", "mul", "minimum", "maximum") and dt == BOOL:
+            raise UnsupportedTermError(f"user term: '{op}' of two bool values")
+        ca, cb = self.cast(a, dt), self.cast(b, dt)
+        if op in ("lt", "le", "gt", "ge", "eq", "ne"):
+            return self.add(op, (ca._id, cb._id), None, shape, BOOL)
+        return self.add(op, (ca._id, cb._id), None, shape, dt)
+
+    def where(self, c, a, b) -> Sym:
+        c, a, b = self.lift(c), self.lift(a), self.lift(b)
+        if c.dtype_ != BOOL:
+            raise UnsupportedTermError("user term: where() with a non-bool condition")
+        if a.weak and b.weak:
+            dt = a.dtype_ if _RANK[a.dtype_] >= _RANK[b.dtype_] else b.dtype_
+        else:
+            dt = _promote(a, b)
+        shape = max((c.shape_, a.shape_, b.shape_), key=len)
+        for s in (c.shape_, a.shape_, b.shape_):
+            if s and s != shape:
+                raise UnsupportedTermError("user term: where() operands do not broadcast row by row")
+        if c.weak:
+            raise UnsupportedTermError("user term: where() with a scalar condition")
+        return self.add("where", (c._id, self.cast(a, dt)._id, self.cast(b, dt)._id), None, shape, dt)
+
+    def clamp(self, x, lo, hi) -> Sym:
+        x = self.lift(x)
+        if lo is None and hi is None:
+            raise UnsupportedTermError("user term: clamp() without bounds")
+        if x.dtype_ == BOOL:
+            raise UnsupportedTermError("user term: clamp() of a bool value")
+        out = x
+        # torch.clamp(x, lo, hi) == min(max(x, lo), hi), NaN propagating
+        if lo is not None:
+            lo = self.lift(lo)
+            dt = _promote(out, lo)
+            out = self.add("clamp_lo", (self.cast(out, dt)._id, self.cast(lo, dt)._id), None, _bshape(out, lo, "clamp"), dt)
+        if hi is not None:
+            hi = self.lift(hi)
+            dt = _promote(out, hi)
+            out = self.add("clamp_hi", (self.cast(out, dt)._id, self.cast(hi, dt)._id), None, _bshape(out, hi, "clamp"), dt)
+        return out
+
+    def reduce(self, kind: str, x, dim, keepdim=False) -> Sym:
+        x = self.lift(x)
+        if keepdim:
+            raise UnsupportedTermError(f"user term: {kind}(keepdim=True)")
+        if isinstance(dim, (tuple, list)):
+            if len(dim) != 1:
+                raise UnsupportedTermError(f"user term: {kind} over several dims")
+            dim = dim[0]
+        rank = len(x.shape_) + 1
+        if dim is None or rank == 1:
+            raise UnsupportedTermError(f"user term: {kind} over the env dimension")
+        if isinstance(dim, Sym):
+            dim._control("dim")
+        d = dim + rank if dim < 0 else dim
+        if not 1 <= d < rank:
+            raise UnsupportedTermError(f"user term: {kind}(dim={dim}) of a rank-{rank} value")
+        axis = d - 1  # in the per-env shape
+        shape = x.shape_[:axis] + x.shape_[axis + 1:]
+        dt = x.dtype_
+        if kind in ("any", "all"):
+            src = self.cast(x, BOOL) if dt != BOOL else x
+            return self.add(kind, (src._id,), axis, shape, BOOL)
+        if kind == "sum":
+            out = I32 if dt in (BOOL, I32) else F32
+            return self.add("sum", (self.cast(x, out)._id,), axis, shape, out)
+        if kind in ("mean", "norm"):
+            if dt != F32:
+                raise UnsupportedTermError(f"user term: {kind} of a non-float value")
+            return self.add(kind, (x._id,), axis, shape, F32)
+        if dt == BOOL:
+            raise UnsupportedTermError(f"user term: {kind} of a bool value")
+        return self.add(kind, (x._id,), axis, shape, dt)
+
+    def index(self, x: Sym, key) -> Sym:
+        shape = x.shape_
+        if not isinstance(key, tuple):
+            key = (key,)
+        if not key or not (key[0] == slice(None) or key[0] is Ellipsis):
+            raise UnsupportedTermError("user term: indexing that selects envs (only [:, ...] / [..., j] keep every env)")
+        rest = list(key[1:]) if key[0] == slice(None) else None
+        if key[0] is Ellipsis:  # [..., j]: the trailing dims
+            tail = list(key[1:])
+            if any(k is Ellipsis for k in tail) or len(tail) > len(shape):
+                raise UnsupportedTermError("user term: unsupported index")
+            rest = [slice(None)] * (len(shape) - len(tail)) + tail
+        if len(rest) > len(shape):
+            raise UnsupportedTermError("user term: too many indices")
+        rest += [slice(None)] * (len(shape) - len(rest))
+        spec, out_shape = [], []
+        for k, n in zip(rest, shape):
+            if isinstance(k, Sym):
+                k._control("index")
+            if isinstance(k, bool) or not isinstance(k, (int, slice)):
+                raise UnsupportedTermError(f"user term: index {k!r} (ints and basic slices only)")
+            if isinstance(k, int):
+                if not -n <= k < n:
+                    raise UnsupportedTermError(f"user term: index {k} out of range for size {n}")
+                spec.append(k % n)
+            else:
+                start, stop, step = k.indices(n)
+                if step != 1:
+                    raise UnsupportedTermError("user term: strided slice")
+                spec.append((start, max(start, stop)))
+                out_shape.append(max(0, stop - start))
+        if all(isinstance(s, tuple) and s == (0, n) for s, n in zip(spec, shape)):
+            return x
+        return self.add("index", (x._id,), tuple(spec), tuple(out_shape), x.dtype_)
+
+    def torch_function(self, func, args, kwargs):
+        name = getattr(func, "__name__", str(func))
+        if name in ("__get__",) or name.endswith("__setitem__"):
+            raise UnsupportedTermError("user term: in-place write")
+        name = name.strip("_") if name.startswith("__") else name
+        name = {"radd": "add", "rmul": "mul"}.get(name, name)
+        if name.endswith("_") and not name.startswith("_"):
+            raise UnsupportedTermError(f"user term: in-place op {name}")
+        if name in ("rsub", "rtruediv", "rmod"):
+            return self.binary(name[1:].replace("truediv", "div"), args[1], args[0])
+        if name in ("truediv",):
+            name = "div"
+        if name in _UNARY_TORCH and len(args) == 1:
+            return self.unary(_UNARY_TORCH[name], args[0])
+        if name in _BINARY_TORCH:
+            other = args[1] if len(args) > 1 else kwargs.get("other")
+            return self.binary(_BINARY_TORCH[name], args[0], other)
+        if name in ("where",):
+            return self.where(*args[:3])
+        if name in ("clamp", "clip"):
+            lo = args[1] if len(args) > 1 else kwargs.get("min")
+            hi = args[2] if len(args) > 2 else kwargs.get("max")
+            return self.clamp(args[0], lo, hi)
+        if name in _REDUCE_TORCH:
+            dim = args[1] if len(args) > 1 else kwargs.get("dim")
+            return self.reduce(_REDUCE_TORCH[name], args[0], dim, kwargs.get("keepdim", False))
+        if name in ("norm", "vector_norm"):
+            p = kwargs.get("p", kwargs.get("ord", args[1] if len(args) > 1 and name == "norm" else 2))
+            if p not in (2, 2.0, None, "fro"):
+                raise UnsupportedTermError(f"user term: norm(p={p!r})")
+            dim = kwargs.get("dim", args[2] if len(args) > 2 else None)
+            return self.reduce("norm", args[0], dim, kwargs.get("keepdim", False))
+        if name == "pow":
+            return self.lift(args[0]).__pow__(args[1])
+        if name in ("float",):
+            return self.cast(args[0], F32)
+        if name == "getitem":
+            return self.index(self.lift(args[0]), args[1])
+        if name == "nonzero":
+            raise UnsupportedTermError("user term: nonzero() (data-dependent shape)")
+        raise UnsupportedTermError(f"user term: torch function '{name}' is not supported by the expression IR")
+
+
+# ------------------------------------------------------------------------------------------------
+# trace: sources swapped in for the duration of one call
+# ------------------------------------------------------------------------------------------------
+class _EntityProxy:
+    """Stands for the primary entity while a term is traced."""
+
+    def __init__(self, tr: Tracer, dofs_idx, n_dofs: int):
+        self._tr, self._dofs_idx, self._D = tr, dofs_idx, n_dofs
+
+    def get_pos(self, envs_idx=None):
+        return self._plain("pos", 3, envs_idx)
+
+    def get_quat(self, envs_idx=None):
+        return self._plain("quat", 4, envs_idx)
+
+    def get_vel(self, envs_idx=None):
+        return self._plain("vel", 3, envs_idx)
+
+    def get_ang(self, envs_idx=None):
+        return self._plain("ang", 3, envs_idx)
+
+    def _plain(self, key, width, envs_idx):
+        if envs_idx is not None:
+            raise UnsupportedTermError(f"user term: robot.get_{key}(envs_idx=...)")
+        return self._tr.source((key,), (width,), F32)
+
+    def _dofs(self, key, dofs_idx, envs_idx):
+        same = dofs_idx is not None and self._dofs_idx is not None and list(dofs_idx) == list(self._dofs_idx)
+        if envs_idx is not None or not same or self._D == 0:
+            raise UnsupportedTermError(f"user term: robot.get_dofs_{key}() of DOFs other than the action manager's")
+        return self._tr.source((f"dof_{key}",), (self._D,), F32)
+
+    def get_dofs_position(self, dofs_idx=None, envs_idx=None):
+        return self._dofs("pos", dofs_idx, envs_idx)
+
+    def get_dofs_velocity(self, dofs_idx=None, envs_idx=None):
+        return self._dofs("vel", dofs_idx, envs_idx)
+
+    def __getattr__(self, name):
+        raise UnsupportedTermError(f"user term: robot.{name} is not a source of the expression IR")
+
+
+class _AirProxy:
+    def __init__(self, tr: Tracer, m: int, n_links: int):
+        self._tr, self._m, self._L = tr, m, n_links
+
+    def __getitem__(self, j):
+        if not isinstance(j, int) or not 0 <= j < 4:
+            raise UnsupportedTermError("user term: air-time state indexing")
+        return self._tr.source(("air", self._m, j), (self._L,), F32)
+
+
+class _Swap:
+    """Set attributes for the duration of a trace and put the originals back afterwards."""
+
+    def __init__(self):
+        self.saved: list = []
+
+    def set(self, obj, name, value):
+        self.saved.append((obj, name, obj.__dict__.get(name, _MISSING)))
+        setattr(obj, name, value)
+
+    def set_item(self, d: dict, key, value):
+        self.saved.append((d, key, d.get(key, _MISSING)))
+        d[key] = value
+
+    def restore(self):
+        for obj, name, old in reversed(self.saved):
+            if isinstance(obj, dict):
+                if old is _MISSING:
+                    obj.pop(name, None)
+                else:
+                    obj[name] = old
+            elif old is _MISSING:
+                obj.__dict__.pop(name, None)
+            else:
+                setattr(obj, name, old)
+        self.saved = []
+
+
+_MISSING = object()
+
+
+class ExprMode:
+    """env._tracing while a user term is traced: the manager getters' `_trace_or` lands here."""
+
+    def __init__(self, tr: Tracer, fused):
+        self.tr, self.fused = tr, fused
+
+    def source(self, key, compute):
+        tr, D = self.tr, self.fused.D
+        if key in ("lin_vel_b", "ang_vel_b", "gravity_b"):
+            return tr.source((key,), (3,), F32)
+        if key in ("dof_pos", "dof_vel", "targets") and D > 0:
+            return tr.source((key,), (D,), F32)
+        if key == "env_actions" and D > 0:
+            return tr.source(("actions",), (D,), F32)
+        if isinstance(key, tuple) and key[0] == "command":
+            return key[1].command
+        return compute()
+
+
+def param_kinds(params) -> tuple:
+    """Per live-param candidate: int or float (a live param's kernel type, int32 or fp32, follows it)."""
+    return tuple(sorted((k, type(v).__name__) for k, v in dict(params or {}).items()
+                        if isinstance(v, (int, float)) and not isinstance(v, bool)))
+
+
+def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> Program:
+    """Trace one user-defined reward / termination into a Program (raises UnsupportedTermError)."""
+    env = fused.env
+    fn = item.fn
+    what = f"{kind} '{name}'"
+    if not hasattr(getattr(fn, "__func__", fn), "__code__"):  # an MdpFnClass instance (or a builtin)
+        raise UnsupportedTermError(f"{what}: class-style terms keep their own state and are not lowered")
+    tr = Tracer(fused.N, kind, fused.device)
+    params = {}
+    for k, v in dict(item.params or {}).items():
+        if live_params and isinstance(v, (int, float)) and not isinstance(v, bool):
+            params[k] = tr.param(k, v)
+        else:
+            params[k] = v
+    swap = _Swap()
+    try:
+        _install_sources(fused, tr, swap, kind)
+        env._tracing = ExprMode(tr, fused)
+        result = fn(env, **params)
+    finally:
+        env._tracing = None
+        swap.restore()
+    if not isinstance(result, Sym):
+        raise UnsupportedTermError(f"{what}: the result does not depend on per-env state the kernel holds "
+                                   f"({type(result).__name__})")
+    if result.weak or result.shape_ != ():
+        raise UnsupportedTermError(f"{what}: the result has shape {tuple(result.shape)}, not (N,)")
+    if kind == "termination" and result.dtype_ != BOOL:
+        raise UnsupportedTermError(f"{what}: a termination must return a bool tensor")
+    out = result._id
+    if kind == "reward" and result.dtype_ != F32:
+        out = tr.cast(result, F32)._id
+    nodes = _live_nodes(tr.nodes, out)
+    return Program(kind, nodes[0], nodes[1], tr.params, tr.param_types)
+
+
+def lower_term(fused, kind: str, name: str, item) -> tuple[Program, bool]:
+    """(program, params_live): trace with live params, or once more with params as constants."""
+    try:
+        return trace_term(fused, kind, name, item, live_params=True), True
+    except _ParamControlFlow:
+        pass
+    try:
+        return trace_term(fused, kind, name, item, live_params=False), False
+    except _ParamControlFlow as e:
+        raise UnsupportedTermError(f"{kind} '{name}': Python scalar arithmetic on '{e}' inside the term") from None
+
+
+def _live_nodes(nodes: list, out: int) -> tuple[list, int]:
+    """Dead-node elimination + renumbering."""
+    keep, stack = set(), [out]
+    while stack:
+        i = stack.pop()
+        if i in keep:
+            continue
+        keep.add(i)
+        stack.extend(nodes[i].args)
+    order = sorted(keep)
+    remap = {old: new for new, old in enumerate(order)}
+    new = []
+    for old in order:
+        n = nodes[old]
+        new.append(Node(n.op, [remap[a] for a in n.args], n.attr, n.shape, n.dtype, n.weak))
+    return new, remap[out]
+
+
+def _install_sources(fused, tr: Tracer, swap: _Swap, kind: str):
+    env = fused.env
+    robot = fused.primary_entity
+    dofs_idx = fused.action.dofs_idx if fused.action is not None else None
+    proxy = _EntityProxy(tr, dofs_idx, fused.D)
+    if robot is not None:
+        for attr, value in list(vars(env).items()):
+            if value is robot:
+                swap.set(env, attr, proxy)
+    if fused.entity_manager is not None:
+        em = fused.entity_manager
+        swap.set(em, "entity", proxy)
+        swap.set(em, "_base_pos", tr.source(("pos",), (3,), F32))
+        swap.set(em, "_base_quat", tr.source(("quat",), (4,), F32))
+    for k, mgr in enumerate(fused.commands):
+        if mgr in fused.python_commands or mgr._external_controller is not None:
+            continue  # a user-level manager's state stays concrete: refused where it is used
+        swap.set(mgr, "_command", tr.source(("command", k), (mgr._command.shape[1],), F32))
+    for m, mgr in enumerate(fused.contacts):
+        L = int(mgr._link_ids.shape[0])
+        swap.set(mgr, "contacts", tr.source(("contacts", m), (L, 3), F32))
+        if mgr._track_air_time:
+            swap.set(mgr, "_air", _AirProxy(tr, m, L))
+    swap.set(env, "episode_length", tr.source(("episode_length",), (), I32))
+    if env.max_episode_length is not None:
+        swap.set(env, "max_episode_length", tr.source(("max_episode_length",), (), I32))
+    if fused.D > 0:
+        swap.set(env, "_actions", tr.source(("actions",), (fused.D,), F32))
+        swap.set(env, "_last_actions", tr.source(("last_actions",), (fused.D,), F32))
+    extras = env.extras
+    for key, src in (("terminations", "terminated"), ("time_outs", "truncated")):
+        if fused.termination is None:  # nothing publishes the key: reading it fails in the function itself
+            swap.set_item(extras, key, _Refused(f"extras['{key}'] without a termination manager"))
+        elif kind == "reward":
+            swap.set_item(extras, key, tr.source((src,), (), BOOL))
+        else:
+            swap.set_item(extras, key, _Refused(f"extras['{key}'] inside a termination term"))
+
+
+class _Refused:
+    def __init__(self, what):
+        self._what = what
+
+    def __getattr__(self, name):
+        raise UnsupportedTermError(f"user term: {object.__getattribute__(self, '_what')}")
+
+    def _refuse(self, *a, **k):
+        raise UnsupportedTermError(f"user term: {self._what}")
+
+    __invert__ = __and__ = __or__ = __rand__ = __ror__ = __getitem__ = __bool__ = _refuse
+
+    @classmethod
+    def __torch_function__(cls, func, types, args=(), kwargs=None):
+        what = next(a for a in args if isinstance(a, _Refused))._what
+        raise UnsupportedTermError(f"user term: {what}")
+
+
+# ------------------------------------------------------------------------------------------------
+# device code
+# ------------------------------------------------------------------------------------------------
+_CT = {F32: "float", I32: "int", BOOL: "bool"}
+
+
+def _lit(v, dtype) -> str:
+    if dtype == BOOL:
+        return "true" if v else "false"
+    if dtype == I32:
+        return f"({int(v)})"
+    v = _f32(v)
+    if math.isnan(v):
+        return "__int_as_float(0x7fc00000)"
+    if math.isinf(v):
+        return "__int_as_float(0x7f800000)" if v > 0 else "__int_as_float(0xff800000)"
+    return f"{v.hex()}f" if v >= 0 else f"(-{(-v).hex()}f)"
+
+
+_SLAB = {"pos": "off_pos", "quat": "off_quat", "vel": "off_vel", "ang": "off_ang"}  # staged slab rows (plan.h)
+
+
+def _src_elems(key: tuple, shape: tuple, lines: list, v: str) -> list[str]:
+    """C expressions of a source's elements for this env (row-major over `shape`)."""
+    n = int(np.prod(shape)) if shape else 1
+    name = key[0]
+    row = {"pos": ("GFB_B_POS", 3), "quat": ("GFB_B_QUAT", 4), "vel": ("GFB_B_VEL", 3), "ang": ("GFB_B_ANG", 3),
+           "dof_pos": ("GFB_B_DOF_POS", n), "dof_vel": ("GFB_B_DOF_VEL", n), "targets": ("GFB_B_TARGETS", n),
+           "actions": ("GFB_B_ENV_ACTIONS", n), "last_actions": ("GFB_B_ENV_LAST_ACTIONS", n)}
+    if name in row:
+        buf, w = row[name]
+        glob = f"reinterpret_cast<const float*>(c.b.buf[{buf}]) + (size_t)c.e * {w}"
+        if name in _SLAB:  # the slab row when the plan stages the array (a compile-time choice)
+            off = f"c.plan.{_SLAB[name]}"
+            lines.append(f"const float* {v}p = {off} >= 0 ? c.S + {off} + c.tid * {w} : {glob};")
+        else:
+            lines.append(f"const float* {v}p = {glob};")
+        return [f"{v}p[{i}]" for i in range(n)]
+    if name == "command":
+        lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[GFB_B_COMMAND0 + {key[1]}]) + "
+                     f"(size_t)c.e * {n};")
+        return [f"{v}p[{i}]" for i in range(n)]
+    if name == "contacts":
+        lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[GFB_B_CONTACTS0 + {key[1]}]) + "
+                     f"(size_t)c.e * {n};")
+        return [f"{v}p[{i}]" for i in range(n)]
+    if name == "air":
+        m, j = key[1], key[2]
+        return [f"c.st[c.plan.st_air[{m}] + {l * 4 + j}]" for l in range(n)]
+    if name in ("lin_vel_b", "ang_vel_b", "gravity_b"):
+        # the kernel's own register when the plan computes it (same rotation), else rotated here
+        reg, need = {"lin_vel_b": ("lin_b", "NEED_LIN"), "ang_vel_b": ("ang_b", "NEED_ANG"),
+                     "gravity_b": ("grav_b", "NEED_GRAV")}[name]
+        if name == "gravity_b":
+            vec = "V3{0.0f, 0.0f, -1.0f}"
+        else:
+            buf = "GFB_B_VEL" if name == "lin_vel_b" else "GFB_B_ANG"
+            lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[{buf}]) + (size_t)c.e * 3;")
+            vec = f"V3{{{v}p[0], {v}p[1], {v}p[2]}}"
+        lines.append(f"const V3 {v}r = (c.plan.needs & {need}) ? c.{reg} : rotate({vec}, c.iw, c.iq);")
+        return [f"{v}r.x", f"{v}r.y", f"{v}r.z"]
+    if name == "episode_length":
+        return ["c.ep_len"]
+    if name == "max_episode_length":
+        return ["c.max_len"]
+    if name == "terminated":
+        return ["c.terminated"]
+    if name == "truncated":
+        return ["c.truncated"]
+    raise UnsupportedTermError(f"user term: source {key!r}")
+
+
+def _strides(shape):
+    out, s = [], 1
+    for n in reversed(shape):
+        out.append(s)
+        s *= n
+    return list(reversed(out))
+
+
+def _binop(op, a, b, dtype):
+    if dtype == F32:
+        arith = {"add": f"add({a}, {b})", "sub": f"sub({a}, {b})", "mul": f"mul({a}, {b})", "div": f"fdiv({a}, {b})"}
+    else:
+        arith = {"add": f"({a} + {b})", "sub": f"({a} - {b})", "mul": f"({a} * {b})"}
+    if op in arith:
+        return arith[op]
+    if op == "mod":
+        return f"gfb_user_mod({a}, {b})"
+    if op in ("minimum", "clamp_hi"):
+        # NaN propagates (torch.minimum / torch.clamp)
+        return f"gfb_user_min({a}, {b})" if dtype == F32 else f"min({a}, {b})"
+    if op in ("maximum", "clamp_lo"):
+        return f"gfb_user_max({a}, {b})" if dtype == F32 else f"max({a}, {b})"
+    cmp = {"lt": "<", "le": "<=", "gt": ">", "ge": ">=", "eq": "==", "ne": "!="}
+    if op in cmp:
+        return f"({a} {cmp[op]} {b})"
+    if op == "and":
+        return f"({a} && {b})"
+    if op == "or":
+        return f"({a} || {b})"
+    raise UnsupportedTermError(op)
+
+
+def _unop(op, a, dtype):
+    if op == "neg":
+        return f"(-{a})"
+    if op == "not":
+        return f"(!{a})"
+    if op == "abs":
+        return f"fabsf({a})" if dtype == F32 else f"abs({a})"
+    if op == "square":
+        return f"sq({a})" if dtype == F32 else f"({a} * {a})"
+    fn = {"sqrt": "__fsqrt_rn", "exp": "expf", "log": "logf", "sin": "sinf", "cos": "cosf", "tanh": "tanhf"}[op]
+    return f"{fn}({a})"
+
+
+def function_body(prog: Program, fname: str) -> str:
+    """One `__device__` function for the program (straight-line code, one variable per element)."""
+    lines: list[str] = []
+    elems: list[list[str]] = []
+    for i, n in enumerate(prog.nodes):
+        v = f"v{i}"
+        ct = _CT[n.dtype]
+        size = int(np.prod(n.shape)) if n.shape else 1
+        if n.op == "src":
+            exprs = _src_elems(n.attr, n.shape, lines, v)
+        elif n.op == "param":
+            p = f"c.p[{n.attr}]"
+            exprs = [f"((int){p})" if n.dtype == I32 else p]
+        elif n.op == "const":
+            exprs = [_lit(n.attr, n.dtype)]
+        elif n.op == "constvec":
+            exprs = [_lit(x, n.dtype) for x in n.attr]
+        elif n.op == "cast":
+            src = prog.nodes[n.args[0]].dtype
+            a = elems[n.args[0]]
+            if n.dtype == BOOL:
+                exprs = [f"({x} != 0)" for x in a]
+            elif n.dtype == F32 and src == I32:
+                exprs = [f"__int2float_rn({x})" for x in a]
+            elif n.dtype == F32:
+                exprs = [f"({x} ? 1.0f : 0.0f)" for x in a]
+            elif src == F32:
+                exprs = [f"__float2int_rz({x})" for x in a]
+            else:
+                exprs = [f"(int)({x})" for x in a]
+        elif n.op in ("neg", "not", "abs", "square", "sqrt", "exp", "log", "sin", "cos", "tanh"):
+            exprs = [_unop(n.op, x, n.dtype) for x in elems[n.args[0]]]
+        elif n.op == "where":
+            c, a, b = (elems[j] for j in n.args)
+            exprs = [f"({c[k if len(c) > 1 else 0]} ? {a[k if len(a) > 1 else 0]} : {b[k if len(b) > 1 else 0]})"
+                     for k in range(size)]
+        elif n.op == "index":
+            src_shape = prog.nodes[n.args[0]].shape
+            a = elems[n.args[0]]
+            st = _strides(src_shape)
+            ranges = [[s] if isinstance(s, int) else list(range(s[0], s[1])) for s in n.attr]
+            exprs = []
+            for combo in np.ndindex(*[len(r) for r in ranges]) if ranges else [()]:
+                flat = sum(ranges[d][combo[d]] * st[d] for d in range(len(ranges)))
+                exprs.append(a[flat])
+        elif n.op in ("sum", "mean", "any", "all", "amax", "amin", "norm"):
+            src_shape = prog.nodes[n.args[0]].shape
+            a = elems[n.args[0]]
+            axis = n.attr
+            st = _strides(src_shape)
+            outs = []
+            out_shape = n.shape
+            for combo in (np.ndindex(*out_shape) if out_shape else [()]):
+                idx = list(combo)
+                terms = []
+                for r in range(src_shape[axis]):
+                    full = idx[:axis] + [r] + idx[axis:]
+                    terms.append(a[sum(full[d] * st[d] for d in range(len(src_shape)))])
+                outs.append(_reduce_expr(n.op, terms, n.dtype, lines, f"{v}_{len(outs)}"))
+            exprs = outs
+        else:
+            a = elems[n.args[0]]
+            b = elems[n.args[1]]
+            exprs = [_binop(n.op, a[k if len(a) > 1 else 0], b[k if len(b) > 1 else 0], prog.nodes[n.args[0]].dtype)
+                     for k in range(size)]
+        # every element is materialised once, in node order (torch's operation order)
+        names = []
+        for k, x in enumerate(exprs):
+            nm = f"{v}_{k}" if n.op not in ("sum", "mean", "any", "all", "amax", "amin", "norm") else x
+            if nm != x:
+                lines.append(f"const {ct} {nm} = {x};")
+            names.append(nm)
+        elems.append(names)
+    ret = elems[prog.out][0]
+    rtype = "bool" if prog.kind == "termination" else "float"
+    body = "\n".join("  " + ln for ln in lines)
+    return (f"__device__ __forceinline__ {rtype} {fname}(const UserCtx& c) {{\n{body}\n  return {ret};\n}}\n")
+
+
+def _reduce_expr(op, terms, dtype, lines, acc) -> str:
+    ct = _CT[dtype]
+    if op in ("any", "all"):
+        j = " || " if op == "any" else " && "
+        lines.append(f"const bool {acc} = {j.join(terms) if terms else ('false' if op == 'any' else 'true')};")
+        return acc
+    if not terms:
+        raise UnsupportedTermError(f"user term: {op} over an empty dimension")
+    if op in ("sum", "mean", "norm"):
+        first = terms[0] if op != "norm" else (f"sq({terms[0]})")
+        lines.append(f"{ct} {acc} = {first};")
+        for t in terms[1:]:
+            x = f"sq({t})" if op == "norm" else t
+            lines.append(f"{acc} = add({acc}, {x});" if dtype == F32 else f"{acc} = {acc} + {x};")
+        if op == "mean":
+            lines.append(f"{acc} = fdiv({acc}, {_lit(float(len(terms)), F32)});")
+        if op == "norm":
+            lines.append(f"{acc} = __fsqrt_rn({acc});")
+        return acc
+    fn = ("gfb_user_max" if op == "amax" else "gfb_user_min") if dtype == F32 else ("max" if op == "amax" else "min")
+    lines.append(f"{ct} {acc} = {terms[0]};")
+    for t in terms[1:]:
+        lines.append(f"{acc} = {fn}({acc}, {t});")
+    return acc
+
+
+def device_code(rewards: dict[int, Program], terminations: dict[int, Program]) -> str:
+    """The user-term functions of one table and their dispatchers, keyed by table row."""
+    parts = []
+    for r, prog in sorted(rewards.items()):
+        parts.append(f"/* reward row {r} */\n" + function_body(prog, f"gfb_user_r{r}"))
+    for t, prog in sorted(terminations.items()):
+        parts.append(f"/* termination row {t} */\n" + function_body(prog, f"gfb_user_t{t}"))
+    cases_r = "".join(f"    case {r}: return gfb_user_r{r}(c);\n" for r in sorted(rewards))
+    cases_t = "".join(f"    case {t}: return gfb_user_t{t}(c);\n" for t in sorted(terminations))
+    parts.append("__device__ __forceinline__ float user_reward(int r, const UserCtx& c) {\n  switch (r) {\n"
+                 f"{cases_r}    default: return 0.0f;\n  }}\n}}\n")
+    parts.append("__device__ __forceinline__ bool user_termination(int t, const UserCtx& c) {\n  switch (t) {\n"
+                 f"{cases_t}    default: return false;\n  }}\n}}\n")
+    return "".join(parts)

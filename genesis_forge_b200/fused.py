@@ -18,6 +18,7 @@ buffers (`inject()`), which is how the parity harness feeds the reference's own 
 from __future__ import annotations
 
 import ctypes as C
+import logging
 import math
 import os
 
@@ -40,6 +41,7 @@ except Exception:
 
 
 _F32 = np.float32
+_log = logging.getLogger(__name__)
 
 
 def _f32(x) -> float:
@@ -78,6 +80,10 @@ def asin_tilt_threshold(limit_angle_deg: float) -> float:
 
 
 from .managers.observation import UnsupportedTermError  # noqa: E402  (one class, importable from here too)
+
+
+class UserTermsDemoted(Exception):
+    """Raised before a step's first post-physics launch when its lowered user terms became host callbacks."""
 
 
 def combine_logging(acc: torch.Tensor, n_reward: int, n_termination: int, global_num_envs: int) -> torch.Tensor:
@@ -143,6 +149,8 @@ class FusedStep:
         self._program_ever_pushed = False
         self._injected_bound = object()
         self._spec_tried: set = set()
+        self._spec_ok: dict = {}  # _spec_tag -> a specialised library was attached for it
+        self.first_launch_of_step = False  # set by ManagedEnvironment.step: check lowered user terms first
         self._spec_checked: set = set()  # phase sets looked at since the last re-pack
         self._eval_handle = None  # second library handle for directly called mdp terms
         self._obs_ptrs = None
@@ -220,30 +228,6 @@ class FusedStep:
         self.log_acc = torch.zeros(n_r + n_t + 1, device=dev, dtype=torch.float64)
         self._fixed_command = None
         self._fixed_command_parts = None
-        # terms.  Functions that are not mdp descriptors are user-defined: they stay Python callbacks
-        # whose (N,) result is handed to the kernel as a row of the external-values buffer, and the step
-        # runs in split mode (see ManagedEnvironment._step_split).
-        self.reward_terms = []
-        self.external_rows: list[tuple[str, str, object]] = []  # (kind, name, config item)
-        if self.reward is not None:
-            for name, item in self.reward.cfg.items():
-                opcode = self._opcode_of(item.fn, "reward")
-                if opcode is None or self._other_entity(item, f"reward '{name}'") is not None:
-                    opcode = nat.K["GFB_R_EXTERNAL"]
-                    self.external_rows.append(("reward", name, item))
-                self.reward_terms.append((name, item, opcode))
-        self.termination_terms = []
-        if self.termination is not None:
-            for name, item in self.termination.term_cfg.items():
-                opcode = self._opcode_of(item.fn, "termination")
-                if opcode is None or self._other_entity(item, f"termination '{name}'") is not None:
-                    opcode = nat.K["GFB_T_EXTERNAL"]
-                    self.external_rows.append(("termination", name, item))
-                self.termination_terms.append((name, item, opcode))
-        self.ext_values = None
-        if self.external_rows:
-            self.ext_values = torch.zeros((len(self.external_rows), N), device=dev)
-        self.ext_row = {(kind, name): j for j, (kind, name, _) in enumerate(self.external_rows)}
         # command managers with overridden behaviour are stepped / reset in Python
         from .managers.command import CommandManager, VelocityCommandManager
 
@@ -255,6 +239,37 @@ class FusedStep:
             return True
 
         self.python_commands = [m for m in self.commands if not stock(m)]
+        # terms.  Functions that are not mdp descriptors are user-defined: they stay Python callbacks
+        # whose (N,) result is handed to the kernel as a row of the external-values buffer, and the step
+        # runs in split mode (see ManagedEnvironment._step_split).
+        # With ManagedEnvironment.fuse_user_terms they are first traced into the expression IR (expr.py) and,
+        # where that succeeds, evaluated inside the kernel (GFB_R_USER / GFB_T_USER).
+        self.reward_terms = []
+        self.external_rows: list[tuple[str, str, object]] = []  # (kind, name, config item)
+        self.user_terms: dict = {}  # (kind, name) -> [Program, params live, params traced as constants]
+        self.user_term_refusals: dict = {}  # (kind, name) -> why the term stays a host callback
+        self._user_code = None
+        self._lower_user = bool(getattr(env, "fuse_user_terms", False)) and self._can_specialise_user_terms()
+        if self.reward is not None:
+            for name, item in self.reward.cfg.items():
+                opcode = self._opcode_of(item.fn, "reward")
+                if opcode is None and self._lower_user_term("reward", name, item):
+                    opcode = nat.K["GFB_R_USER"]
+                if opcode is None or self._other_entity(item, f"reward '{name}'") is not None:
+                    opcode = nat.K["GFB_R_EXTERNAL"]
+                    self.external_rows.append(("reward", name, item))
+                self.reward_terms.append((name, item, opcode))
+        self.termination_terms = []
+        if self.termination is not None:
+            for name, item in self.termination.term_cfg.items():
+                opcode = self._opcode_of(item.fn, "termination")
+                if opcode is None and self._lower_user_term("termination", name, item):
+                    opcode = nat.K["GFB_T_USER"]
+                if opcode is None or self._other_entity(item, f"termination '{name}'") is not None:
+                    opcode = nat.K["GFB_T_EXTERNAL"]
+                    self.external_rows.append(("termination", name, item))
+                self.termination_terms.append((name, item, opcode))
+        self._external_values()
         self._has_command_override = any(m._external_controller is not None for m in self.commands)
         self._controller_bound = [False] * len(self.commands)  # GFB_B_COMMAND0+k points at a controller's tensor
         self.any_controller = False
@@ -270,11 +285,136 @@ class FusedStep:
                     width += w
         self.ext_obs_width = width
         self.ext_obs = torch.zeros((N, width), device=dev) if width else None
+        self._plan_launches()
+        self._static_buffers()
+
+    def _external_values(self):
+        """The (J, N) buffer of host-evaluated term values, one row per external reward / termination."""
+        self.ext_values = None
+        if self.external_rows:
+            self.ext_values = torch.zeros((len(self.external_rows), self.N), device=self.device)
+        self.ext_row = {(kind, name): j for j, (kind, name, _) in enumerate(self.external_rows)}
+
+    def _plan_launches(self):
         self.split_mode = bool(self.external_rows or self.python_commands or self.external_obs)
         self.split_plan = self._make_split_plan() if self.split_mode else []
         for _, phases, _ in self.split_plan:
             self._spec_phases.add(phases)
-        self._static_buffers()
+
+    def _can_specialise_user_terms(self) -> bool:
+        """
+        Lowered user terms run in the specialised kernel only, and the library selects a specialisation only
+        for launches that can use TMA: it must exist or be compilable, and the batch must be TMA-eligible.
+        """
+        from . import spec
+
+        return (not spec.disabled() and spec.jit_allowed() and self.N % 4 == 0
+                and os.environ.get("GFB_DISABLE_TMA", "0") != "1")
+
+    # buffers the slab plan may stage or store with TMA (gfb200.cu tma_eligible): 16-byte aligned
+    _TMA_BUFFERS = ("GFB_B_POS", "GFB_B_QUAT", "GFB_B_VEL", "GFB_B_ANG", "GFB_B_DOF_POS", "GFB_B_DOF_VEL",
+                    "GFB_B_DOF_FORCE", "GFB_B_TARGETS", "GFB_B_ENV_ACTIONS", "GFB_B_C_FORCE", "GFB_B_C_POS",
+                    "GFB_B_C_LINK_A", "GFB_B_C_LINK_B", "GFB_B_OBS_EXT0", "GFB_B_EP_SUMS", "GFB_B_BASE_POS",
+                    "GFB_B_BASE_QUAT") + tuple(f"GFB_B_{a}{k}" for a in ("COMMAND", "CONTACTS", "CONTACT_POS")
+                                               for k in range(4))
+
+    def _user_terms_blocked(self) -> str | None:
+        """
+        Why a launch of this split step that evaluates lowered user terms could not run their specialised
+        kernel (None: every one can) -- the library's own conditions (gfb200.cu), checked before the step's
+        first post-physics launch with the step's buffers bound: no specialisation attached for a phase set
+        (compile failure, no JIT), or a buffer the slab plan transfers with TMA that is not 16-byte aligned.
+        (The one launch of a fused step needs no such check: the library refuses it before anything runs.)
+        """
+        if self.dry_run:
+            return None
+        if not self._can_specialise_user_terms():
+            return "the specialised kernel cannot be used (GFB_NO_SPEC, no nvcc, GFB_DISABLE_TMA or num_envs % 4)"
+        K = nat.K
+        buf = self.buffers.buf
+        for name in self._TMA_BUFFERS:
+            ptr = buf[K[name]]
+            if ptr and ptr % 16:
+                return f"{name} is not 16-byte aligned (the specialised kernel's TMA transfers need it)"
+        sets = [p for _, p, _ in self.split_plan] if self.split_mode else [self.step_phases]
+        for phases in sets:
+            phases &= self._phase_mask
+            if not phases & (K["GFB_PHASE_REWARD"] | K["GFB_PHASE_TERMINATION"]):
+                continue
+            self._maybe_specialise(phases)
+            if not self._spec_ok.get(self._spec_tag(phases)):
+                return f"no specialised kernel could be attached for phases {phases:#x}"
+        return None
+
+    def _demote_user_terms(self, why: str):
+        """Every lowered user term becomes a host callback again (split execution), for the rest of the run."""
+        K = nat.K
+        _log.warning("lowered user terms run as host callbacks from now on: %s", why)
+        for key in self.user_terms:
+            self.user_term_refusals[key] = why
+        self.user_terms = {}
+        self._user_code = None
+        self._lower_user = False
+        self.reward_terms = [(n, i, K["GFB_R_EXTERNAL"] if op == K["GFB_R_USER"] else op) for n, i, op in self.reward_terms]
+        self.termination_terms = [(n, i, K["GFB_T_EXTERNAL"] if op == K["GFB_T_USER"] else op)
+                                  for n, i, op in self.termination_terms]
+        self.external_rows = (
+            [("reward", n, i) for n, i, op in self.reward_terms if op == K["GFB_R_EXTERNAL"]]
+            + [("termination", n, i) for n, i, op in self.termination_terms if op == K["GFB_T_EXTERNAL"]])
+        self._external_values()
+        self._set(K["GFB_B_EXT_VALUES"], self.ext_values)
+        self._plan_launches()
+        self._fingerprint = None
+        self._fp_items = None
+        self._program_pushed = False
+        self._spec_checked = set()
+
+    def _lower_user_term(self, kind: str, name: str, item) -> bool:
+        """Trace a user-defined term into the expression IR; False (and the reason kept) when it stays a callback."""
+        if not self._lower_user:
+            return False
+        from . import expr
+
+        try:
+            prog, live = expr.lower_term(self, kind, name, item)
+        except Exception as e:  # noqa: BLE001 - whatever the function does on symbolic inputs, it stays a callback
+            why = str(e) if isinstance(e, UnsupportedTermError) else f"{type(e).__name__} while tracing: {e}"
+            self.user_term_refusals[(kind, name)] = why
+            _log.debug("%s '%s' stays a host callback: %s", kind, name, why)
+            return False
+        self.user_terms[(kind, name)] = [prog, live, None if live else dict(item.params or {}),
+                                         expr.param_kinds(item.params)]
+        return True
+
+    @property
+    def user_code(self) -> str:
+        """Device functions of the lowered user terms for the specialised kernel's header ('' if none)."""
+        if self._user_code is None:
+            from . import expr
+
+            rows = {"reward": {}, "termination": {}}
+            for kind, terms in (("reward", self.reward_terms), ("termination", self.termination_terms)):
+                for row, (name, _, _) in enumerate(terms):
+                    if (kind, name) in self.user_terms:
+                        rows[kind][row] = self.user_terms[(kind, name)][0]
+            self._user_code = expr.device_code(rows["reward"], rows["termination"]) if self.user_terms else ""
+        return self._user_code
+
+    def _user_program(self, kind: str, name: str, item):
+        """The term's Program for its current params (a term traced with constant params is traced again
+        when they change: its expression, and with it the specialised kernel, changes)."""
+        from . import expr
+
+        entry = self.user_terms[(kind, name)]
+        # traced with constant params and they changed, or a live param changed between int and float (its
+        # kernel type, int32 or fp32, was fixed by the trace)
+        changed = entry[2] is not None and dict(item.params or {}) != entry[2]
+        if changed or expr.param_kinds(item.params) != entry[3]:
+            entry[0], live = expr.lower_term(self, kind, name, item)
+            entry[2] = None if live else dict(item.params or {})
+            entry[3] = expr.param_kinds(item.params)
+            self._user_code = None
+        return entry[0]
 
     def _make_split_plan(self) -> list:
         """
@@ -487,6 +627,13 @@ class FusedStep:
                 return k
         raise UnsupportedTermError(f"{what}: contact manager is not registered with this environment")
 
+    def _pack_user_term(self, t, kind: str, name: str, item):
+        prog = self._user_program(kind, name, item)
+        t.i0 = prog.digest()  # structural: part of what a specialised kernel is matched on
+        params = item.params or {}
+        for k, pname in enumerate(prog.params):
+            t.p[k] = params[pname]  # live: a curriculum may change them without a new kernel
+
     def _tilt_threshold(self, limit_angle: float) -> float:
         key = float(limit_angle)
         if key not in self._threshold_cache:
@@ -582,6 +729,9 @@ class FusedStep:
             if opcode == K["GFB_R_EXTERNAL"]:
                 t.ext_col = self.ext_row[("reward", name)]
                 continue
+            if opcode == K["GFB_R_USER"]:
+                self._pack_user_term(t, "reward", name, item)
+                continue
             sig = getattr(item.fn, "gfb_signature", None) or item.fn.__func__.gfb_signature
             p = sig(env, **item.params)
             what = f"reward '{name}'"
@@ -658,6 +808,9 @@ class FusedStep:
             t.op, t.mgr, t.time_out = opcode, -1, 1 if item.time_out else 0
             if opcode == K["GFB_T_EXTERNAL"]:
                 t.i0 = self.ext_row[("termination", name)]
+                continue
+            if opcode == K["GFB_T_USER"]:
+                self._pack_user_term(t, "termination", name, item)
                 continue
             sig = getattr(item.fn, "gfb_signature", None) or item.fn.__func__.gfb_signature
             p = sig(env, **item.params)
@@ -969,7 +1122,7 @@ class FusedStep:
 
         if spec.disabled() or self.dry_run:
             return
-        tag = (self._fingerprint_structure(), self.injected is not None, phases)
+        tag = self._spec_tag(phases)
         if tag in self._spec_tried:
             return
         self._spec_tried.add(tag)
@@ -978,8 +1131,13 @@ class FusedStep:
             if path is not None and path not in self.spec_paths:
                 spec.attach(self, path)
                 self.spec_paths.append(path)
+            self._spec_ok[tag] = path is not None
         except Exception as e:  # a failed specialisation is not fatal: the generic kernel runs
+            self._spec_ok[tag] = False
             print(f"[genesis_forge_b200] kernel specialisation skipped: {e}")
+
+    def _spec_tag(self, phases: int):
+        return (self._fingerprint_structure(), self.injected is not None, phases)
 
     def _fingerprint_structure(self):
         """Cheap proxy for 'the table structure may have changed' (exact matching is done in C)."""
@@ -1046,6 +1204,14 @@ class FusedStep:
         self._injection_buffers()
         self._set_program()
         phases &= self._phase_mask
+        first = self.first_launch_of_step
+        self.first_launch_of_step = False
+        if first and self.user_terms and self.split_mode:
+            # a later launch of the split step evaluates the lowered terms: check before anything is launched
+            why = self._user_terms_blocked()
+            if why is not None:
+                self._demote_user_terms(why)
+                raise UserTermsDemoted(why)
         if phases in self._spec_phases:
             self._maybe_specialise(phases)
         if phases & self._PHASE_REWARD:
@@ -1056,6 +1222,12 @@ class FusedStep:
         stream = self._stream()
         rc = self.lib.gfb_post_physics(self._h, self._buffers_ref, phases, stream)
         if rc:
+            if first and rc == nat.K["GFB_ERR_UNSUPPORTED"] and self.user_terms and not self.split_mode:
+                # the one launch of the fused step was refused before anything ran: no specialised kernel
+                # matched the table with its lowered terms (not attached, or the launch cannot use TMA)
+                why = self.lib.gfb_last_error(self._h).decode()
+                self._demote_user_terms(why)
+                raise UserTermsDemoted(why)
             self.handle.check(rc, "gfb_post_physics")
         if not read_report:
             return None
@@ -1150,6 +1322,10 @@ class FusedStep:
         terms given an `entity_manager` use the base pose cached by the last step, the others the
         entity's current pose; contact terms read the last step's net forces.
         """
+        from .expr import ExprMode
+
+        if isinstance(self.env._tracing, ExprMode):
+            raise UnsupportedTermError(f"user term: a direct call of the stock term {fn.__name__} is not inlined")
         if self.dry_run:
             raise nat.NativeLibraryError("direct evaluation of mdp terms needs a CUDA device (dry-run handle)")
         K = nat.K

@@ -26,7 +26,7 @@ import torch
 
 from . import _native as nat
 from ._gs import gs
-from .fused import FusedStep, UnsupportedTermError, combine_logging, make_obs_dict
+from .fused import FusedStep, UnsupportedTermError, UserTermsDemoted, combine_logging, make_obs_dict
 from .genesis_env import GenesisEnv
 from .managers.base import BaseManager, ManagerType
 
@@ -39,6 +39,12 @@ class ManagedEnvironment(GenesisEnv):
     # GFB_COPY_OBSERVATIONS=1 in the environment -- to get a private copy per step (one extra
     # (N, O*H) device copy).
     copy_observations = os.environ.get("GFB_COPY_OBSERVATIONS", "0") == "1"
+    # User-defined reward / termination functions are host callbacks between separate kernel launches
+    # (split execution).  With this set to True -- or GFB_FUSE_USER_TERMS=1 in the environment -- build()
+    # traces them into a small expression IR (expr.py) and the ones that lower run inside the specialised
+    # post-physics kernel next to the stock terms; a table without other host callbacks is then one launch
+    # per step again.  Terms the IR does not cover stay callbacks (FusedStep.user_term_refusals says why).
+    fuse_user_terms = os.environ.get("GFB_FUSE_USER_TERMS", "0") == "1"
 
     def __init__(
         self,
@@ -132,6 +138,8 @@ class ManagedEnvironment(GenesisEnv):
         """Manager getters call this: a tagged placeholder while tracing, the real value otherwise."""
         if self._tracing is None:
             return compute()
+        if not isinstance(self._tracing, dict):  # a user term traced into the expression IR (expr.py)
+            return self._tracing.source(key, compute)
         if key not in self._tracing:
             self._tracing[key] = torch.empty((0, self._trace_width(key)))
         return self._tracing[key]
@@ -229,12 +237,18 @@ class ManagedEnvironment(GenesisEnv):
         self.scene.step()
         for entity_manager in fused.secondary_entities:  # (the first one's step is the kernel's entity phase)
             entity_manager.step()
-        if fused.split_mode:
+        # lowered user terms are checked before the first post-physics launch; if their specialised kernel
+        # cannot run, they become host callbacks and the step runs split (FusedStep._demote_user_terms)
+        fused.first_launch_of_step = True
+        try:
+            if fused.split_mode:
+                return self._finish_step_split()
+            # two-stage report: the rank's own reset count first -- on a sharded env the kernel's last block
+            # then still waits for the slowest peer's logging partials, and that wait now overlaps the reset
+            # fan-out and the re-observation launch below instead of preceding them
+            n_reset = fused.post_physics_local(fused.step_phases)
+        except UserTermsDemoted:
             return self._finish_step_split()
-        # two-stage report: the rank's own reset count first -- on a sharded env the kernel's last block
-        # then still waits for the slowest peer's logging partials, and that wait now overlaps the reset
-        # fan-out and the re-observation launch below instead of preceding them
-        n_reset = fused.post_physics_local(fused.step_phases)
         if n_reset > 0:
             reset_idx = fused.reset_idx[:n_reset]
             self._host_reset(reset_idx)

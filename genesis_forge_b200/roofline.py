@@ -47,6 +47,16 @@ def _program_facts(fused):
         "targets": K["GFB_O_TARGETS"] in srcs,
         "action_rate": K["GFB_R_ACTION_RATE"] in ops,
     }
+    # lowered user-defined terms (expr.py): each distinct array they read counts once, like the stock
+    # terms' (contact forces / air time are this kernel's own outputs, actions and commands always counted)
+    user = {"vel": "vel", "lin_vel_b": "vel", "ang": "ang", "ang_vel_b": "ang", "pos": "pos",
+            "dof_pos": "dof_pos", "dof_vel": "dof_vel", "targets": "targets"}
+    for (kind, name), entry in getattr(fused, "user_terms", {}).items():
+        if kind == "reward" and fused.reward.cfg[name].weight == 0.0:
+            continue
+        for key in entry[0].sources():
+            if key[0] in user:
+                uses[user[key[0]]] = True
     contact_in = contact_out = air = 0
     if P.n_contact > 0:
         C, L = P.n_contact_slots, P.n_links_total

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define GFB_ABI_VERSION 11
+#define GFB_ABI_VERSION 12
 
 /* ---- limits ------------------------------------------------------------------------------- */
 #define GFB_MAX_DOFS 32
@@ -138,7 +138,10 @@ typedef enum {
   GFB_R_CONTACT_FORCE,       /* rewards.py:413-428 p0=threshold */
   GFB_R_FEET_AIR_TIME,       /* rewards.py:431-469 p0=time_threshold p1=max-thr p2=dt+margin; i0=command mgr or -1 */
   GFB_R_FEET_SLIDE,          /* rewards.py:472-504 */
-  GFB_R_EXTERNAL             /* value column supplied by the host (user-defined term) */
+  GFB_R_EXTERNAL,            /* value column supplied by the host (user-defined term) */
+  GFB_R_USER                 /* user-defined term lowered to device code (genesis_forge_b200/expr.py): i0 = identity
+                                of its expression, p = its live scalar params.  Only a specialised kernel generated
+                                for that expression evaluates it; the generic kernel refuses the launch. */
 } gfb_reward_op;
 
 typedef enum {
@@ -150,7 +153,8 @@ typedef enum {
   GFB_T_HAS_CONTACT,         /* terminations.py:139-155 p0=threshold, i0=min_contacts */
   GFB_T_CONTACT_FORCE,       /* terminations.py:158-172 p0=threshold */
   GFB_T_CONTACT_FORCE_GRACE, /* terminations.py:175-205 p0=threshold, i0=grace */
-  GFB_T_EXTERNAL             /* host-evaluated term: fires where row i0 of GFB_B_EXT_VALUES is non-zero */
+  GFB_T_EXTERNAL,            /* host-evaluated term: fires where row i0 of GFB_B_EXT_VALUES is non-zero */
+  GFB_T_USER                 /* lowered user-defined term, as GFB_R_USER */
 } gfb_termination_op;
 
 /* observation column sources (mdp/observations.py:16-193 and the manager getters they wrap) */
