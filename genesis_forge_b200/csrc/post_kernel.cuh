@@ -151,8 +151,20 @@ struct UserCtx {
 };
 
 #if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
+// NaN propagating; on a tie (+0 / -0) the second operand.  amax / amin pass (element, accumulator), so a
+// row's first element is kept on a tie, as torch-CPU does.
 __device__ __forceinline__ float gfb_user_min(float a, float b) { return (a < b || a != a) ? a : b; }
 __device__ __forceinline__ float gfb_user_max(float a, float b) { return (a > b || a != a) ? a : b; }
+// torch.clamp: x is kept on a tie; a NaN bound propagates, except a NaN Python-scalar bound given alone
+// (a Python float or a live param), which torch-CPU ignores
+__device__ __forceinline__ float gfb_user_clamp_lo(float x, float lo) { return (x < lo || lo != lo) ? lo : x; }
+__device__ __forceinline__ float gfb_user_clamp_hi(float x, float hi) { return (x > hi || hi != hi) ? hi : x; }
+__device__ __forceinline__ float gfb_user_clamp_lo_scalar(float x, float lo) { return x < lo ? lo : x; }
+__device__ __forceinline__ float gfb_user_clamp_hi_scalar(float x, float hi) { return x > hi ? hi : x; }
+// float -> int32 as torch-CPU (x86 cvttss2si): truncation; NaN, +-Inf and |x| >= 2^31 give INT_MIN
+__device__ __forceinline__ int gfb_user_f2i(float x) {
+  return (x > -2147483904.0f && x < 2147483648.0f) ? __float2int_rz(x) : (int)0x80000000;
+}
 __device__ __forceinline__ int gfb_user_mod(int a, int b) {  // torch's remainder: the sign of the divisor
   const int r = a % b;
   return (r != 0 && ((r < 0) != (b < 0))) ? r + b : r;

@@ -37,6 +37,8 @@ F32, I32, BOOL = "f32", "i32", "bool"
 _RANK = {BOOL: 0, I32: 1, F32: 2}
 MAX_CONST_VEC = 32  # GFB_MAX_DOFS: small constant vectors (per-joint limits, gains) are folded in
 MAX_LIVE_PARAMS = 4  # gfb_reward_term.p / gfb_termination_term.p
+# bumped whenever `function_body` emits different code for the same IR: the digest changes with it
+CODEGEN_REVISION = 2
 
 
 class _ParamControlFlow(Exception):
@@ -73,8 +75,10 @@ class Program:
         return head + "\n".join(n.text(i) for i, n in enumerate(self.nodes))
 
     def digest(self) -> int:
-        """31-bit identity of the expression (stored in the term's structural `i0` field)."""
-        return int.from_bytes(hashlib.sha1(self.text().encode()).digest()[:4], "little") & 0x7FFFFFFF
+        """31-bit identity of the expression and of the code `function_body` emits for it (stored in the
+        term's structural `i0` field)."""
+        text = f"codegen {CODEGEN_REVISION}\n" + self.text()
+        return int.from_bytes(hashlib.sha1(text.encode()).digest()[:4], "little") & 0x7FFFFFFF
 
     def sources(self) -> list[tuple]:
         return [n.attr for n in self.nodes if n.op == "src"]
@@ -245,9 +249,14 @@ class Sym:
 
     def to(self, *args, **kwargs):
         dtype = kwargs.get("dtype") or next((a for a in args if isinstance(a, torch.dtype)), None)
-        return self._tr.cast(self, _dtype_of(dtype)) if dtype is not None else self
+        return self._cast_to(dtype) if dtype is not None else self
 
     def type(self, dtype):
+        return self._cast_to(dtype)
+
+    def _cast_to(self, dtype):
+        if dtype is torch.int64 and self.dtype_ == F32:  # torch keeps |x| >= 2^31; the kernel's int is 32-bit
+            raise UnsupportedTermError("user term: float -> int64 cast (int32 holds a different result)")
         return self._tr.cast(self, _dtype_of(dtype))
 
     def __getitem__(self, key):
@@ -391,6 +400,8 @@ class Tracer:
             dt = F32  # true division
         if op == "mod" and dt != I32:
             raise UnsupportedTermError("user term: '%' is supported for integers only")
+        if op == "mod" and b._node.op == "const" and b._node.attr == 0:
+            raise UnsupportedTermError("user term: '%' by the constant 0 (torch raises ZeroDivisionError)")
         if op in ("add", "sub", "mul", "minimum", "maximum") and dt == BOOL:
             raise UnsupportedTermError(f"user term: '{op}' of two bool values")
         ca, cb = self.cast(a, dt), self.cast(b, dt)
@@ -421,15 +432,18 @@ class Tracer:
         if x.dtype_ == BOOL:
             raise UnsupportedTermError("user term: clamp() of a bool value")
         out = x
-        # torch.clamp(x, lo, hi) == min(max(x, lo), hi), NaN propagating
-        if lo is not None:
-            lo = self.lift(lo)
-            dt = _promote(out, lo)
-            out = self.add("clamp_lo", (self.cast(out, dt)._id, self.cast(lo, dt)._id), None, _bshape(out, lo, "clamp"), dt)
-        if hi is not None:
-            hi = self.lift(hi)
-            dt = _promote(out, hi)
-            out = self.add("clamp_hi", (self.cast(out, dt)._id, self.cast(hi, dt)._id), None, _bshape(out, hi, "clamp"), dt)
+        # torch.clamp(x, lo, hi) == min(max(x, lo), hi): x kept on a tie, NaN in x propagating.  A NaN bound
+        # propagates, except that torch-CPU ignores it when it is the only bound and a Python scalar (a live
+        # param is one): attr "scalar"
+        for op, bound in (("clamp_lo", lo), ("clamp_hi", hi)):
+            if bound is None:
+                continue
+            scalar = (lo is None or hi is None) and (isinstance(bound, (int, float, np.generic))
+                                                     or (isinstance(bound, Sym) and bound._node.op == "param"))
+            bound = self.lift(bound)
+            dt = _promote(out, bound)
+            out = self.add(op, (self.cast(out, dt)._id, self.cast(bound, dt)._id), "scalar" if scalar else None,
+                           _bshape(out, bound, "clamp"), dt)
         return out
 
     def reduce(self, kind: str, x, dim, keepdim=False) -> Sym:
@@ -854,7 +868,7 @@ def _strides(shape):
     return list(reversed(out))
 
 
-def _binop(op, a, b, dtype):
+def _binop(op, a, b, dtype, attr=None):
     if dtype == F32:
         arith = {"add": f"add({a}, {b})", "sub": f"sub({a}, {b})", "mul": f"mul({a}, {b})", "div": f"fdiv({a}, {b})"}
     else:
@@ -863,8 +877,10 @@ def _binop(op, a, b, dtype):
         return arith[op]
     if op == "mod":
         return f"gfb_user_mod({a}, {b})"
+    if op in ("clamp_lo", "clamp_hi") and dtype == F32:
+        return f"gfb_user_{op}{'_scalar' if attr == 'scalar' else ''}({a}, {b})"
     if op in ("minimum", "clamp_hi"):
-        # NaN propagates (torch.minimum / torch.clamp)
+        # NaN propagates (torch.minimum)
         return f"gfb_user_min({a}, {b})" if dtype == F32 else f"min({a}, {b})"
     if op in ("maximum", "clamp_lo"):
         return f"gfb_user_max({a}, {b})" if dtype == F32 else f"max({a}, {b})"
@@ -918,7 +934,7 @@ def function_body(prog: Program, fname: str) -> str:
             elif n.dtype == F32:
                 exprs = [f"({x} ? 1.0f : 0.0f)" for x in a]
             elif src == F32:
-                exprs = [f"__float2int_rz({x})" for x in a]
+                exprs = [f"gfb_user_f2i({x})" for x in a]
             else:
                 exprs = [f"(int)({x})" for x in a]
         elif n.op in ("neg", "not", "abs", "square", "sqrt", "exp", "log", "sin", "cos", "tanh"):
@@ -954,8 +970,8 @@ def function_body(prog: Program, fname: str) -> str:
         else:
             a = elems[n.args[0]]
             b = elems[n.args[1]]
-            exprs = [_binop(n.op, a[k if len(a) > 1 else 0], b[k if len(b) > 1 else 0], prog.nodes[n.args[0]].dtype)
-                     for k in range(size)]
+            exprs = [_binop(n.op, a[k if len(a) > 1 else 0], b[k if len(b) > 1 else 0], prog.nodes[n.args[0]].dtype,
+                            n.attr) for k in range(size)]
         # every element is materialised once, in node order (torch's operation order)
         names = []
         for k, x in enumerate(exprs):
@@ -978,8 +994,13 @@ def _reduce_expr(op, terms, dtype, lines, acc) -> str:
         return acc
     if not terms:
         raise UnsupportedTermError(f"user term: {op} over an empty dimension")
+    if op == "norm" and len(terms) <= 3:  # torch-CPU: |x|, and the fma chains of device_utils.cuh
+        fn = {1: "fabsf", 2: "norm2", 3: "norm3"}[len(terms)]
+        lines.append(f"const float {acc} = {fn}({', '.join(terms)});")
+        return acc
     if op in ("sum", "mean", "norm"):
-        first = terms[0] if op != "norm" else (f"sq({terms[0]})")
+        # torch's sum starts from +0 (a row of -0 sums to +0)
+        first = f"sq({terms[0]})" if op == "norm" else (f"add(0.0f, {terms[0]})" if dtype == F32 else terms[0])
         lines.append(f"{ct} {acc} = {first};")
         for t in terms[1:]:
             x = f"sq({t})" if op == "norm" else t
@@ -992,7 +1013,7 @@ def _reduce_expr(op, terms, dtype, lines, acc) -> str:
     fn = ("gfb_user_max" if op == "amax" else "gfb_user_min") if dtype == F32 else ("max" if op == "amax" else "min")
     lines.append(f"{ct} {acc} = {terms[0]};")
     for t in terms[1:]:
-        lines.append(f"{acc} = {fn}({acc}, {t});")
+        lines.append(f"{acc} = {fn}({t}, {acc});")  # (on a tie the accumulator: the first element is kept)
     return acc
 
 
