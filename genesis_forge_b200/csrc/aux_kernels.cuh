@@ -3,6 +3,7 @@
 #pragma once
 #include "device_utils.cuh"
 #include "plan.h"
+#include "tail_math.cuh"
 
 namespace gfb {
 
@@ -169,16 +170,16 @@ __global__ void __launch_bounds__(TILE) action_kernel(const __grid_constant__ Ac
 // envs reset: it runs while the host wakes up and walks through its reset fan-out, and whatever
 // reads the list (engine setters, the re-observation) is enqueued behind it.
 // Every block derives the number of reset envs before its own range by summing the population counts
-// of all earlier words (the mask array is 128 KB at 1M envs: L2 hits), then scans its range.
+// of all earlier words (the mask array is 128 KB at 1M envs: L2 hits), then scans its range.  The
+// launch geometry (tail_math.cuh compact_geometry) starts every block inside the array.
 // ---------------------------------------------------------------------------------------------
-constexpr int CMP_THREADS = 256;
-
 __global__ void __launch_bounds__(CMP_THREADS) compact_kernel(const uint32_t* __restrict__ words, int n_words,
                                                                int words_per_block, int64_t* __restrict__ out) {
   __shared__ int s_warp[CMP_THREADS / 32];
   __shared__ int s_base;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int w0 = blockIdx.x * words_per_block;
+  if (w0 >= n_words) return;  // (block-uniform)
   const int w1 = min(w0 + words_per_block, n_words);
   // reset envs in all words before this block's range (w0 is a multiple of 256: 16-byte loads)
   int before = 0;

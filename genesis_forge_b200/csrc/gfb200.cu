@@ -560,7 +560,11 @@ int build_plan(gfb_handle* h, const gfb_buffers& b, uint32_t phases, int tile, i
   plan.stage_words = (cursor + 31) & ~31;
   plan.n_stages = n_stages;
   plan.cols_off = plan.stage_words * n_stages;
-  plan.smem_words = plan.cols_off + align4(plan.table_words);
+  // behind the table: the reward terms' exact sums of a RESET launch, 160 bytes a term (post_kernel.cuh)
+  plan.rew_acc_off = plan.cols_off + align4(plan.table_words);
+  const bool reward_log = h->prog.head.n_reward > 0 && !(h->prog.head.manager_flags & GFB_MF_REWARD_DISABLED);
+  const int acc_words = (phases & GFB_PHASE_RESET) && reward_log ? h->prog.head.n_reward * XS_WORDS * 4 : 0;
+  plan.smem_words = plan.rew_acc_off + acc_words;
   if (const char* pad = getenv("GFB_PAD_SMEM_KB"))  // occupancy experiments: unused shared memory per block
     plan.smem_words += atoi(pad) * 256;
   return GFB_OK;
@@ -741,12 +745,12 @@ int gfb_create(int32_t num_envs, int32_t device, gfb_handle** out) {
   CUDA_TRY(cudaMalloc(&h->scratch.tile_bits, (size_t)(nt + 8) * sizeof(uint32_t)));  // (+ the tail slab's padding)
   CUDA_TRY(cudaMemset(h->scratch.tile_bits, 0, (size_t)(nt + 8) * sizeof(uint32_t)));
   CUDA_TRY(cudaMalloc(&h->scratch.term_count, GFB_MAX_TERMINATION_TERMS * sizeof(int32_t)));
-  CUDA_TRY(cudaMalloc(&h->scratch.rew_acc, GFB_MAX_REWARD_TERMS * sizeof(unsigned long long)));
+  CUDA_TRY(cudaMalloc(&h->scratch.rew_acc, GFB_MAX_REWARD_TERMS * XS_WORDS * sizeof(unsigned long long)));
   CUDA_TRY(cudaMalloc(&h->scratch.rew_flags, GFB_MAX_REWARD_TERMS * sizeof(uint32_t)));
   CUDA_TRY(cudaMalloc(&h->scratch.counters, CTR_COUNT * sizeof(uint32_t)));
   CUDA_TRY(cudaMalloc(&h->scratch.status, sizeof(uint32_t)));
   CUDA_TRY(cudaMemset(h->scratch.term_count, 0, GFB_MAX_TERMINATION_TERMS * sizeof(int32_t)));
-  CUDA_TRY(cudaMemset(h->scratch.rew_acc, 0, GFB_MAX_REWARD_TERMS * sizeof(unsigned long long)));
+  CUDA_TRY(cudaMemset(h->scratch.rew_acc, 0, GFB_MAX_REWARD_TERMS * XS_WORDS * sizeof(unsigned long long)));
   CUDA_TRY(cudaMemset(h->scratch.rew_flags, 0, GFB_MAX_REWARD_TERMS * sizeof(uint32_t)));
   CUDA_TRY(cudaMemset(h->scratch.counters, 0, CTR_COUNT * sizeof(uint32_t)));
   CUDA_TRY(cudaMemset(h->scratch.status, 0, sizeof(uint32_t)));
@@ -1105,10 +1109,9 @@ int gfb_post_physics(gfb_handle* h, const gfb_buffers* b, uint32_t phases, void*
     // the ascending index list from the slabs' reset masks: behind the post kernel, which has told the
     // host the counts by then -- this runs while the host wakes up (see compact_kernel)
     const int n_words = n_tiles * (tile / 32);
-    const int n_blocks = std::max(1, std::min(128, (n_words + CMP_THREADS - 1) / CMP_THREADS));
-    const int words_per_block = ((n_words + n_blocks - 1) / n_blocks + CMP_THREADS - 1) / CMP_THREADS * CMP_THREADS;
+    const CompactGeometry g = compact_geometry(n_words);
     cudaEvent_t cmp_end = aux_begin(h, 0, stream);
-    compact_kernel<<<n_blocks, CMP_THREADS, 0, stream>>>(h->scratch.tile_bits, n_words, words_per_block,
+    compact_kernel<<<g.n_blocks, CMP_THREADS, 0, stream>>>(h->scratch.tile_bits, n_words, g.words_per_block,
                                                          static_cast<int64_t*>(b->buf[GFB_B_RESET_IDX]));
     CUDA_TRY(cudaGetLastError());
     if (cmp_end) cudaEventRecord(cmp_end, stream);

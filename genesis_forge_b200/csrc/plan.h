@@ -83,7 +83,8 @@ struct Plan {
   int32_t grp_mixed_count[GFB_MAX_OBS_GROUPS];
   int32_t stage_words;                         // shared words of one ring stage
   int32_t n_stages;                            // 2 = prefetch ring, 1 = single buffer
-  int32_t smem_words;
+  int32_t rew_acc_off;                         // exact episode-quotient sums (RESET launches, post_kernel.cuh)
+  int32_t smem_words;                          // (last: spec.py reads it from the end of the plan)
 };
 
 // Logging exchange between the ranks of one NVLink domain (gfb_peer_connect): every rank owns an
@@ -117,7 +118,7 @@ enum : int {
 struct Scratch {
   uint32_t* tile_bits;             // (ceil(N / 32) words, in env order) reset masks, 32 envs per word
   int32_t* term_count;             // (GFB_MAX_TERMINATION_TERMS) fire counts since the last report
-  unsigned long long* rew_acc;     // (GFB_MAX_REWARD_TERMS) signed 64-bit fixed-point sums (tail.cuh)
+  unsigned long long* rew_acc;     // (GFB_MAX_REWARD_TERMS x XS_WORDS) exact sums (tail_math.cuh)
   uint32_t* rew_flags;             // (GFB_MAX_REWARD_TERMS) non-finite episode quotients seen
   uint32_t* counters;              // CTR_*
   uint32_t* status;                // sticky status bits

@@ -185,7 +185,6 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
   extern __shared__ __align__(128) float Sbase[];
   __shared__ __align__(8) uint64_t bars[3];  // [0] slab loads, [1] late load group, [2] prefetched arrays
   __shared__ int32_t s_term_count[GFB_MAX_TERMINATION_TERMS];
-  __shared__ unsigned long long s_rew_acc[GFB_MAX_REWARD_TERMS];  // fixed-point sums of the slab (tail.cuh)
   __shared__ uint32_t s_rew_flags[GFB_MAX_REWARD_TERMS];
   __shared__ uint32_t s_reset_bits[TILE / 32];
   __shared__ uint32_t s_status;
@@ -234,8 +233,14 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
   const Philox rng(P.rng_seed);
   // reset_reward_log: the reset phase logs and clears the episode sums (reward manager enabled)
   const bool reward_log = SP.n_reward > 0 && !(SP.manager_flags & GFB_MF_REWARD_DISABLED);
+  // exact sums of the episode quotients (tail_math.cuh), in the plan's shared memory (RESET launches): per
+  // slab two 32-bit counters of 16-bit pieces per word, per block one 64-bit word (word i: thread i)
+  const int n_acc_words = (ph & GFB_PHASE_RESET) && reward_log ? SP.n_reward * XS_WORDS : 0;
+  int* const s_rew_acc = reinterpret_cast<int*>(Sbase + plan.rew_acc_off);
+  unsigned long long* const s_rew_blk = reinterpret_cast<unsigned long long*>(s_rew_acc + 2 * n_acc_words);
 
   if (tid == 0) s_arrived = 0;
+  for (int i = tid; i < n_acc_words; i += TILE) s_rew_blk[i] = 0ull;
   // barrier setup in straight-line code (thread 0 selected by predicate: uniform-datapath rule)
   mbar_init(tid == 0, &bars[0], 1);
   mbar_init(tid == 0, &bars[1], 1);
@@ -271,10 +276,8 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
 
   if (tid < GFB_MAX_TERMINATION_TERMS) s_term_count[tid] = 0;
   if (tid == 0) s_status = 0;
-  for (int i = tid; i < GFB_MAX_REWARD_TERMS; i += TILE) {
-    s_rew_acc[i] = 0ull;
-    s_rew_flags[i] = 0u;
-  }
+  for (int i = tid; i < 2 * n_acc_words; i += TILE) s_rew_acc[i] = 0;
+  if (tid < GFB_MAX_REWARD_TERMS) s_rew_flags[tid] = 0u;
 
   // ------------------------------------------------------------------------------------------
   // slab loads: every staged array and the episode-sum rows are single cp.async.bulk transfers;
@@ -958,7 +961,9 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
           for (int k = 0; k < SP.contact[m].n_links * 4; ++k) st[plan.st_air[m] + k] = 0.0f;
     }
     // reward_manager.py:197-222: per-term episode mean over the reset envs, then clear.  Resets are
-    // sparse: every reset env adds its quotient to the slab's exact fixed-point sums (tail.cuh).
+    // sparse: every reset env adds its quotient to the slab's exact sums (tail_math.cuh): two words, as
+    // four native 32-bit shared atomics without a return value (a 64-bit one is a compare-and-swap loop,
+    // whose latency the reset lane's slab waits for at the next barrier).
     if (reset) {
       if (reward_log) {
         GFB_UNROLL_TERMS
@@ -966,8 +971,16 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
           float* sum = S + plan.sums_off + r * TILE + tid;
           if (P.reward[r].weight != 0.0f) {
             uint32_t fl = 0;
-            const long long f = to_fixed(fdiv(*sum, ep_secs), fl);
-            if (f) atomicAdd(&s_rew_acc[r], (unsigned long long)f);
+            long long lo, hi;
+            const int k = xs_split(fdiv(*sum, ep_secs), lo, hi, fl);
+            int* acc = s_rew_acc + (r * XS_WORDS + k) * 2;
+            int p0, p1, p2, p3;
+            xs_pieces(lo, p0, p1);
+            xs_pieces(hi, p2, p3);
+            if (p0) atomicAdd(acc, p0);
+            if (p1) atomicAdd(acc + 1, p1);
+            if (p2) atomicAdd(acc + 2, p2);
+            if (p3) atomicAdd(acc + 3, p3);
             if (fl) atomicOr(&s_rew_flags[r], fl);
           }
           *sum = 0.0f;
@@ -1055,11 +1068,14 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
   }
 
   // ------------------------------------------------------------------------------------------
-  // the slab's logging partials -> the launch's accumulators (integer atomics: order-independent)
+  // the slab's logging partials -> the block's sums (plain adds: thread i owns word i), flags -> the launch's
+  // (rare; integer atomics: order-independent).  The block adds its sums to the launch's when it leaves: one
+  // atomic per word and block instead of per slab, which would queue up behind each other in L2.
   // ------------------------------------------------------------------------------------------
-  if ((ph & GFB_PHASE_RESET) && reward_log && tid < SP.n_reward) {
-    if (s_rew_acc[tid]) atomicAdd(K.s.rew_acc + tid, s_rew_acc[tid]);  // (no return value: RED, fire and forget)
-    if (s_rew_flags[tid]) atomicOr(K.s.rew_flags + tid, s_rew_flags[tid]);
+  if ((ph & GFB_PHASE_RESET) && reward_log) {
+    for (int i = tid; i < n_acc_words; i += TILE)
+      s_rew_blk[i] += (unsigned long long)xs_join(s_rew_acc[2 * i], s_rew_acc[2 * i + 1]);
+    if (tid < SP.n_reward && s_rew_flags[tid]) atomicOr(K.s.rew_flags + tid, s_rew_flags[tid]);
   }
   if (!(ph & (GFB_PHASE_TERMINATION | GFB_PHASE_RESET)) && tid == 0 && s_status) atomicOr(K.s.status, s_status);
 
@@ -1198,6 +1214,9 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
   }  // slab loop
 
   if (use_tma && warp == 0) bulk_wait_all();
+  if ((ph & GFB_PHASE_RESET) && reward_log)  // only the nonzero words (no return value: RED, fire and forget)
+    for (int i = tid; i < n_acc_words; i += TILE)
+      if (s_rew_blk[i]) atomicAdd(K.s.rew_acc + i, s_rew_blk[i]);
 
   // ------------------------------------------------------------------------------------------
   // the last block to leave turns the reward sums into logged means and re-arms the counters

@@ -3,8 +3,13 @@
 //
 //   * termination fire counts and the number of reset envs are integer atomics, fire and forget.
 //   * the episode means of the reward terms over the reset envs (reward_manager.py:205-216) are
-//     accumulated as 64-bit fixed-point sums (integer atomics commute, so the logged values are
-//     run-to-run deterministic) and turned into means by the last block to leave the kernel.
+//     accumulated as exact integer sums of the fp32 quotients (tail_math.cuh: XS_WORDS words per term;
+//     integer atomics commute, so the logged values are run-to-run deterministic) and turned into means
+//     by the last block to leave the kernel.  Contract of a logged mean, S the exact sum of the n
+//     quotients: NaN if a quotient is NaN or both infinities occur, else an infinite quotient; +-Inf if
+//     S rounded to fp32 overflows (as an fp32 sum of the same values does); else S / n within 1 fp32 ulp,
+//     +0 for a zero sum.  Sharded over ranks, each rank's S travels as a double and the doubles are
+//     summed in rank order: deterministic, but within W * 2^-53 * sum|q| rather than exact.
 //   * that block also writes the step report into the host's mapped memory and, last, its sequence
 //     word, on which the host spins.
 //   * envs sharded over ranks: both reductions are exchanged over NVLink peer memory (plan.h PeerInbox).
@@ -26,6 +31,7 @@
 #pragma once
 #include "device_utils.cuh"
 #include "plan.h"
+#include "tail_math.cuh"
 
 namespace gfb {
 
@@ -54,33 +60,6 @@ __device__ __forceinline__ unsigned long long global_timer_ns() {
   unsigned long long t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
-}
-
-// ---------------------------------------------------------------------------------------------
-// order-independent sums of fp32 values: signed 64-bit fixed point with 32 fractional bits.
-// Integer additions commute, so the per-slab and per-launch sums can be fire-and-forget atomics (RED,
-// no return value -- a returning atomic costs the issuing warp an L2 round trip, and its slab waits
-// for it at the next block barrier) and the logged means are still run-to-run deterministic.  Each
-// addend is rounded to 2^-32 (2.3e-10, far below the fp32 resolution of the logged mean); the sum
-// holds +-2^31.
-// ---------------------------------------------------------------------------------------------
-constexpr uint32_t FX_NAN = 1u, FX_POS_INF = 2u, FX_NEG_INF = 4u;
-__device__ __forceinline__ long long to_fixed(float q, uint32_t& flags) {
-  if (q != q) {
-    flags |= FX_NAN;
-    return 0ll;
-  }
-  if (fabsf(q) >= 1048576.0f) {  // 2^20 per addend (x 2^11 reset envs per slab, x 2^20 slabs): treated as infinite
-    flags |= q > 0.0f ? FX_POS_INF : FX_NEG_INF;
-    return 0ll;
-  }
-  return __float2ll_rn(__fmul_rn(q, 4294967296.0f));
-}
-__device__ __forceinline__ double fixed_to_double(long long v, uint32_t flags) {
-  if ((flags & FX_NAN) || ((flags & FX_POS_INF) && (flags & FX_NEG_INF))) return __longlong_as_double(0x7ff8000000000000ll);
-  if (flags & FX_POS_INF) return __longlong_as_double(0x7ff0000000000000ll);
-  if (flags & FX_NEG_INF) return __longlong_as_double((long long)0xfff0000000000000ull);
-  return (double)v * 2.3283064365386963e-10;  // 2^-32
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -143,11 +122,13 @@ __device__ __forceinline__ void finalize_step(const KParams& K, int lane) {
   const int n_reset = (int)ld_acquire_gpu_u32(sc.counters + CTR_TOTAL_RESET);  // every slab has added its share
   const int count = lane < n_t ? atomicExch(sc.term_count + lane, 0) : 0;
   uint32_t status = lane == 0 ? atomicExch(sc.status, 0u) : 0u;
-  const long long acc = lane < n_r ? (long long)atomicExch(sc.rew_acc + lane, 0ull) : 0ll;
+  long long acc[XS_WORDS];  // lane = reward term
+#pragma unroll
+  for (int k = 0; k < XS_WORDS; ++k) acc[k] = lane < n_r ? (long long)atomicExch(sc.rew_acc + lane * XS_WORDS + k, 0ull) : 0ll;
   const uint32_t acc_flags = lane < n_r ? atomicExch(sc.rew_flags + lane, 0u) : 0u;
 
   double counts = lane < n_t ? (double)count : (lane == n_t ? (double)n_reset : 0.0);  // lane n_t: reset envs
-  double sum = lane < n_r ? fixed_to_double(acc, acc_flags) : 0.0;
+  double sum = lane < n_r ? xs_to_double(acc, acc_flags) : 0.0;
   double* log_acc = GFB_BUF(double, GFB_B_LOG_ACC);
   float* log_out = GFB_BUF(float, GFB_B_LOG_OUT);
   if (log_acc) {  // local partials (what the NCCL fallback path all-reduces)
@@ -181,7 +162,7 @@ __device__ __forceinline__ void finalize_step(const KParams& K, int lane) {
   }
   if (lane < n_r && log_out) {
     const bool logged = P.reward[lane].weight != 0.0f;  // reward_manager.py:208-209
-    log_out[lane] = (g_reset > 0.0 && logged) ? (float)(sum / g_reset) : 0.0f;
+    log_out[lane] = (g_reset > 0.0 && logged) ? xs_mean(sum, g_reset) : 0.0f;
   }
   if (lane == n_t) rep->global_n_reset = (long long)counts;
   if (lane == 0) rep->status = status;  // (again: the exchange may have added GFB_STATUS_PEER_TIMEOUT)

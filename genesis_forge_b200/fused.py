@@ -99,7 +99,8 @@ def combine_logging(acc: torch.Tensor, n_reward: int, n_termination: int, global
     """
     out = torch.empty(n_reward + n_termination, device=acc.device, dtype=torch.float32)
     n_reset = acc[n_reward + n_termination].clamp(min=1.0)
-    out[:n_reward] = (acc[:n_reward] / n_reset).float()
+    s = acc[:n_reward].float()  # a sum past the fp32 range is logged as +-Inf, as in tail.cuh (xs_mean)
+    out[:n_reward] = torch.where(torch.isfinite(s), (acc[:n_reward] / n_reset).float(), s)
     out[n_reward:] = (acc[n_reward:n_reward + n_termination] / float(global_num_envs)).float()
     return out
 
@@ -1494,7 +1495,9 @@ class FusedStep:
             self._log_out_host = torch.empty(n_r + n_t, dtype=torch.float32).pin_memory()
         out = self._log_out_host.numpy()
         n_reset = max(float(acc[n_r + n_t]), 1.0)
-        out[:n_r] = acc[:n_r] / n_reset
+        with np.errstate(over="ignore", invalid="ignore"):
+            s = acc[:n_r].astype(np.float32)  # a sum past the fp32 range is logged as +-Inf (tail.cuh xs_mean)
+        out[:n_r] = np.where(np.isfinite(s), acc[:n_r] / n_reset, s)
         out[n_r:] = acc[n_r:n_r + n_t] / float(self.global_num_envs)
         snap = torch.empty(n_r + n_t, device=self.device, dtype=torch.float32)
         snap.copy_(self._log_out_host, non_blocking=True)

@@ -93,6 +93,22 @@ def test_sm100a_code_is_what_was_built():
     assert "HMMA" not in sass and "UTCHMMA" not in sass  # nothing here is a dense contraction
 
 
+def test_post_kernel_static_shared_memory_fits_the_launch_margins():
+    """The launchers count the slab plan's dynamic shared memory and allow 2 KB per block for the static shared
+    memory and the 1 KB reservation (gfb200.cu plan_for_launch); they raise the dynamic limit only above
+    44 KB (the 48 KB default minus static memory).  Per-table arrays belong in the plan, not in static memory.
+    cuobjdump's SHARED includes the reservation.  The main library and a sample of the specialised kernels."""
+    import shutil
+    if shutil.which("cuobjdump") is None:
+        pytest.skip("cuobjdump not available")
+    libs = [_native.LIB_PATH, *sorted((ROOT / "genesis_forge_b200" / "_spec").glob("spec_*.so"))[:3]]
+    for so in libs:
+        out = subprocess.run(["cuobjdump", "-res-usage", str(so)], capture_output=True, text=True, timeout=300).stdout
+        shared = [int(s) for s in re.findall(r"Function \S*post_kernel\S*:\s*\n\s*REG:\d+ STACK:\d+ SHARED:(\d+)", out)]
+        assert shared, so.name
+        assert max(shared) <= 2048, (so.name, shared)
+
+
 def test_sass_obeys_the_uniform_datapath_rule():
     """No mbarrier / bulk-copy instruction sits in a lane-divergent region whose sibling lanes write a
     uniform register before the warp reconverges (csrc/device_utils.cuh; the bug it guards against --
