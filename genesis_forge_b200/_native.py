@@ -104,7 +104,7 @@ class ObsCol(C.Structure):
 
 
 class ObsGroup(C.Structure):
-    _fields_ = [("n_cols", C.c_int32), ("history", C.c_int32), ("col_begin", C.c_int32), ("_pad", C.c_int32)]
+    _fields_ = [("n_cols", C.c_int32), ("history", C.c_int32), ("col_begin", C.c_int32), ("user_id", C.c_int32)]
 
 
 class ProgramHead(C.Structure):
@@ -231,7 +231,7 @@ def lib() -> C.CDLL:
     L.gfb_spec_attach.restype = C.c_int
     L.gfb_spec_attach.argtypes = [vp, C.c_char_p]
     L.gfb_spec_stats.restype = C.c_int
-    L.gfb_spec_stats.argtypes = [vp, C.POINTER(i64), C.POINTER(i64)]
+    L.gfb_spec_stats.argtypes = [vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]
     L.gfb_profile_enable.restype = C.c_int
     L.gfb_profile_enable.argtypes = [vp, i32]
     L.gfb_profile_read.restype = C.c_int

@@ -71,6 +71,8 @@ struct AttachedSpec {
   void* dl = nullptr;
   int (*launch)(const KParams*, int, unsigned, void*) = nullptr;
   int (*blocks_per_sm)(unsigned) = nullptr;
+  // reset path of the lowered user-defined observation terms (spec_kernel.cu), if the library has them
+  int (*user_observe)(const gfb_buffers*, int, const int64_t*, int, int, void*) = nullptr;
   int tile = 0;
   uint32_t phases = 0;
   gfb_program_head canon;
@@ -79,7 +81,7 @@ struct AttachedSpec {
 
 struct gfb_handle {
   std::vector<AttachedSpec> specs;
-  int64_t n_spec_launches = 0, n_generic_launches = 0;
+  int64_t n_spec_launches = 0, n_generic_launches = 0, n_user_observe_launches = 0;
   bool host_only = false;
   int device = 0;
   int num_envs = 0;
@@ -117,12 +119,12 @@ struct gfb_handle {
   int n_post = 0, n_action = 0;
   float post_ms = 0.f, action_ms = 0.f, post_obs_ms = 0.f;
   int post_count = 0, action_count = 0, post_obs_count = 0;
-  // the small kernels: 0 index compaction, 1 observe (reset envs), 2 spawn
+  // the small kernels: 0 index compaction, 1 observe (reset envs), 2 spawn, 3 lowered user observation terms
   std::vector<cudaEvent_t> ev_aux;
   std::vector<uint8_t> ev_aux_kind;
   int n_aux = 0;
-  float aux_ms[3] = {0.f, 0.f, 0.f};
-  int aux_count[3] = {0, 0, 0};
+  float aux_ms[4] = {0.f, 0.f, 0.f, 0.f};
+  int aux_count[4] = {0, 0, 0, 0};
   int smem_attr_post[4] = {0, 0, 0, 0};
   int smem_attr_action[4] = {0, 0, 0, 0};
 };
@@ -172,7 +174,14 @@ void canonicalize(gfb_program_head& c) {
   }
 }
 
+bool has_user_observations(const gfb_program_head& P) {
+  for (int g = 0; g < P.n_obs_groups; ++g)
+    if (P.obs_group[g].user_id != 0) return true;
+  return false;
+}
+
 bool uses_user_terms(const gfb_program_head& P, uint32_t phases) {
+  if ((phases & GFB_PHASE_OBSERVE) && has_user_observations(P)) return true;
   if (phases & GFB_PHASE_REWARD)
     for (int r = 0; r < P.n_reward; ++r)
       if (P.reward[r].op == GFB_R_USER && P.reward[r].weight != 0.0f) return true;
@@ -258,8 +267,9 @@ uint32_t compute_needs(const gfb_program& prog, uint32_t phases) {
 
 // Lay out the shared-memory slab for one (program, phases, tile) combination and lower the
 // observation columns to device descriptors.
+// observe_only: the plan of gfb_observe, whose observe_kernel reads every column from global memory
 int build_plan(gfb_handle* h, const gfb_buffers& b, uint32_t phases, int tile, int n_stages, Plan& plan,
-               std::vector<int32_t>& table) {
+               std::vector<int32_t>& table, bool observe_only = false) {
   std::vector<DevObsCol> cols;
   const gfb_program& prog = h->prog;
   const gfb_program_head& P = prog.head;
@@ -376,6 +386,17 @@ int build_plan(gfb_handle* h, const gfb_buffers& b, uint32_t phases, int tile, i
     plan.st_air[m] = stride;
     if (P.contact[m].track_air_time) stride += 4 * P.contact[m].n_links;
   }
+  // the lowered user-defined observation terms' values (GFB_O_USER), written by the owner threads
+  // (post_kernel.cuh: user_stash_base); `mgr` of such a column is the terms' total width
+  const int st_user = stride;
+  int user_words = 0;
+  if ((phases & GFB_PHASE_OBSERVE) && !observe_only)
+    for (int g = 0; g < P.n_obs_groups; ++g)
+      for (int c = 0; c < P.obs_group[g].n_cols; ++c) {
+        const gfb_obs_col& oc = prog.obs_cols[P.obs_group[g].col_begin + c];
+        if (oc.src == GFB_O_USER) user_words = std::max(user_words, (int)oc.mgr);
+      }
+  stride += user_words;
   if ((stride & 1) == 0) ++stride;  // odd stride: conflict-free per-thread rows
   plan.stash_stride = stride;
   plan.stash_off = cursor;
@@ -452,6 +473,16 @@ int build_plan(gfb_handle* h, const gfb_buffers& b, uint32_t phases, int tile, i
       case GFB_O_EXTERNAL:
         if (oc.mgr <= 0) return fail(h, GFB_ERR_INVALID, "obs: external column needs its array width in mgr");
         global_src(GFB_B_OBS_EXT0, oc.mgr);
+        break;
+      case GFB_O_USER:
+        if (oc.mgr <= 0 || oc.col < 0 || oc.col >= oc.mgr)
+          return fail(h, GFB_ERR_INVALID, "obs: user column needs the terms' width in mgr and col < mgr");
+        if (observe_only) {
+          global_src(GFB_B_OBS_EXT1, oc.mgr);  // written by the specialised library's user_observe
+        } else {
+          d.kind = 3;
+          d.a = st_user + oc.col;
+        }
         break;
       case GFB_O_ZERO:
         d.kind = 0;
@@ -1009,8 +1040,8 @@ int gfb_post_physics(gfb_handle* h, const gfb_buffers* b, uint32_t phases, void*
     // user-defined terms lowered to device code exist only in the specialised kernel generated for them
     if (c.spec_index < 0 && uses_user_terms(P, phases))
       return fail(h, GFB_ERR_UNSUPPORTED,
-                  "the program has GFB_R_USER / GFB_T_USER terms and no specialised kernel generated for them is "
-                  "attached (the generic kernel does not evaluate them)");
+                  "the program has GFB_R_USER / GFB_T_USER terms or GFB_O_USER columns and no specialised kernel "
+                  "generated for them is attached (the generic kernel does not evaluate them)");
     c.prog_epoch = h->prog_epoch;
     c.spec_gen = h->spec_gen;
     c.phases = phases;
@@ -1254,7 +1285,7 @@ int gfb_observe(gfb_handle* h, const gfb_buffers* b, const int64_t* idx, int32_t
   int rc = GFB_OK;
   if (!(oc.valid && oc.prog_epoch == h->prog_epoch && oc.key == key)) {
     oc.valid = false;
-    rc = build_plan(h, *b, GFB_PHASE_OBSERVE, kObserveTile, 1, oc.plan, oc.table);
+    rc = build_plan(h, *b, GFB_PHASE_OBSERVE, kObserveTile, 1, oc.plan, oc.table, true);
     if (rc != GFB_OK) return rc;
     oc.prog_epoch = h->prog_epoch;
     oc.key = key;
@@ -1264,6 +1295,22 @@ int gfb_observe(gfb_handle* h, const gfb_buffers* b, const int64_t* idx, int32_t
   const std::vector<int32_t>& table = oc.table;
   if ((op.plan.needs & NEED_LIN) && !b->buf[GFB_B_VEL]) return fail(h, GFB_ERR_INVALID, "VEL missing");
   if ((op.plan.needs & NEED_ANG) && !b->buf[GFB_B_ANG]) return fail(h, GFB_ERR_INVALID, "ANG missing");
+  // lowered user-defined observation terms: only the library generated for them (same structure, so the
+  // same user_id) computes them -- into GFB_B_OBS_EXT1, which the plan's GFB_O_USER columns read
+  const AttachedSpec* user_spec = nullptr;
+  if (has_user_observations(P)) {
+    gfb_program_head canon = P;
+    canonicalize(canon);
+    for (const AttachedSpec& sp : h->specs)
+      if (sp.user_observe && memcmp(&sp.canon, &canon, sizeof(canon)) == 0) {
+        user_spec = &sp;
+        break;
+      }
+    if (!user_spec)
+      return fail(h, GFB_ERR_UNSUPPORTED,
+                  "gfb_observe: the program has GFB_O_USER columns and no specialised kernel generated for them is "
+                  "attached (the generic kernel does not evaluate them)");
+  }
   rc = upload_table(h, h->observe_slot, table, stream);
   if (rc != GFB_OK) return rc;
   op.P.n_contact = P.n_contact;
@@ -1285,6 +1332,14 @@ int gfb_observe(gfb_handle* h, const gfb_buffers* b, const int64_t* idx, int32_t
   op.cols = reinterpret_cast<const DevObsCol*>(h->observe_slot.table_dev);
   op.idx = idx;
   op.n = n;
+  if (user_spec) {
+    cudaEvent_t user_end = aux_begin(h, 3, stream);
+    if (user_spec->user_observe(b, P.num_envs, idx, n, P.base_max_episode_length > 0 ? 1 : 0, stream) != 0)
+      return fail(h, GFB_ERR_CUDA, std::string("user observation kernel: ") + cudaGetErrorString(cudaGetLastError()));
+    if (user_end) cudaEventRecord(user_end, stream);
+    h->n_user_observe_launches += 1;
+    h->launches += 1;
+  }
   const int grid = (n + OBS_WARPS * OBS_ROWS - 1) / (OBS_WARPS * OBS_ROWS);
   cudaEvent_t obs_end = aux_begin(h, 1, stream);
   observe_kernel<<<grid, OBS_WARPS * 32, 0, stream>>>(op);
@@ -1440,15 +1495,18 @@ int gfb_spec_attach(gfb_handle* h, const char* path) {
   sp.dl = dl;
   sp.launch = launch;
   sp.blocks_per_sm = reinterpret_cast<int (*)(unsigned)>(dlsym(dl, "gfb_spec_blocks_per_sm"));
+  sp.user_observe = reinterpret_cast<int (*)(const gfb_buffers*, int, const int64_t*, int, int, void*)>(
+      dlsym(dl, "gfb_spec_user_observe"));
   h->specs.push_back(sp);
   h->spec_gen += 1;
   return GFB_OK;
 }
 
-int gfb_spec_stats(const gfb_handle* h, int64_t* specialised, int64_t* generic) {
+int gfb_spec_stats(const gfb_handle* h, int64_t* specialised, int64_t* generic, int64_t* user_observe) {
   if (!h) return GFB_ERR_INVALID;
   if (specialised) *specialised = h->n_spec_launches;
   if (generic) *generic = h->n_generic_launches;
+  if (user_observe) *user_observe = h->n_user_observe_launches;
   return GFB_OK;
 }
 
@@ -1468,7 +1526,7 @@ int gfb_profile_enable(gfb_handle* h, int32_t enabled) {
   h->n_post = h->n_action = h->n_aux = 0;
   h->post_ms = h->action_ms = h->post_obs_ms = 0.f;
   h->post_count = h->action_count = h->post_obs_count = 0;
-  for (int k = 0; k < 3; ++k) {
+  for (int k = 0; k < 4; ++k) {
     h->aux_ms[k] = 0.f;
     h->aux_count[k] = 0;
   }
@@ -1517,7 +1575,7 @@ int gfb_profile_read_aux(gfb_handle* h, float* ms_total, int32_t* launches) {
   if (!h || !ms_total || !launches) return GFB_ERR_INVALID;
   int rc = gfb_profile_read(h, nullptr, nullptr, nullptr, nullptr);  // folds pending event pairs
   if (rc != GFB_OK) return rc;
-  for (int k = 0; k < 3; ++k) {
+  for (int k = 0; k < 4; ++k) {
     ms_total[k] = h->aux_ms[k];
     launches[k] = h->aux_count[k];
   }

@@ -135,6 +135,7 @@ __device__ __forceinline__ void issue_slab_loads(const KParams& K, const Plan& p
 // body-frame registers the plan already has (pos / quat / vel / ang, lin_b / ang_b / grav_b), otherwise its
 // env's rows of the engine / environment arrays in global memory; the owner thread's registers (episode
 // counters, this step's termination flags, the inverse base quaternion) and stash; its live params.
+// The reset path of the observation terms (spec_kernel.cu) reads global memory only (S, st: null).
 struct UserCtx {
   const gfb_buffers& b;
   size_t e;
@@ -148,7 +149,15 @@ struct UserCtx {
   const float* st;
   const Plan& plan;
   const float* p;
+  int n_envs;  // (global-memory reads of the air-time planes)
 };
+
+// First stash word of the lowered user-defined observation values (gfb200.cu build_plan: st_user)
+__device__ __forceinline__ int user_stash_base(const gfb_program_head& SP) {
+  int s = 9;
+  for (int m = 0; m < SP.n_contact; ++m) s += SP.contact[m].n_links * (SP.contact[m].track_air_time ? 5 : 1);
+  return s;
+}
 
 #if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
 // NaN propagating; on a tie (+0 / -0) the second operand.  amax / amin pass (element, accumulator), so a
@@ -989,6 +998,15 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
       ep_secs = 1e-10f;
     }
   }
+
+#if defined(GFB_SPEC) && defined(GFB_SPEC_USER_OBS)
+  // lowered user-defined observation terms: from what a stock column of this launch sees (the post-resample
+  // command, the body-frame registers, the staged rows) into the stash words the GFB_O_USER columns read
+  if (ph & GFB_PHASE_OBSERVE)
+    user_observations(UserCtx{K.b, (size_t)e, ep_len, max_len, terminated, truncated, iw, iq, lin_b, ang_b, grav_b, S,
+                              tid, st, plan, nullptr, N},
+                      st + user_stash_base(SP));
+#endif
 
   // ------------------------------------------------------------------------------------------
   // per-env outputs

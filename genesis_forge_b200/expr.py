@@ -1,5 +1,5 @@
 """
-User-defined reward / termination terms lowered into the specialised post-physics kernel.
+User-defined reward / termination / observation terms lowered into the specialised post-physics kernel.
 
 A user term is a plain Python function of the environment, e.g.
 
@@ -19,6 +19,13 @@ the same kernel binary; everything else the function captures is a compile-time 
 operation order with the kernel's round-to-nearest helpers; reductions accumulate in index order.
 The generated functions go into the header of the specialised kernel (spec.py) and are called in the
 owner phase of post_kernel, in the GFB_R_USER / GFB_T_USER cases of the term switches.
+
+Observation terms (kind "observation", ManagedEnvironment.fuse_user_observations) may return any
+per-env shape of at most MAX_CONST_VEC elements, which is flattened row-major into their columns and cast
+to fp32, and may build rows with the layout ops torch.stack / torch.cat over the last dimension,
+unsqueeze, None in an index and reshape / view / flatten of a row.  Their params are constants (traced
+again when they change).  Their device code comes twice: for the owner phase of post_kernel and, reading
+global memory only, for the reset path that re-observes reset envs (spec_kernel.cu).
 
 Anything outside this subset raises UnsupportedTermError naming the op or source; the term then
 stays a host callback (split execution), with exactly the results it had before.
@@ -262,6 +269,12 @@ class Sym:
     def __getitem__(self, key):
         return self._tr.index(self, key)
 
+    # -- layout (observation terms) --------------------------------------------------------------
+    def unsqueeze(self, dim): return self._tr.unsqueeze(self, dim)
+    def reshape(self, *shape): return self._tr.reshape(self, shape)
+    view = reshape
+    def flatten(self, start_dim=0, end_dim=-1): return self._tr.flatten(self, start_dim, end_dim)
+
     def nonzero(self, *a, **k):
         raise UnsupportedTermError("user term: nonzero() (data-dependent shape)")
 
@@ -273,7 +286,10 @@ class Sym:
         tr = next((a._tr for a in operands if isinstance(a, Sym)), None)
         if tr is None:  # the symbolic values sit inside a sequence argument (torch.stack, torch.cat, ...)
             name = getattr(func, "__name__", str(func))
-            raise UnsupportedTermError(f"user term: torch function '{name}' of a sequence of per-env values")
+            seq = [a for op in operands if isinstance(op, (list, tuple)) for a in op]
+            tr = next((a._tr for a in seq if isinstance(a, Sym)), None)
+            if tr is None or tr.kind != "observation" or name not in _LAYOUT_SEQ:
+                raise UnsupportedTermError(f"user term: torch function '{name}' of a sequence of per-env values")
         return tr.torch_function(func, args, kwargs)
 
 
@@ -298,6 +314,7 @@ _BINARY_TORCH = {
     "bitwise_or": "or", "minimum": "minimum", "maximum": "maximum",
 }
 _REDUCE_TORCH = {"sum": "sum", "mean": "mean", "any": "any", "all": "all", "amax": "amax", "amin": "amin"}
+_LAYOUT_SEQ = ("stack", "cat", "concat", "concatenate")  # over a sequence of values (observation terms only)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -479,10 +496,118 @@ class Tracer:
             raise UnsupportedTermError(f"user term: {kind} of a bool value")
         return self.add(kind, (x._id,), axis, shape, dt)
 
+    # -- layout ops: observation terms build their rows with them ------------------------------------
+    def _layout(self, what: str):
+        if self.kind != "observation":
+            raise UnsupportedTermError(f"user term: {what} (layout ops are lowered in observation terms only)")
+
+    def _as_row(self, shape: tuple, x: Sym) -> Sym:
+        """x with the per-env shape `shape` (same elements, row-major)."""
+        if tuple(shape) == x.shape_:
+            return x
+        return self.add("reshape", (x._id,), None, tuple(shape), x.dtype_)
+
+    def _dim(self, dim, rank: int, what: str, extra: int = 0) -> int:
+        """A dim argument over the full (N, ...) rank as a per-env axis; the env axis is refused."""
+        if isinstance(dim, Sym):
+            dim._control("dim")
+        if not isinstance(dim, int) or isinstance(dim, bool):
+            raise UnsupportedTermError(f"user term: {what}(dim={dim!r})")
+        d = dim + rank + extra if dim < 0 else dim
+        if not 1 <= d < rank + extra:
+            raise UnsupportedTermError(f"user term: {what}(dim={dim}) of a rank-{rank} value (the env dimension "
+                                       "stays first)")
+        return d - 1
+
+    def unsqueeze(self, x, dim) -> Sym:
+        self._layout("unsqueeze")
+        x = self.lift(x)
+        axis = self._dim(dim, len(x.shape_) + 1, "unsqueeze", extra=1)
+        return self._as_row(x.shape_[:axis] + (1,) + x.shape_[axis:], x)
+
+    def reshape(self, x, shape) -> Sym:
+        self._layout("reshape / view")
+        x = self.lift(x)
+        if len(shape) == 1 and isinstance(shape[0], (tuple, list, torch.Size)):
+            shape = tuple(shape[0])
+        if any(isinstance(v, Sym) for v in shape):
+            next(v for v in shape if isinstance(v, Sym))._control("reshape")
+        size = int(np.prod(x.shape_)) if x.shape_ else 1
+        total = self.N * size
+        shape = [int(v) for v in shape]
+        if shape.count(-1) > 1:
+            raise UnsupportedTermError("user term: reshape with more than one -1")
+        known = int(np.prod([v for v in shape if v != -1])) if shape else 1
+        if -1 in shape:
+            if known == 0 or total % known:
+                raise UnsupportedTermError(f"user term: reshape to {tuple(shape)}")
+            shape[shape.index(-1)] = total // known
+        if not shape or shape[0] != self.N or int(np.prod(shape)) != total:
+            raise UnsupportedTermError(f"user term: reshape to {tuple(shape)} (rows of the {self.N} envs only)")
+        return self._as_row(tuple(shape[1:]), x)
+
+    def flatten(self, x, start_dim=0, end_dim=-1) -> Sym:
+        self._layout("flatten")
+        x = self.lift(x)
+        rank = len(x.shape_) + 1
+        s = start_dim + rank if start_dim < 0 else start_dim
+        t = end_dim + rank if end_dim < 0 else end_dim
+        if s < 1 or t < s or t >= rank:
+            if rank == 1 and s == 1:
+                return x
+            raise UnsupportedTermError(f"user term: flatten({start_dim}, {end_dim}) (rows of the envs only)")
+        a, b = s - 1, t - 1
+        return self._as_row(x.shape_[:a] + (int(np.prod(x.shape_[a:b + 1])),) + x.shape_[b + 1:], x)
+
+    def stack_cat(self, name: str, seq, dim) -> Sym:
+        self._layout(f"torch.{name}")
+        if not isinstance(seq, (list, tuple)) or not seq:
+            raise UnsupportedTermError(f"user term: torch.{name} of {type(seq).__name__}")
+        xs = [self.lift(v) for v in seq]
+        if any(v.weak for v in xs):
+            raise UnsupportedTermError(f"user term: torch.{name} of a Python scalar")
+        dt = max((v.dtype_ for v in xs), key=_RANK.get)  # torch.result_type of tensors alone
+        xs = [self.cast(v, dt) for v in xs]
+        if name == "stack":
+            shape = xs[0].shape_
+            if any(v.shape_ != shape for v in xs):
+                raise UnsupportedTermError("user term: torch.stack of values with different shapes")
+            axis = self._dim(dim, len(shape) + 1, "stack", extra=1)
+            if axis != len(shape):
+                raise UnsupportedTermError(f"user term: torch.stack(dim={dim}) (over the last dimension only)")
+            return self.add("stack", tuple(v._id for v in xs), None, shape + (len(xs),), dt)
+        rank = len(xs[0].shape_) + 1
+        if rank == 1:
+            raise UnsupportedTermError(f"user term: torch.{name} of (N,) values (it joins envs)")
+        axis = self._dim(dim, rank, name)
+        if axis != rank - 2 or any(len(v.shape_) != rank - 1 or v.shape_[:-1] != xs[0].shape_[:-1] for v in xs):
+            raise UnsupportedTermError(f"user term: torch.{name}(dim={dim}) (over the last dimension only)")
+        shape = xs[0].shape_[:-1] + (sum(v.shape_[-1] for v in xs),)
+        return self.add("cat", tuple(v._id for v in xs), None, shape, dt)
+
     def index(self, x: Sym, key) -> Sym:
-        shape = x.shape_
         if not isinstance(key, tuple):
             key = (key,)
+        if any(k is None for k in key[1:]):  # None inserts a size-1 axis: the indexed value, reshaped
+            self._layout("None in an index")
+            kept = tuple(k for k in key if k is not None)
+            out = self.index(x, kept)
+            rest = list(key[1:])
+            if key[0] is Ellipsis:
+                n_tail = sum(1 for k in rest if k is not None)
+                rest = [slice(None)] * (len(x.shape_) - n_tail) + rest
+            shape, src = [], list(out.shape_)
+            for k in rest:
+                if k is None:
+                    shape.append(1)
+                elif isinstance(k, slice):
+                    shape.append(src.pop(0))
+            shape += src
+            return self._as_row(tuple(shape), out)
+        return self._index(x, key)
+
+    def _index(self, x: Sym, key: tuple) -> Sym:
+        shape = x.shape_
         if not key or not (key[0] == slice(None) or key[0] is Ellipsis):
             raise UnsupportedTermError("user term: indexing that selects envs (only [:, ...] / [..., j] keep every env)")
         rest = list(key[1:]) if key[0] == slice(None) else None
@@ -546,6 +671,17 @@ class Tracer:
                 raise UnsupportedTermError(f"user term: norm(p={p!r})")
             dim = kwargs.get("dim", args[2] if len(args) > 2 else None)
             return self.reduce("norm", args[0], dim, kwargs.get("keepdim", False))
+        if name in _LAYOUT_SEQ:
+            seq = args[0] if args else kwargs.get("tensors")
+            dim = args[1] if len(args) > 1 else kwargs.get("dim", 0)
+            return self.stack_cat("stack" if name == "stack" else "cat", seq, dim)
+        if name == "unsqueeze":
+            return self.unsqueeze(args[0], args[1] if len(args) > 1 else kwargs.get("dim"))
+        if name in ("reshape", "view"):
+            return self.reshape(args[0], tuple(args[1:]) if len(args) > 1 else (kwargs.get("shape"),))
+        if name == "flatten":
+            return self.flatten(args[0], args[1] if len(args) > 1 else kwargs.get("start_dim", 0),
+                                args[2] if len(args) > 2 else kwargs.get("end_dim", -1))
         if name == "pow":
             return self.lift(args[0]).__pow__(args[1])
         if name in ("float",):
@@ -656,6 +792,13 @@ class ExprMode:
             return tr.source(("actions",), (D,), F32)
         if isinstance(key, tuple) and key[0] == "command":
             return key[1].command
+        # body-frame vectors the kernel does not hold: a further EntityManager's (its own cached quaternion) and
+        # those of a term without an entity_manager (the current quaternion); refused without evaluating them
+        if isinstance(key, tuple) and isinstance(key[0], str) and key[0].startswith("entity_"):
+            raise UnsupportedTermError("user term: a body-frame getter of a further EntityManager (the kernel "
+                                       "holds the first manager's pose)")
+        if isinstance(key, str) and key.endswith("_uncached"):
+            raise UnsupportedTermError("user term: a body-frame term without an entity_manager")
         return compute()
 
 
@@ -666,7 +809,7 @@ def param_kinds(params) -> tuple:
 
 
 def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> Program:
-    """Trace one user-defined reward / termination into a Program (raises UnsupportedTermError)."""
+    """Trace one user-defined reward / termination / observation into a Program (raises UnsupportedTermError)."""
     env = fused.env
     fn = item.fn
     what = f"{kind} '{name}'"
@@ -683,13 +826,23 @@ def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> P
     try:
         _install_sources(fused, tr, swap, kind)
         env._tracing = ExprMode(tr, fused)
-        result = fn(env, **params)
+        result = fn(env=env, **params) if kind == "observation" else fn(env, **params)
     finally:
         env._tracing = None
         swap.restore()
     if not isinstance(result, Sym):
         raise UnsupportedTermError(f"{what}: the result does not depend on per-env state the kernel holds "
                                    f"({type(result).__name__})")
+    if kind == "observation":
+        # flattened row-major into its columns and cast to fp32, as FusedStep.evaluate_external_obs copies it
+        if result.weak:
+            raise UnsupportedTermError(f"{what}: the result is a Python scalar")
+        width = int(np.prod(result.shape_)) if result.shape_ else 1
+        if width > MAX_CONST_VEC:
+            raise UnsupportedTermError(f"{what}: {width} columns (at most {MAX_CONST_VEC} are lowered)")
+        out = tr.cast(tr._as_row((width,), result), F32)._id
+        nodes = _live_nodes(tr.nodes, out)
+        return Program(kind, nodes[0], nodes[1], [], [])
     if result.weak or result.shape_ != ():
         raise UnsupportedTermError(f"{what}: the result has shape {tuple(result.shape)}, not (N,)")
     if kind == "termination" and result.dtype_ != BOOL:
@@ -702,7 +855,13 @@ def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> P
 
 
 def lower_term(fused, kind: str, name: str, item) -> tuple[Program, bool]:
-    """(program, params_live): trace with live params, or once more with params as constants."""
+    """(program, params_live): trace with live params, or once more with params as constants (always for
+    observation terms: only their scale and noise are live, as for stock columns)."""
+    if kind == "observation":
+        try:
+            return trace_term(fused, kind, name, item, live_params=False), False
+        except _ParamControlFlow as e:
+            raise UnsupportedTermError(f"{kind} '{name}': Python scalar arithmetic on '{e}' inside the term") from None
     try:
         return trace_term(fused, kind, name, item, live_params=True), True
     except _ParamControlFlow:
@@ -743,8 +902,11 @@ def _install_sources(fused, tr: Tracer, swap: _Swap, kind: str):
     if fused.entity_manager is not None:
         em = fused.entity_manager
         swap.set(em, "entity", proxy)
-        swap.set(em, "_base_pos", tr.source(("pos",), (3,), F32))
-        swap.set(em, "_base_quat", tr.source(("quat",), (4,), F32))
+        # (rewards and terminations run after the entity phase: the cache IS this step's pose; the observation
+        #  of a reset env sees the pre-reset cache next to the post-reset engine state)
+        cached = kind == "observation"
+        swap.set(em, "_base_pos", tr.source(("base_pos",) if cached else ("pos",), (3,), F32))
+        swap.set(em, "_base_quat", tr.source(("base_quat",) if cached else ("quat",), (4,), F32))
     for k, mgr in enumerate(fused.commands):
         if mgr in fused.python_commands or mgr._external_controller is not None:
             continue  # a user-level manager's state stays concrete: refused where it is used
@@ -767,7 +929,7 @@ def _install_sources(fused, tr: Tracer, swap: _Swap, kind: str):
         elif kind == "reward":
             swap.set_item(extras, key, tr.source((src,), (), BOOL))
         else:
-            swap.set_item(extras, key, _Refused(f"extras['{key}'] inside a termination term"))
+            swap.set_item(extras, key, _Refused(f"extras['{key}'] inside a {kind} term"))
 
 
 class _Refused:
@@ -810,21 +972,34 @@ def _lit(v, dtype) -> str:
 _SLAB = {"pos": "off_pos", "quat": "off_quat", "vel": "off_vel", "ang": "off_ang"}  # staged slab rows (plan.h)
 
 
-def _src_elems(key: tuple, shape: tuple, lines: list, v: str) -> list[str]:
-    """C expressions of a source's elements for this env (row-major over `shape`)."""
+def _src_elems(key: tuple, shape: tuple, lines: list, v: str, glob: bool = False) -> list[str]:
+    """C expressions of a source's elements for this env (row-major over `shape`).  `glob`: global memory
+    only (the reset path of observation terms, which has no slab, stash or body-frame registers)."""
     n = int(np.prod(shape)) if shape else 1
     name = key[0]
+    if name in ("base_pos", "base_quat"):  # the EntityManager's cached pose (observation terms)
+        w, eng = (3, "pos") if name == "base_pos" else (4, "quat")
+        cache = f"reinterpret_cast<const float*>(c.b.buf[GFB_B_BASE_{eng.upper()}]) + (size_t)c.e * {w}"
+        if glob:
+            lines.append(f"const float* {v}p = {cache};")
+        else:
+            # a launch with the entity phase (the only one that stages quat) writes the cache from these rows
+            off = f"c.plan.{_SLAB[eng]}"
+            engine = f"reinterpret_cast<const float*>(c.b.buf[GFB_B_{eng.upper()}]) + (size_t)c.e * {w}"
+            lines.append(f"const float* {v}p = c.plan.off_quat >= 0 ? ({off} >= 0 ? c.S + {off} + c.tid * {w} : "
+                         f"{engine}) : {cache};")
+        return [f"{v}p[{i}]" for i in range(n)]
     row = {"pos": ("GFB_B_POS", 3), "quat": ("GFB_B_QUAT", 4), "vel": ("GFB_B_VEL", 3), "ang": ("GFB_B_ANG", 3),
            "dof_pos": ("GFB_B_DOF_POS", n), "dof_vel": ("GFB_B_DOF_VEL", n), "targets": ("GFB_B_TARGETS", n),
            "actions": ("GFB_B_ENV_ACTIONS", n), "last_actions": ("GFB_B_ENV_LAST_ACTIONS", n)}
     if name in row:
         buf, w = row[name]
-        glob = f"reinterpret_cast<const float*>(c.b.buf[{buf}]) + (size_t)c.e * {w}"
-        if name in _SLAB:  # the slab row when the plan stages the array (a compile-time choice)
+        gaddr = f"reinterpret_cast<const float*>(c.b.buf[{buf}]) + (size_t)c.e * {w}"
+        if name in _SLAB and not glob:  # the slab row when the plan stages the array (a compile-time choice)
             off = f"c.plan.{_SLAB[name]}"
-            lines.append(f"const float* {v}p = {off} >= 0 ? c.S + {off} + c.tid * {w} : {glob};")
+            lines.append(f"const float* {v}p = {off} >= 0 ? c.S + {off} + c.tid * {w} : {gaddr};")
         else:
-            lines.append(f"const float* {v}p = {glob};")
+            lines.append(f"const float* {v}p = {gaddr};")
         return [f"{v}p[{i}]" for i in range(n)]
     if name == "command":
         lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[GFB_B_COMMAND0 + {key[1]}]) + "
@@ -836,6 +1011,10 @@ def _src_elems(key: tuple, shape: tuple, lines: list, v: str) -> list[str]:
         return [f"{v}p[{i}]" for i in range(n)]
     if name == "air":
         m, j = key[1], key[2]
+        if glob:  # (4, N, Lc) planes
+            lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[GFB_B_AIR0 + {m}]) + "
+                         f"(size_t){j} * c.n_envs * {n} + c.e * {n};")
+            return [f"{v}p[{l}]" for l in range(n)]
         return [f"c.st[c.plan.st_air[{m}] + {l * 4 + j}]" for l in range(n)]
     if name in ("lin_vel_b", "ang_vel_b", "gravity_b"):
         # the kernel's own register when the plan computes it (same rotation), else rotated here
@@ -847,7 +1026,10 @@ def _src_elems(key: tuple, shape: tuple, lines: list, v: str) -> list[str]:
             buf = "GFB_B_VEL" if name == "lin_vel_b" else "GFB_B_ANG"
             lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[{buf}]) + (size_t)c.e * 3;")
             vec = f"V3{{{v}p[0], {v}p[1], {v}p[2]}}"
-        lines.append(f"const V3 {v}r = (c.plan.needs & {need}) ? c.{reg} : rotate({vec}, c.iw, c.iq);")
+        if glob:
+            lines.append(f"const V3 {v}r = rotate({vec}, c.iw, c.iq);")
+        else:
+            lines.append(f"const V3 {v}r = (c.plan.needs & {need}) ? c.{reg} : rotate({vec}, c.iw, c.iq);")
         return [f"{v}r.x", f"{v}r.y", f"{v}r.z"]
     if name == "episode_length":
         return ["c.ep_len"]
@@ -907,8 +1089,12 @@ def _unop(op, a, dtype):
     return f"{fn}({a})"
 
 
-def function_body(prog: Program, fname: str) -> str:
-    """One `__device__` function for the program (straight-line code, one variable per element)."""
+_PASS = ("sum", "mean", "any", "all", "amax", "amin", "norm", "reshape", "stack", "cat")  # no new variables
+
+
+def function_body(prog: Program, fname: str, glob: bool = False) -> str:
+    """One `__device__` function for the program (straight-line code, one variable per element).  An
+    observation term writes its columns to `out`; `glob` reads global memory only (see _src_elems)."""
     lines: list[str] = []
     elems: list[list[str]] = []
     for i, n in enumerate(prog.nodes):
@@ -916,7 +1102,16 @@ def function_body(prog: Program, fname: str) -> str:
         ct = _CT[n.dtype]
         size = int(np.prod(n.shape)) if n.shape else 1
         if n.op == "src":
-            exprs = _src_elems(n.attr, n.shape, lines, v)
+            exprs = _src_elems(n.attr, n.shape, lines, v, glob)
+        elif n.op == "reshape":
+            exprs = list(elems[n.args[0]])
+        elif n.op == "stack":
+            parts = [elems[j] for j in n.args]
+            exprs = [p[k] for k in range(len(parts[0])) for p in parts]
+        elif n.op == "cat":
+            parts = [(elems[j], prog.nodes[j].shape[-1]) for j in n.args]
+            rows = len(parts[0][0]) // parts[0][1] if parts[0][1] else 0
+            exprs = [x for r in range(rows) for p, w in parts for x in p[r * w:(r + 1) * w]]
         elif n.op == "param":
             p = f"c.p[{n.attr}]"
             exprs = [f"((int){p})" if n.dtype == I32 else p]
@@ -975,14 +1170,17 @@ def function_body(prog: Program, fname: str) -> str:
         # every element is materialised once, in node order (torch's operation order)
         names = []
         for k, x in enumerate(exprs):
-            nm = f"{v}_{k}" if n.op not in ("sum", "mean", "any", "all", "amax", "amin", "norm") else x
+            nm = f"{v}_{k}" if n.op not in _PASS else x
             if nm != x:
                 lines.append(f"const {ct} {nm} = {x};")
             names.append(nm)
         elems.append(names)
+    body = "\n".join("  " + ln for ln in lines)
+    if prog.kind == "observation":
+        stores = "\n".join(f"  out[{k}] = {x};" for k, x in enumerate(elems[prog.out]))
+        return f"__device__ __forceinline__ void {fname}(const UserCtx& c, float* out) {{\n{body}\n{stores}\n}}\n"
     ret = elems[prog.out][0]
     rtype = "bool" if prog.kind == "termination" else "float"
-    body = "\n".join("  " + ln for ln in lines)
     return (f"__device__ __forceinline__ {rtype} {fname}(const UserCtx& c) {{\n{body}\n  return {ret};\n}}\n")
 
 
@@ -1017,8 +1215,10 @@ def _reduce_expr(op, terms, dtype, lines, acc) -> str:
     return acc
 
 
-def device_code(rewards: dict[int, Program], terminations: dict[int, Program]) -> str:
-    """The user-term functions of one table and their dispatchers, keyed by table row."""
+def device_code(rewards: dict[int, Program], terminations: dict[int, Program],
+                observations: list[tuple[int, Program]] = (), obs_words: int = 0) -> str:
+    """The user-term functions of one table and their dispatchers, keyed by table row; the observation terms
+    as (first word in the (N, obs_words) user-observation row, program), each twice (owner phase, reset path)."""
     parts = []
     for r, prog in sorted(rewards.items()):
         parts.append(f"/* reward row {r} */\n" + function_body(prog, f"gfb_user_r{r}"))
@@ -1030,4 +1230,15 @@ def device_code(rewards: dict[int, Program], terminations: dict[int, Program]) -
                  f"{cases_r}    default: return 0.0f;\n  }}\n}}\n")
     parts.append("__device__ __forceinline__ bool user_termination(int t, const UserCtx& c) {\n  switch (t) {\n"
                  f"{cases_t}    default: return false;\n  }}\n}}\n")
+    if observations:
+        calls, calls_g = "", ""
+        for j, (col0, prog) in enumerate(observations):
+            parts.append(f"/* observation term {j}: words {col0}.. */\n" + function_body(prog, f"gfb_user_o{j}"))
+            parts.append(function_body(prog, f"gfb_user_og{j}", glob=True))
+            calls += f"  gfb_user_o{j}(c, out + {col0});\n"
+            calls_g += f"  gfb_user_og{j}(c, out + {col0});\n"
+        parts.append(f"constexpr int kUserObsWords = {obs_words};\n")
+        parts.append(f"__device__ __forceinline__ void user_observations(const UserCtx& c, float* out) {{\n{calls}}}\n")
+        parts.append("__device__ __forceinline__ void user_observations_global(const UserCtx& c, float* out) {\n"
+                     f"{calls_g}}}\n")
     return "".join(parts)

@@ -183,6 +183,9 @@ class FusedStep:
         if self.entity_manager is None:
             self._inv_base_quat = torch.zeros((self.N, 4), device=self.device)
         self.global_num_envs = self.N
+        # set by ObservationManager.resolve_external around a dry run's evaluation of a user observation term for
+        # its width: body-frame rotations return zeros of the right shape (a dry run has no device)
+        self.width_probe = False
         if compile_now:
             self._compile()
 
@@ -275,19 +278,77 @@ class FusedStep:
         self._controller_bound = [False] * len(self.commands)  # GFB_B_COMMAND0+k points at a controller's tensor
         self.any_controller = False
         self._has_command_override = False  # set by CommandManager.use_external_controller / use_gamepad
-        # user-defined observation terms: one (N, W) array filled on the host
-        self.external_obs: list[tuple[object, str, object, int, int]] = []  # (manager, name, item, col0, width)
-        width = 0
-        for om in self.observations:
-            for name, key, w in om._sources:
-                if isinstance(key, tuple) and key[0] == "external":
-                    self.external_obs.append((om, name, om.cfg[name], width, w))
-                    om._external_col0[name] = width
-                    width += w
-        self.ext_obs_width = width
-        self.ext_obs = torch.zeros((N, width), device=dev) if width else None
+        # user-defined observation terms: one (N, W) array filled on the host; with
+        # ManagedEnvironment.fuse_user_observations the ones that lower are evaluated in the kernel instead
+        self.user_obs: dict = {}  # (group, name) -> [Program, params it was traced with, first word, width]
+        self._lower_obs = bool(getattr(env, "fuse_user_observations", False)) and self._can_specialise_user_terms()
+        self._observation_columns()
         self._plan_launches()
         self._static_buffers()
+
+    def _observation_columns(self):
+        """
+        Columns of the user-defined observation terms: lowered ones are words of the (N, user_obs_width)
+        user-observation row (GFB_O_USER: the kernel's stash, GFB_B_OBS_EXT1 on the reset path), the rest
+        columns of the host-filled (N, ext_obs_width) array (GFB_O_EXTERNAL).
+        """
+        self.external_obs: list[tuple[object, str, object, int, int]] = []  # (manager, name, item, col0, width)
+        width = words = 0
+        for g, om in enumerate(self.observations):
+            for name, key, w in om._sources:
+                if not (isinstance(key, tuple) and key[0] == "external"):
+                    continue
+                item = om.cfg[name]
+                if name not in om._host_columns and self._lower_user_obs(g, name, item, w):
+                    self.user_obs[(g, name)][2] = words
+                    words += w
+                    continue
+                self.external_obs.append((om, name, item, width, w))
+                om._external_col0[name] = width
+                width += w
+        self.ext_obs_width = width
+        self.ext_obs = torch.zeros((self.N, width), device=self.device) if width else None
+        self.user_obs_width = words
+        self.user_obs_values = torch.zeros((self.N, words), device=self.device) if words else None
+        self._obs_user_id = 0
+        self._obs_reads_pose = any(n.op == "src" and n.attr[0] in ("pos", "quat")
+                                   for prog, *_ in self.user_obs.values() for n in prog.nodes)
+
+    def _lower_user_obs(self, g: int, name: str, item, width: int) -> bool:
+        """Trace a user-defined observation term into the expression IR; False (reason kept) when it stays a host column."""
+        if not self._lower_obs:
+            return False
+        from . import expr
+
+        try:
+            prog, _ = expr.lower_term(self, "observation", name, item)
+            if prog.nodes[prog.out].shape != (width,):
+                raise UnsupportedTermError(f"observation '{name}': traced {prog.nodes[prog.out].shape[0]} columns, "
+                                           f"the function returned {width}")
+        except Exception as e:  # noqa: BLE001 - whatever the function does on symbolic inputs, it stays a host column
+            why = str(e) if isinstance(e, UnsupportedTermError) else f"{type(e).__name__} while tracing: {e}"
+            self.user_term_refusals[("observation", name)] = why
+            _log.debug("observation '%s' stays a host column: %s", name, why)
+            return False
+        self.user_obs[(g, name)] = [prog, dict(item.params or {}), 0, width]
+        return True
+
+    def _user_obs_program(self, g: int, name: str, item):
+        """The term's Program for its current params (folded as constants: traced again when they change)."""
+        from . import expr
+
+        entry = self.user_obs[(g, name)]
+        if dict(item.params or {}) != entry[1]:
+            prog, _ = expr.lower_term(self, "observation", name, item)
+            if prog.nodes[prog.out].shape != (entry[3],):
+                raise UnsupportedTermError(f"observation '{name}': its width changed with its params")
+            entry[0], entry[1] = prog, dict(item.params or {})
+            self._user_code = None
+        return entry[0]
+
+    @property
+    def lowered_user_terms(self) -> bool:
+        return bool(self.user_terms or self.user_obs)
 
     def _external_values(self):
         """The (J, N) buffer of host-evaluated term values, one row per external reward / termination."""
@@ -332,15 +393,18 @@ class FusedStep:
         if not self._can_specialise_user_terms():
             return "the specialised kernel cannot be used (GFB_NO_SPEC, no nvcc, GFB_DISABLE_TMA or num_envs % 4)"
         K = nat.K
+        if self.user_obs and not self.buffers.buf[K["GFB_B_OBS_EXT1"]]:
+            return "GFB_B_OBS_EXT1 (the user-observation rows of the reset path) is not bound"
         buf = self.buffers.buf
         for name in self._TMA_BUFFERS:
             ptr = buf[K[name]]
             if ptr and ptr % 16:
                 return f"{name} is not 16-byte aligned (the specialised kernel's TMA transfers need it)"
         sets = [p for _, p, _ in self.split_plan] if self.split_mode else [self.step_phases]
+        lowered = K["GFB_PHASE_REWARD"] | K["GFB_PHASE_TERMINATION"] | (K["GFB_PHASE_OBSERVE"] if self.user_obs else 0)
         for phases in sets:
             phases &= self._phase_mask
-            if not phases & (K["GFB_PHASE_REWARD"] | K["GFB_PHASE_TERMINATION"]):
+            if not phases & lowered:
                 continue
             self._maybe_specialise(phases)
             if not self._spec_ok.get(self._spec_tag(phases)):
@@ -353,9 +417,16 @@ class FusedStep:
         _log.warning("lowered user terms run as host callbacks from now on: %s", why)
         for key in self.user_terms:
             self.user_term_refusals[key] = why
+        for _, name in self.user_obs:
+            self.user_term_refusals[("observation", name)] = why
         self.user_terms = {}
+        self.user_obs = {}
         self._user_code = None
         self._lower_user = False
+        self._lower_obs = False
+        self._observation_columns()
+        self._set(K["GFB_B_OBS_EXT0"], self.ext_obs)
+        self._set(K["GFB_B_OBS_EXT1"], None)
         self.reward_terms = [(n, i, K["GFB_R_EXTERNAL"] if op == K["GFB_R_USER"] else op) for n, i, op in self.reward_terms]
         self.termination_terms = [(n, i, K["GFB_T_EXTERNAL"] if op == K["GFB_T_USER"] else op)
                                   for n, i, op in self.termination_terms]
@@ -398,7 +469,9 @@ class FusedStep:
                 for row, (name, _, _) in enumerate(terms):
                     if (kind, name) in self.user_terms:
                         rows[kind][row] = self.user_terms[(kind, name)][0]
-            self._user_code = expr.device_code(rows["reward"], rows["termination"]) if self.user_terms else ""
+            obs = sorted((entry[2], entry[0]) for entry in self.user_obs.values())
+            self._user_code = (expr.device_code(rows["reward"], rows["termination"], obs, self.user_obs_width)
+                               if self.lowered_user_terms else "")
         return self._user_code
 
     def _user_program(self, kind: str, name: str, item):
@@ -539,6 +612,7 @@ class FusedStep:
         s(K["GFB_B_DONES"], getattr(env, "dones", None))
         s(K["GFB_B_EXT_VALUES"], self.ext_values)
         s(K["GFB_B_OBS_EXT0"], self.ext_obs)
+        s(K["GFB_B_OBS_EXT1"], self.user_obs_values)
 
     def bind_action_buffers(self):
         K = nat.K
@@ -574,6 +648,8 @@ class FusedStep:
              self.action is None or self.action.enabled, [m.enabled for m in self.commands]),
             [(om.noise, om.enabled) for om in self.observations],
             [(i.scale, i.noise) for i in obs_items],
+            # lowered user observation terms fold their params in: a change traces them again (pack)
+            [repr(sorted(dict(self.observations[g].cfg[n].params or {}).items())) for g, n in self.user_obs],
         )
 
     def _entity_of(self, params: dict):
@@ -841,6 +917,13 @@ class FusedStep:
 
         # observations
         P.n_obs_groups = len(self.observations)
+        if self.user_obs:
+            import hashlib
+
+            progs = {key: self._user_obs_program(*key, self.observations[key[0]].cfg[key[1]]) for key in self.user_obs}
+            text = "".join(f"{self.user_obs[k][2]}:{self.user_obs[k][3]}:{progs[k].digest()};" for k in sorted(progs))
+            uid = int.from_bytes(hashlib.sha1(text.encode()).digest()[:4], "little") & 0x7FFFFFFF
+            self._obs_user_id = uid or 1  # structural: the specialised kernels are matched on it
         col = 0
         src_of = {
             "targets": K["GFB_O_TARGETS"], "dof_pos": K["GFB_O_DOF_POS"], "dof_vel": K["GFB_O_DOF_VEL"],
@@ -851,6 +934,7 @@ class FusedStep:
             og = P.obs_group[g]
             cols = om.columns() if om.enabled else []
             og.n_cols, og.history, og.col_begin = len(cols), om._history_len, col
+            og.user_id = self._obs_user_id
             if col + len(cols) > nat.MAX_OBS_COLS:
                 raise UnsupportedTermError(f"more than {nat.MAX_OBS_COLS} observation columns")
             for c in cols:
@@ -861,6 +945,9 @@ class FusedStep:
                     oc.src, oc.mgr = K["GFB_O_COMMAND"], self._command_index(key[1], "observation")
                 elif isinstance(key, tuple) and key[0] == "contact_norm":
                     oc.src, oc.mgr = K["GFB_O_CONTACT_NORM"], self._contact_index(key[1], "observation")
+                elif isinstance(key, tuple) and key[0] == "external" and (g, key[1]) in self.user_obs:
+                    oc.src, oc.mgr = K["GFB_O_USER"], self.user_obs_width
+                    oc.col = self.user_obs[(g, key[1])][2] + c["col"]
                 elif isinstance(key, tuple) and key[0] == "external":
                     oc.src, oc.mgr = K["GFB_O_EXTERNAL"], self.ext_obs_width
                     oc.col = om._external_col0[key[1]] + c["col"]
@@ -880,7 +967,9 @@ class FusedStep:
         self._keepalive = []
         robot = self.primary_entity
         f32 = torch.float32
-        if not post_reset:  # the re-observation of reset envs reads the cached quaternion, not pos/quat
+        # the re-observation of reset envs reads the cached quaternion, not pos/quat -- except lowered user
+        # observation terms that read the engine's pose
+        if not post_reset or self._obs_reads_pose:
             s(B["GFB_B_POS"], robot.get_pos(), f32)
             s(B["GFB_B_QUAT"], robot.get_quat(), f32)
         s(B["GFB_B_VEL"], robot.get_vel(), f32)
@@ -1148,12 +1237,16 @@ class FusedStep:
             tuple(item.version for _, item, _ in self.termination_terms),
             tuple(m._external_controller is None for m in self.commands),
             self._contact_dims,
+            self._obs_user_id,
         )
 
     def spec_stats(self) -> dict:
-        a, b = C.c_int64(), C.c_int64()
-        self.lib.gfb_spec_stats(self.handle.ptr, C.byref(a), C.byref(b))
-        return {"specialised_launches": a.value, "generic_launches": b.value, "libraries": [p.name for p in self.spec_paths]}
+        a, b, u = C.c_int64(), C.c_int64(), C.c_int64()
+        self.lib.gfb_spec_stats(self.handle.ptr, C.byref(a), C.byref(b), C.byref(u))
+        stats = {"specialised_launches": a.value, "generic_launches": b.value, "libraries": [p.name for p in self.spec_paths]}
+        if self.user_obs:  # the reset path's kernel of the lowered observation terms (gfb_observe)
+            stats["user_observe_launches"] = u.value
+        return stats
 
     def evaluate_external(self, kind: str):
         """Run the user-defined reward / termination functions; their values become kernel inputs."""
@@ -1207,7 +1300,7 @@ class FusedStep:
         phases &= self._phase_mask
         first = self.first_launch_of_step
         self.first_launch_of_step = False
-        if first and self.user_terms and self.split_mode:
+        if first and self.lowered_user_terms and self.split_mode:
             # a later launch of the split step evaluates the lowered terms: check before anything is launched
             why = self._user_terms_blocked()
             if why is not None:
@@ -1223,7 +1316,7 @@ class FusedStep:
         stream = self._stream()
         rc = self.lib.gfb_post_physics(self._h, self._buffers_ref, phases, stream)
         if rc:
-            if first and rc == nat.K["GFB_ERR_UNSUPPORTED"] and self.user_terms and not self.split_mode:
+            if first and rc == nat.K["GFB_ERR_UNSUPPORTED"] and self.lowered_user_terms and not self.split_mode:
                 # the one launch of the fused step was refused before anything ran: no specialised kernel
                 # matched the table with its lowered terms (not attached, or the launch cannot use TMA)
                 why = self.lib.gfb_last_error(self._h).decode()
@@ -1259,7 +1352,17 @@ class FusedStep:
         self._obs_buffers()
         self._injection_buffers()
         self._set_program()
+        if self.user_obs:  # the lowered observation terms' reset path is a kernel of the table's specialised library
+            K = nat.K
+            self._maybe_specialise(K["GFB_PHASE_OBSERVE"] if self.split_mode else self.step_phases & self._phase_mask)
         rc = self.lib.gfb_observe(self._h, self._buffers_ref, idx.data_ptr() if idx is not None else None, n, self._stream())
+        if rc == nat.K["GFB_ERR_UNSUPPORTED"] and self.user_obs:
+            # no specialised library for the lowered terms: they become host columns (split execution from now on)
+            self._demote_user_terms(self.lib.gfb_last_error(self._h).decode())
+            self.evaluate_external_obs()
+            self._set_program()
+            rc = self.lib.gfb_observe(self._h, self._buffers_ref, idx.data_ptr() if idx is not None else None, n,
+                                      self._stream())
         if rc:
             self.handle.check(rc, "gfb_observe")
 
@@ -1301,6 +1404,8 @@ class FusedStep:
     def _rotate(self, vec, quat, conjugate: int) -> torch.Tensor:
         quat = quat.to(self.device, torch.float32).contiguous()
         n = quat.shape[0]
+        if self.width_probe:  # a dry run's width probe of a user observation term: no device, the shape only
+            return torch.zeros((n, 3), device=self.device)
         out = torch.empty((n, 3), device=self.device)
         vptr = None
         if vec is not None:
@@ -1518,11 +1623,12 @@ class FusedStep:
         self.handle.check(self.lib.gfb_profile_enable(self.handle.ptr, 1 if enabled else 0), "gfb_profile_enable")
 
     def profile_read_aux(self) -> dict:
-        """Average device time (us) of the small kernels since profiling was enabled."""
-        ms, n = (C.c_float * 3)(), (C.c_int32 * 3)()
+        """Average device time (us) of the small kernels since profiling was enabled (the reset path of lowered
+        user observation terms only for tables that have them)."""
+        ms, n = (C.c_float * 4)(), (C.c_int32 * 4)()
         self.handle.check(self.lib.gfb_profile_read_aux(self.handle.ptr, ms, n), "gfb_profile_read_aux")
-        return {name: {"kernel_us": ms[k] / max(n[k], 1) * 1e3, "launches": n[k]}
-                for k, name in enumerate(("compact_kernel", "observe_kernel", "spawn_kernel"))}
+        names = ("compact_kernel", "observe_kernel", "spawn_kernel") + (("user_observe_kernel",) if self.user_obs else ())
+        return {name: {"kernel_us": ms[k] / max(n[k], 1) * 1e3, "launches": n[k]} for k, name in enumerate(names)}
 
     def profile_read(self) -> dict:
         post_ms, act_ms = C.c_float(), C.c_float()

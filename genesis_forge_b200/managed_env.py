@@ -45,6 +45,11 @@ class ManagedEnvironment(GenesisEnv):
     # post-physics kernel next to the stock terms; a table without other host callbacks is then one launch
     # per step again.  Terms the IR does not cover stay callbacks (FusedStep.user_term_refusals says why).
     fuse_user_terms = os.environ.get("GFB_FUSE_USER_TERMS", "0") == "1"
+    # The same for user-defined observation functions (independent of fuse_user_terms): with this set to True
+    # -- or GFB_FUSE_USER_OBS=1 in the environment -- the ones that lower are evaluated by the specialised
+    # kernel instead of the host, and re-observed reset envs by a small kernel of the same library
+    # (FusedStep.user_term_refusals[("observation", name)] says why a term stays a host column).
+    fuse_user_observations = os.environ.get("GFB_FUSE_USER_OBS", "0") == "1"
 
     def __init__(
         self,

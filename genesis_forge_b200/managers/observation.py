@@ -41,6 +41,9 @@ class ObservationManager(BaseManager):
         self._buffers: list[torch.Tensor] = []            # ping-pong (N, O*H) rows
         self._current = 0
         self._external_col0: dict[str, int] = {}          # user-defined terms: first column in the host-filled array
+        # host-evaluated terms that are not user functions (body-frame terms without an entity_manager, terms of
+        # a further EntityManager): never lowered into the kernel (FusedStep, fuse_user_observations)
+        self._host_columns: set[str] = set()
 
     @property
     def name(self) -> str:
@@ -57,6 +60,7 @@ class ObservationManager(BaseManager):
     def build(self):
         self._sources = []
         self._pending: list[str] = []
+        self._host_columns = set()
         for name, cfg in self.cfg.items():
             cfg.build()
             assert callable(cfg.fn), f"Observation function {name} is not callable"
@@ -67,6 +71,8 @@ class ObservationManager(BaseManager):
                 key, width = ("external", name), getattr(e, "width", None)
                 if width is None:
                     self._pending.append(name)
+                else:
+                    self._host_columns.add(name)
             self._sources.append((name, key, width))
         if not self._pending:
             self._allocate()
@@ -78,7 +84,12 @@ class ObservationManager(BaseManager):
             return
         for i, (name, key, width) in enumerate(self._sources):
             if name in self._pending:
-                value = self.cfg[name].fn(env=self.env, **self.cfg[name].params)
+                fused = self.env._fused
+                fused.width_probe = fused.dry_run  # (a dry run cannot launch: shapes only)
+                try:
+                    value = self.cfg[name].fn(env=self.env, **self.cfg[name].params)
+                finally:
+                    fused.width_probe = False
                 self._sources[i] = (name, key, int(value.reshape(self.env.num_envs, -1).shape[1]))
         self._pending = []
         self._allocate()

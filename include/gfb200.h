@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define GFB_ABI_VERSION 12
+#define GFB_ABI_VERSION 13
 
 /* ---- limits ------------------------------------------------------------------------------- */
 #define GFB_MAX_DOFS 32
@@ -170,7 +170,11 @@ typedef enum {
   GFB_O_TARGETS,       /* action_manager.get_actions(): processed targets                  */
   GFB_O_ENV_ACTIONS,   /* env.actions (raw)                                                */
   GFB_O_CONTACT_NORM,  /* |contacts[mgr][:, col]|  observations.py:181-193                 */
-  GFB_O_EXTERNAL       /* column `col` of GFB_B_OBS_EXT0, a (N, mgr) array of host-evaluated terms */
+  GFB_O_EXTERNAL,      /* column `col` of GFB_B_OBS_EXT0, a (N, mgr) array of host-evaluated terms */
+  GFB_O_USER           /* word `col` of the (N, mgr) values of the lowered user-defined observation terms
+                          (genesis_forge_b200/expr.py): the post kernel's owner threads compute them into the
+                          stash; gfb_observe has the specialised library compute them into GFB_B_OBS_EXT1.
+                          Only a specialised kernel generated for them evaluates them (obs_group.user_id). */
 } gfb_obs_src;
 
 /* gfb_program_head.manager_flags */
@@ -239,7 +243,9 @@ typedef struct {
   int32_t n_cols;    /* O_g: width of one frame                     */
   int32_t history;   /* H_g >= 1 (observation_manager.py:152-153)   */
   int32_t col_begin; /* first entry in gfb_program.obs_cols         */
-  int32_t _pad;
+  int32_t user_id;   /* identity of the lowered user-defined observation terms (GFB_O_USER columns) of
+                        the table, nonzero in every group when it has any; 0 otherwise.  Structural: part
+                        of what a specialised kernel is matched on */
 } gfb_obs_group;
 
 /* The packed term table ("program").  Re-packed by the host every step from the live Python
@@ -412,7 +418,10 @@ int gfb_peer_disconnect(gfb_handle* h);
 /* Observation rows for a list of envs (idx == NULL: all envs) from the CURRENT engine state and
  * the cached inverse base quaternion.  Used after the engine-side reset writes for the envs in
  * GFB_B_RESET_IDX (observations are taken after reset, managed_env.py:322-326) and for the
- * initial get_observations().  Only frame 0 of each group is written.                          */
+ * initial get_observations().  Only frame 0 of each group is written.  A program with GFB_O_USER
+ * columns first has the attached specialised library whose structure matches the program compute
+ * the lowered user terms of those envs into GFB_B_OBS_EXT1 ((N, w) rows, from global memory only);
+ * without one the call is refused (GFB_ERR_UNSUPPORTED) before anything runs.                     */
 int gfb_observe(gfb_handle* h, const gfb_buffers* b, const int64_t* idx, int32_t n, void* stream);
 
 /* Contact net-force scatter alone, with the reference kernel's own argument list
@@ -498,16 +507,18 @@ int gfb_reset_rows(gfb_handle* h, const int64_t* idx, int32_t n, int32_t width, 
 int gfb_spec_describe(gfb_handle* h, const gfb_buffers* b, uint32_t phases, void* canonical_head,
                       int32_t* plan_out, int32_t plan_cap, int32_t* plan_words, int32_t* tile);
 int gfb_spec_attach(gfb_handle* h, const char* path);
-/* number of gfb_post_physics launches so far that ran a specialised / the generic kernel */
-int gfb_spec_stats(const gfb_handle* h, int64_t* specialised, int64_t* generic);
+/* number of gfb_post_physics launches so far that ran a specialised / the generic kernel, and of
+ * gfb_observe calls that ran a specialised library's lowered user-defined observation terms */
+int gfb_spec_stats(const gfb_handle* h, int64_t* specialised, int64_t* generic, int64_t* user_observe);
 
 /* Timing instrumentation: when enabled, each launch of gfb_post_physics' fused kernel is bracketed
  * by CUDA events on its stream; gfb_profile_read returns the accumulated device time.          */
 int gfb_profile_enable(gfb_handle* h, int32_t enabled);
 int gfb_profile_read(gfb_handle* h, float* post_ms_total, int32_t* post_launches, float* action_ms_total,
                      int32_t* action_launches);
-/* Same for the small kernels; ms_total / launches are arrays of 3: [0] index compaction (behind
- * the post kernel), [1] observe (gfb_observe), [2] spawn (gfb_spawn_pose).                       */
+/* Same for the small kernels; ms_total / launches are arrays of 4: [0] index compaction (behind
+ * the post kernel), [1] observe (gfb_observe), [2] spawn (gfb_spawn_pose), [3] the lowered user-
+ * defined observation terms of gfb_observe (specialised library).                                */
 int gfb_profile_read_aux(gfb_handle* h, float* ms_total, int32_t* launches);
 /* kernels launched by this handle since creation (gfb_action_step: 1, gfb_post_physics: 1-2, ...) */
 int64_t gfb_launch_count(const gfb_handle* h);

@@ -1,13 +1,17 @@
 """
 env.step of the user-terms workload (configs/user_terms.py) with its user-defined rewards / terminations
 as host callbacks (split execution, fuse_user_terms off) and lowered into the specialised post-physics
-kernel (fuse_user_terms on), at 65,536 and 1,048,576 envs.  The two modes are built side by side and
+kernel (fuse_user_terms on), at 65,536 and 1,048,576 envs.  `--workload user_observations` does the same
+for workload A of configs/user_observations.py (fuse_user_observations), adds the stock `contacts` table
+as a third, reference environment for the post-physics kernel's time, and reports the reset-path kernel
+of the lowered observation terms.  The two modes are built side by side and
 timed alternately in one process (CUDA events around `steps` steps, in-kernel Philox draws as bench.py
 runs them, on bench.py's pool of pre-generated state sets); the post-physics kernel's device time comes
 from the library's own event brackets.  The outputs of one more step of both modes (same states, same
 actions, same draws) are compared.
 
-    python tools/user_terms_bench.py [--sizes 65536 1048576] [--steps 50] [--warmup 10] [--rounds 3]
+    python tools/user_terms_bench.py [--workload user_terms|user_observations] [--sizes 65536 1048576]
+                                     [--steps 50] [--warmup 10] [--rounds 3]
 """
 from __future__ import annotations
 
@@ -35,25 +39,29 @@ def gpu_info() -> dict:
     return info
 
 
-def make_env(n: int, fuse: bool, dev):
+def make_env(n: int, mode: str, dev, workload: str = "user_terms"):
     import genesis_forge_b200 as gfb
-    from configs import user_terms
+    from configs import specs, user_observations, user_terms
     from configs.env_builder import build_env, dropin_namespace
     from genesis_forge_b200.managed_env import ManagedEnvironment
 
-    ManagedEnvironment.fuse_user_terms = fuse
+    obs = workload == "user_observations"
+    ManagedEnvironment.fuse_user_terms = mode == "fused" and not obs
+    ManagedEnvironment.fuse_user_observations = mode == "fused" and obs
     gfb.set_device(dev)
+    spec = specs.contacts() if mode == "stock" else (user_observations.user_observations() if obs
+                                                     else user_terms.user_terms())
     # as bench.py: a pool of pre-generated state sets rotated by scene.step() (the same states for both modes),
     # engine-side reset writes accepted but not applied
-    env = build_env(user_terms.user_terms(), dropin_namespace(), n, dev, pool=4, seed=7, n_contacts=8,
-                    apply_setters=False)
+    env = build_env(spec, dropin_namespace(), n, dev, pool=4, seed=7, n_contacts=8, apply_setters=False)
     env.build()
     env.reset()
     return env
 
 
-def timed(env, actions, steps: int) -> tuple[float, float, int]:
-    """(ms per step, post-physics kernel ms per step, post-physics launches per step)"""
+def timed(env, actions, steps: int) -> tuple[float, float, int, float]:
+    """(ms per step, post-physics kernel ms per step, post-physics launches per step, reset-path kernel us per
+    launch of the lowered observation terms or 0)"""
     import torch
 
     fused = env._fused
@@ -66,9 +74,11 @@ def timed(env, actions, steps: int) -> tuple[float, float, int]:
     end.record()
     end.synchronize()
     after = fused.profile_read()
+    user_us = fused.profile_read_aux().get("user_observe_kernel", {}).get("kernel_us", 0.0)
     fused.profile(False)
     launches = after["post_launches"] - before["post_launches"]
-    return (start.elapsed_time(end) / steps, (after["post_ms"] - before["post_ms"]) / steps, launches // steps)
+    return (start.elapsed_time(end) / steps, (after["post_ms"] - before["post_ms"]) / steps, launches // steps,
+            user_us)
 
 
 def main():
@@ -79,11 +89,13 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--workload", choices=["user_terms", "user_observations"], default="user_terms")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     print(json.dumps({"gpu": gpu_info()}), flush=True)
     for n in args.sizes:
-        envs = {mode: make_env(n, mode == "fused", dev) for mode in ("split", "fused")}
+        modes = ("split", "fused") + (("stock",) if args.workload == "user_observations" else ())
+        envs = {mode: make_env(n, mode, dev, args.workload) for mode in modes}
         print(f"# N={n}: both environments built", flush=True)
         assert envs["split"]._fused.split_mode and not envs["fused"]._fused.split_mode
         gen = torch.Generator(device=dev).manual_seed(5)
@@ -97,7 +109,7 @@ def main():
                 rows[mode].append(timed(env, actions, args.steps))
                 print(f"# N={n} round {r} {mode}: {rows[mode][-1]}", flush=True)
         # same seeded state and actions through both modes: compare one more step's outputs
-        outs = {mode: env.step(actions[0]) for mode, env in envs.items()}
+        outs = {mode: envs[mode].step(actions[0]) for mode in ("split", "fused")}
         a, b = outs["split"], outs["fused"]
         diff = {
             "rewards_max_abs": float((a[1] - b[1]).abs().max()),
@@ -105,13 +117,17 @@ def main():
             "truncated_equal": bool(torch.equal(a[3], b[3])),
             "obs_max_abs": float((a[0] - b[0]).abs().max()),
         }
-        result = {"num_envs": n, "steps": args.steps, "rounds": args.rounds, "compare": diff}
+        result = {"workload": args.workload, "num_envs": n, "steps": args.steps, "rounds": args.rounds,
+                  "compare": diff}
         for mode, r in rows.items():
             ms = sorted(x[0] for x in r)[len(r) // 2]
             post = sorted(x[1] for x in r)[len(r) // 2]
             result[mode] = {"ms_per_step_median": round(ms, 4), "env_steps_per_s": round(n / ms * 1e3),
                             "post_kernel_ms_per_step_median": round(post, 4), "post_launches_per_step": r[0][2],
                             "ms_per_step_all": [round(x[0], 4) for x in r]}
+            if args.workload == "user_observations" and mode == "fused":
+                result[mode]["user_observe_kernel_us_median"] = round(sorted(x[3] for x in r)[len(r) // 2], 2)
+                result[mode]["spec_stats"] = envs[mode]._fused.spec_stats()
         print(json.dumps(result), flush=True)
         del envs
         torch.cuda.empty_cache()
