@@ -73,6 +73,7 @@ struct AttachedSpec {
   int (*blocks_per_sm)(unsigned) = nullptr;
   // reset path of the lowered user-defined observation terms (spec_kernel.cu), if the library has them
   int (*user_observe)(const gfb_buffers*, int, const int64_t*, int, int, void*) = nullptr;
+  uint32_t state_slots = 0;  // GFB_B_USER_STATE slots its lowered class-style terms use (bit i: slot i)
   int tile = 0;
   uint32_t phases = 0;
   gfb_program_head canon;
@@ -1072,6 +1073,12 @@ int gfb_post_physics(gfb_handle* h, const gfb_buffers* b, uint32_t phases, void*
 
   const int n_tiles = (P.num_envs + tile - 1) / tile;
   const AttachedSpec* spec = lc->spec_index >= 0 ? &h->specs[lc->spec_index] : nullptr;
+  if (spec && spec->state_slots)  // the kernel reads and writes these rows in place
+    for (int i = 0; i < 8; ++i)
+      if (((spec->state_slots >> i) & 1u) && !b->buf[GFB_B_USER_STATE0 + i])
+        return fail(h, GFB_ERR_INVALID,
+                    "buffer USER_STATE" + std::to_string(i) + " is NULL (the attached specialised kernel keeps the "
+                    "state of a lowered class-style term there)");
   // persistent grid: every block of the launch is resident from the start (the in-kernel ordered
   // compaction relies on it: a slab only waits for slabs that are already running)
   if (lc->resident_blocks == 0) {
@@ -1497,6 +1504,7 @@ int gfb_spec_attach(gfb_handle* h, const char* path) {
   sp.blocks_per_sm = reinterpret_cast<int (*)(unsigned)>(dlsym(dl, "gfb_spec_blocks_per_sm"));
   sp.user_observe = reinterpret_cast<int (*)(const gfb_buffers*, int, const int64_t*, int, int, void*)>(
       dlsym(dl, "gfb_spec_user_observe"));
+  if (auto slots = reinterpret_cast<unsigned (*)(void)>(dlsym(dl, "gfb_spec_state_slots"))) sp.state_slots = slots();
   h->specs.push_back(sp);
   h->spec_gen += 1;
   return GFB_OK;

@@ -150,6 +150,7 @@ struct UserCtx {
   const Plan& plan;
   const float* p;
   int n_envs;  // (global-memory reads of the air-time planes)
+  bool active;  // a real env: lanes that shadow env N-1 in a tail slab do not store state
 };
 
 // First stash word of the lowered user-defined observation values (gfb200.cu build_plan: st_user)
@@ -648,7 +649,7 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
 #if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
         case GFB_T_USER:  // user-defined term lowered to device code (generated header)
           v = user_termination(t, UserCtx{K.b, (size_t)e, ep_len, max_len, false, false, iw, iq, lin_b, ang_b, grav_b, S, tid,
-                                          st, plan, tt.p});
+                                          st, plan, tt.p, N, active});
           break;
 #endif
         default:
@@ -879,7 +880,7 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
 #if defined(GFB_SPEC) && defined(GFB_SPEC_USER_TERMS)
         case GFB_R_USER:  // user-defined term lowered to device code (generated header)
           v = user_reward(r, UserCtx{K.b, (size_t)e, ep_len, max_len, terminated, truncated, iw, iq, lin_b, ang_b, grav_b,
-                                     S, tid, st, plan, rt.p});
+                                     S, tid, st, plan, rt.p, N, active});
           break;
 #endif
         default:
@@ -1004,7 +1005,7 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
   // command, the body-frame registers, the staged rows) into the stash words the GFB_O_USER columns read
   if (ph & GFB_PHASE_OBSERVE)
     user_observations(UserCtx{K.b, (size_t)e, ep_len, max_len, terminated, truncated, iw, iq, lin_b, ang_b, grav_b, S,
-                              tid, st, plan, nullptr, N},
+                              tid, st, plan, nullptr, N, active},
                       st + user_stash_base(SP));
 #endif
 

@@ -6,7 +6,8 @@
 // post_kernel.cuh then reads structure from those constants (term loops unroll, switches fold,
 // shared-memory offsets become immediates) and live values from the kernel parameters as usual.
 // A table with lowered user-defined observation terms (GFB_SPEC_USER_OBS) also exports
-// gfb_spec_user_observe, their reset path for gfb_observe.
+// gfb_spec_user_observe, their reset path for gfb_observe.  gfb_spec_state_slots is the mask of the
+// GFB_B_USER_STATE slots the lowered class-style terms read and write (GFB_SPEC_STATE_SLOTS, 0 without).
 #include <cuda_runtime.h>
 
 #include "../../include/gfb200.h"
@@ -34,6 +35,11 @@ extern "C" int gfb_spec_info(int* tile, unsigned* phases, const void** canon, co
   *plan_bytes = (int)sizeof(gfb::Plan);
   return 0;
 }
+
+#ifndef GFB_SPEC_STATE_SLOTS
+#define GFB_SPEC_STATE_SLOTS 0u
+#endif
+extern "C" unsigned gfb_spec_state_slots(void) { return GFB_SPEC_STATE_SLOTS; }
 
 extern "C" int gfb_spec_blocks_per_sm(unsigned smem) {
   if ((int)smem > 44 * 1024 && (int)smem > smem_attr) {
@@ -65,7 +71,7 @@ __global__ void __launch_bounds__(128) user_observe_kernel(const __grid_constant
   const gfb::V3 zero = {0.f, 0.f, 0.f};
   gfb::user_observations_global(
       gfb::UserCtx{b, e, ep_len, max_len, false, false, q.x, gfb::V3{q.y, q.z, q.w}, zero, zero, zero, nullptr, 0,
-                   nullptr, gfb_spec::kPlan, nullptr, num_envs},
+                   nullptr, gfb_spec::kPlan, nullptr, num_envs, true},
       reinterpret_cast<float*>(b.buf[GFB_B_OBS_EXT1]) + e * GFB_SPEC_USER_OBS);
 }
 }  // namespace

@@ -27,6 +27,15 @@ unsqueeze, None in an index and reshape / view / flatten of a row.  Their params
 again when they change).  Their device code comes twice: for the owner phase of post_kernel and, reading
 global memory only, for the reset path that re-observes reset envs (spec_kernel.cu).
 
+Class-style reward / termination terms (an MdpFnClass instance, ManagedEnvironment.fuse_stateful_terms) are
+traced through `type(inst).__call__`.  A per-env tensor attribute of the instance -- (N, *s) with at most
+MAX_CONST_VEC elements a row, fp32 / int32 / bool, on the env's device and contiguous -- is a source
+("state", slot); rebinding it to a value of the same row shape and dtype, `self.x[:] = v` and `self.x.copy_(v)`
+are state writes (`Program.writes`), stored to the env's row after the result is computed.  An attribute
+that is None and gets a per-env value during the call (lazy initialisation) gives a second, first-call
+program (`Program.first`), which the kernel selects while the term's p[0] is 0.  Python-scalar attributes
+and params are trace constants.
+
 Anything outside this subset raises UnsupportedTermError naming the op or source; the term then
 stays a host callback (split execution), with exactly the results it had before.
 """
@@ -44,6 +53,7 @@ F32, I32, BOOL = "f32", "i32", "bool"
 _RANK = {BOOL: 0, I32: 1, F32: 2}
 MAX_CONST_VEC = 32  # GFB_MAX_DOFS: small constant vectors (per-joint limits, gains) are folded in
 MAX_LIVE_PARAMS = 4  # gfb_reward_term.p / gfb_termination_term.p
+MAX_STATE_SLOTS = 8  # GFB_B_USER_STATE0..7
 # bumped whenever `function_body` emits different code for the same IR: the digest changes with it
 CODEGEN_REVISION = 2
 
@@ -73,13 +83,22 @@ class Node:
 class Program:
     """The IR of one term: nodes in evaluation order, the result node, the live parameter names."""
 
-    def __init__(self, kind: str, nodes: list, out: int, params: list[str], param_types: list[str]):
+    def __init__(self, kind: str, nodes: list, out: int, params: list[str], param_types: list[str],
+                 writes: list | None = None):
         self.kind, self.nodes, self.out = kind, nodes, out
         self.params, self.param_types = params, param_types
+        self.writes = writes or []  # [(state slot, node)]: the env's row of the slot after the call
+        self.first = None  # lazily initialised state: the program of the term's first evaluation
+        self.bindings: dict = {}  # class-style terms: attribute -> (slot, row shape, dtype, lazy)
 
     def text(self) -> str:
         head = f"{self.kind} params={self.params} types={self.param_types} out=%{self.out}\n"
-        return head + "\n".join(n.text(i) for i, n in enumerate(self.nodes))
+        text = head + "\n".join(n.text(i) for i, n in enumerate(self.nodes))
+        if self.writes:
+            text += "\nwrites " + ", ".join(f"state{slot}=%{i}" for slot, i in self.writes)
+        if self.first is not None:
+            text += "\nfirst call:\n" + self.first.text()
+        return text
 
     def digest(self) -> int:
         """31-bit identity of the expression and of the code `function_body` emits for it (stored in the
@@ -177,7 +196,18 @@ class Sym:
         raise UnsupportedTermError("user term: iteration over a per-env value")
 
     def __setitem__(self, key, value):
-        raise UnsupportedTermError("user term: in-place write (__setitem__)")
+        if id(self) not in self._tr.state_objs:
+            raise UnsupportedTermError("user term: in-place write (__setitem__)")
+        keys = key if isinstance(key, tuple) else (key,)
+        if not all(k == slice(None) or k is Ellipsis for k in keys) or len(keys) > len(self.shape):
+            raise UnsupportedTermError(f"user term: partial in-place write of state ([{key!r}] = ...)")
+        self._tr.state_write(self, value)
+
+    def copy_(self, src, non_blocking=False):
+        if id(self) not in self._tr.state_objs:
+            raise UnsupportedTermError("user term: in-place op copy_")
+        self._tr.state_write(self, src)
+        return self
 
     def __getattr__(self, name):
         if name.startswith("__"):
@@ -233,7 +263,7 @@ class Sym:
     def int(self): return self._tr.cast(self, I32)
     def bool(self): return self._tr.cast(self, BOOL)
     def detach(self): return self
-    def clone(self): return self
+    def clone(self): return Sym(self._tr, self._id)  # a copy: it does not follow an in-place write of state
     def contiguous(self): return self
 
     def clamp(self, min=None, max=None): return self._tr.clamp(self, min, max)
@@ -267,7 +297,10 @@ class Sym:
         return self._tr.cast(self, _dtype_of(dtype))
 
     def __getitem__(self, key):
-        return self._tr.index(self, key)
+        out = self._tr.index(self, key)
+        if out is not self and id(self) in self._tr.state_objs:  # a view: it would follow an in-place write
+            self._tr.viewed.add(self._tr.state_objs[id(self)][0])
+        return out
 
     # -- layout (observation terms) --------------------------------------------------------------
     def unsqueeze(self, dim): return self._tr.unsqueeze(self, dim)
@@ -327,6 +360,8 @@ class Tracer:
         self._cse: dict = {}
         self.params: list[str] = []
         self.param_types: list[str] = []
+        self.state_objs: dict = {}  # id(Sym) -> (slot, Sym): the instance's state tensors
+        self.viewed: set = set()  # state slots a view was taken of
 
     def add(self, op, args, attr, shape, dtype, weak=False) -> Sym:
         key = (op, tuple(args), repr(attr), tuple(shape), dtype, weak)
@@ -339,6 +374,28 @@ class Tracer:
 
     def source(self, key: tuple, shape: tuple, dtype: str) -> Sym:
         return self.add("src", (), key, shape, dtype)
+
+    def state_write(self, sym: Sym, value):
+        """`self.x[:] = value` / `self.x.copy_(value)`: the state Sym stands for the written value from now on."""
+        slot, _ = self.state_objs[id(sym)]
+        if slot in self.viewed:
+            raise UnsupportedTermError("user term: in-place write of state a view was taken of")
+        v = self.lift(value)
+        if v.shape_ != sym.shape_ or (v.weak and sym.shape_):
+            raise UnsupportedTermError(f"user term: in-place write of a {tuple(v.shape)} value into state of shape "
+                                       f"{tuple(sym.shape)}")
+        sym._id = self.cast(v, sym.dtype_)._id
+
+    def full(self, like, value, dtype=None) -> Sym:
+        """torch.zeros_like / ones_like / full_like of a per-env value."""
+        like = self.lift(like)
+        if like.weak:
+            raise UnsupportedTermError("user term: *_like of a Python scalar")
+        if isinstance(value, Sym) or not isinstance(value, (bool, int, float)):
+            raise UnsupportedTermError("user term: full_like with a non-constant fill value")
+        dt = _dtype_of(dtype) if dtype is not None else like.dtype_
+        value = bool(value) if dt == BOOL else (int(value) if dt == I32 else _f32(value))
+        return self.add("full", (), value, like.shape_, dt)
 
     def param(self, name: str, value) -> Sym:
         dtype = I32 if isinstance(value, int) else F32
@@ -690,6 +747,13 @@ class Tracer:
             return self.index(self.lift(args[0]), args[1])
         if name == "nonzero":
             raise UnsupportedTermError("user term: nonzero() (data-dependent shape)")
+        if name in ("zeros_like", "ones_like", "full_like"):
+            value = {"zeros_like": 0, "ones_like": 1}.get(name)
+            if value is None:
+                value = args[1] if len(args) > 1 else kwargs.get("fill_value")
+            return self.full(args[0], value, kwargs.get("dtype"))
+        if name == "clone":
+            return self.lift(args[0]).clone()
         raise UnsupportedTermError(f"user term: torch function '{name}' is not supported by the expression IR")
 
 
@@ -808,13 +872,36 @@ def param_kinds(params) -> tuple:
                         if isinstance(v, (int, float)) and not isinstance(v, bool)))
 
 
-def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> Program:
-    """Trace one user-defined reward / termination / observation into a Program (raises UnsupportedTermError)."""
+def is_class_term(fn) -> bool:
+    """An MdpFnClass instance (or a builtin): not a plain function."""
+    return not hasattr(getattr(fn, "__func__", fn), "__code__")
+
+
+class StateSlots:
+    """The GFB_B_USER_STATE slots a class-style term may take: its own (by attribute) first, then free ones."""
+
+    def __init__(self, own: dict, free: list):
+        self.own, self.free = dict(own), list(free)
+
+    def slot(self, attr: str) -> int:
+        if attr not in self.own:
+            if not self.free:
+                raise UnsupportedTermError(f"user term: more state tensors than the {MAX_STATE_SLOTS} slots of the "
+                                           "ABI (GFB_B_USER_STATE0..7)")
+            self.own[attr] = self.free.pop(0)
+        return self.own[attr]
+
+
+def trace_term(fused, kind: str, name: str, item, live_params: bool = True, state: StateSlots | None = None) -> Program:
+    """Trace one user-defined reward / termination / observation into a Program (raises UnsupportedTermError).
+    `state`: the slots a class-style reward / termination term may bind (None: class-style terms are refused)."""
     env = fused.env
     fn = item.fn
     what = f"{kind} '{name}'"
-    if not hasattr(getattr(fn, "__func__", fn), "__code__"):  # an MdpFnClass instance (or a builtin)
-        raise UnsupportedTermError(f"{what}: class-style terms keep their own state and are not lowered")
+    if is_class_term(fn):
+        if state is None or kind == "observation" or isinstance(fn, type):
+            raise UnsupportedTermError(f"{what}: class-style terms keep their own state and are not lowered")
+        return _trace_stateful(fused, kind, what, item, state)
     tr = Tracer(fused.N, kind, fused.device)
     params = {}
     for k, v in dict(item.params or {}).items():
@@ -843,6 +930,14 @@ def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> P
         out = tr.cast(tr._as_row((width,), result), F32)._id
         nodes = _live_nodes(tr.nodes, out)
         return Program(kind, nodes[0], nodes[1], [], [])
+    return _term_program(tr, kind, what, result)
+
+
+def _term_program(tr: Tracer, kind: str, what: str, result, writes: dict | None = None) -> Program:
+    """The Program of a reward / termination's result (and of its state writes {slot: node})."""
+    if not isinstance(result, Sym):
+        raise UnsupportedTermError(f"{what}: the result does not depend on per-env state the kernel holds "
+                                   f"({type(result).__name__})")
     if result.weak or result.shape_ != ():
         raise UnsupportedTermError(f"{what}: the result has shape {tuple(result.shape)}, not (N,)")
     if kind == "termination" and result.dtype_ != BOOL:
@@ -850,8 +945,117 @@ def trace_term(fused, kind: str, name: str, item, live_params: bool = True) -> P
     out = result._id
     if kind == "reward" and result.dtype_ != F32:
         out = tr.cast(result, F32)._id
-    nodes = _live_nodes(tr.nodes, out)
-    return Program(kind, nodes[0], nodes[1], tr.params, tr.param_types)
+    slots = sorted(writes or {})
+    nodes, out, extra = _live_nodes(tr.nodes, out, [writes[s] for s in slots])
+    return Program(kind, nodes, out, tr.params, tr.param_types, list(zip(slots, extra)))
+
+
+_SCALARS = (bool, int, float, str, bytes, type(None))
+
+
+def _same(a, b) -> bool:
+    return a is b or (type(a) is type(b) and isinstance(a, _SCALARS) and a == b)
+
+
+def instance_constants(inst) -> tuple:
+    """The Python-scalar attributes of a class-style term: trace constants (a change traces it again)."""
+    return tuple((k, v) for k, v in vars(inst).items() if isinstance(v, _SCALARS) and v is not None)
+
+
+def _holds_env_rows(obj, N: int) -> bool:
+    values = obj.values() if isinstance(obj, dict) else (obj if isinstance(obj, (list, tuple, set)) else
+                                                          vars(obj).values())
+    return any(torch.is_tensor(v) and v.dim() >= 1 and v.shape[0] == N for v in values)
+
+
+def _trace_stateful(fused, kind: str, what: str, item, state: StateSlots) -> Program:
+    """
+    Trace a class-style term: `type(inst).__call__(inst, env, **params)` with the instance's per-env tensors as
+    ("state", slot) sources.  Attributes that are None and get a per-env value during the call are initialised
+    lazily: the call is traced once with them None (the first-call program) and once more with them as state.
+    """
+    env, inst, N = fused.env, item.fn, fused.N
+    params = dict(item.params or {})
+    before = dict(vars(inst))
+    known = {id(env)} | {id(v) for v in vars(env).values()}
+    for mgrs in getattr(env, "managers", {}).values():
+        known |= {id(m) for m in (mgrs if isinstance(mgrs, (list, tuple)) else [mgrs])}
+    rows: dict = {}  # attribute -> (row shape, dtype) of the per-env tensors
+    for attr, v in before.items():
+        if torch.is_tensor(v):
+            if v.dim() == 0 or v.shape[0] != N:
+                continue  # a constant (folded in where it is read); a write to it is refused below
+            if v.dtype == torch.int64:
+                raise UnsupportedTermError(f"{what}: state self.{attr} is int64 (the kernel's integers are 32-bit)")
+            if v.dtype not in (torch.float32, torch.int32, torch.bool):
+                raise UnsupportedTermError(f"{what}: state self.{attr} has dtype {v.dtype} (fp32, int32 or bool)")
+            if int(np.prod(v.shape[1:])) > MAX_CONST_VEC:
+                raise UnsupportedTermError(f"{what}: state self.{attr} has more than {MAX_CONST_VEC} elements a row")
+            if v.device != fused.device or not v.is_contiguous():
+                raise UnsupportedTermError(f"{what}: state self.{attr} is not a contiguous tensor on {fused.device}")
+            rows[attr] = (tuple(v.shape[1:]), _dtype_of(v.dtype))
+        elif id(v) not in known and not callable(v) and (isinstance(v, (list, tuple, set, dict))
+                                                         or hasattr(v, "__dict__")):
+            if _holds_env_rows(v, N):
+                raise UnsupportedTermError(f"{what}: per-env state inside a container or sub-object (self.{attr})")
+    ptrs = [before[a].untyped_storage().data_ptr() for a in rows]
+    if len(set(ptrs)) != len(ptrs):
+        raise UnsupportedTermError(f"{what}: two state tensors share storage")
+
+    def run(lazy_rows: dict):
+        tr = Tracer(N, kind, fused.device)
+        syms, src = {}, {}
+        for attr, (shape, dt) in {**rows, **lazy_rows}.items():
+            slot = state.slot(attr)
+            syms[attr] = tr.source(("state", slot), shape, dt)
+            src[attr] = syms[attr]._id
+            tr.state_objs[id(syms[attr])] = (slot, syms[attr])
+        swap = _Swap()
+        try:
+            _install_sources(fused, tr, swap, kind)
+            env._tracing = ExprMode(tr, fused)
+            inst.__dict__.update(syms)
+            result = type(inst).__call__(inst, env, **params)
+            after = dict(vars(inst))
+        finally:
+            env._tracing = None
+            swap.restore()
+            inst.__dict__.clear()
+            inst.__dict__.update(before)
+        writes = {}  # slot -> node of the value the env's row holds after the call
+        for attr in sorted(set(before) | set(after)):
+            old, new = before.get(attr, _MISSING), after.get(attr, _MISSING)
+            if attr in syms:
+                shape, dt = rows.get(attr) or lazy_rows[attr]
+                if not isinstance(new, Sym) or new.weak or new.shape_ != shape or new.dtype_ != dt:
+                    got = f"{new.dtype_}{list(new.shape_)}" if isinstance(new, Sym) else type(new).__name__
+                    raise UnsupportedTermError(f"{what}: self.{attr} is rebound to {got}, not {dt}{list(shape)} (its "
+                                               "row shape and dtype must stay)")
+                if new._id != src[attr]:
+                    writes[state.slot(attr)] = new._id
+            elif old is None and isinstance(new, Sym) and not lazy_rows:  # lazy initialisation (first call)
+                if new.weak or int(np.prod(new.shape_)) > MAX_CONST_VEC:
+                    raise UnsupportedTermError(f"{what}: self.{attr} is initialised to a value that is not per-env "
+                                               f"state of at most {MAX_CONST_VEC} elements a row")
+                lazy[attr] = (new.shape_, new.dtype_)
+                writes[state.slot(attr)] = new._id
+            elif not _same(old, new):
+                if torch.is_tensor(old) or torch.is_tensor(new):
+                    raise UnsupportedTermError(f"{what}: the call writes self.{attr}, which is not per-env state")
+                raise UnsupportedTermError(f"{what}: self.{attr} changes during the call (host state the kernel "
+                                           "does not keep)")
+        return tr, result, writes
+
+    lazy: dict = {}
+    tr, result, writes = run({})
+    first = None
+    if lazy:
+        first = _term_program(tr, kind, what, result, writes)
+        tr, result, writes = run(dict(lazy))
+    prog = _term_program(tr, kind, what, result, writes)
+    prog.first = first
+    prog.bindings = {attr: (state.slot(attr), shape, dt, attr in lazy) for attr, (shape, dt) in {**rows, **lazy}.items()}
+    return prog
 
 
 def lower_term(fused, kind: str, name: str, item) -> tuple[Program, bool]:
@@ -872,9 +1076,9 @@ def lower_term(fused, kind: str, name: str, item) -> tuple[Program, bool]:
         raise UnsupportedTermError(f"{kind} '{name}': Python scalar arithmetic on '{e}' inside the term") from None
 
 
-def _live_nodes(nodes: list, out: int) -> tuple[list, int]:
-    """Dead-node elimination + renumbering."""
-    keep, stack = set(), [out]
+def _live_nodes(nodes: list, out: int, extra: list | None = None) -> tuple:
+    """Dead-node elimination + renumbering (`extra`: further roots, returned renumbered as a third item)."""
+    keep, stack = set(), [out] + list(extra or [])
     while stack:
         i = stack.pop()
         if i in keep:
@@ -887,7 +1091,9 @@ def _live_nodes(nodes: list, out: int) -> tuple[list, int]:
     for old in order:
         n = nodes[old]
         new.append(Node(n.op, [remap[a] for a in n.args], n.attr, n.shape, n.dtype, n.weak))
-    return new, remap[out]
+    if extra is None:
+        return new, remap[out]
+    return new, remap[out], [remap[i] for i in extra]
 
 
 def _install_sources(fused, tr: Tracer, swap: _Swap, kind: str):
@@ -1101,8 +1307,14 @@ def function_body(prog: Program, fname: str, glob: bool = False) -> str:
         v = f"v{i}"
         ct = _CT[n.dtype]
         size = int(np.prod(n.shape)) if n.shape else 1
-        if n.op == "src":
+        if n.op == "src" and n.attr[0] == "state":  # the env's row of a class-style term's state
+            lines.append(f"const {ct}* {v}p = reinterpret_cast<const {ct}*>(c.b.buf[GFB_B_USER_STATE0 + {n.attr[1]}]) + "
+                         f"c.e * {size};")
+            exprs = [f"{v}p[{k}]" for k in range(size)]
+        elif n.op == "src":
             exprs = _src_elems(n.attr, n.shape, lines, v, glob)
+        elif n.op == "full":
+            exprs = [_lit(n.attr, n.dtype)] * size
         elif n.op == "reshape":
             exprs = list(elems[n.args[0]])
         elif n.op == "stack":
@@ -1181,7 +1393,15 @@ def function_body(prog: Program, fname: str, glob: bool = False) -> str:
         return f"__device__ __forceinline__ void {fname}(const UserCtx& c, float* out) {{\n{body}\n{stores}\n}}\n"
     ret = elems[prog.out][0]
     rtype = "bool" if prog.kind == "termination" else "float"
-    return (f"__device__ __forceinline__ {rtype} {fname}(const UserCtx& c) {{\n{body}\n  return {ret};\n}}\n")
+    stores = []
+    for slot, i in prog.writes:  # after the result; lanes that shadow env N-1 in a tail slab do not store
+        ct = _CT[prog.nodes[i].dtype]
+        row = elems[i]
+        stores.append(f"    {ct}* s{slot} = reinterpret_cast<{ct}*>(c.b.buf[GFB_B_USER_STATE0 + {slot}]) + c.e * "
+                      f"{len(row)};")
+        stores += [f"    s{slot}[{k}] = {x};" for k, x in enumerate(row)]
+    store = ("\n  if (c.active) {\n" + "\n".join(stores) + "\n  }") if stores else ""
+    return (f"__device__ __forceinline__ {rtype} {fname}(const UserCtx& c) {{\n{body}{store}\n  return {ret};\n}}\n")
 
 
 def _reduce_expr(op, terms, dtype, lines, acc) -> str:
@@ -1220,10 +1440,17 @@ def device_code(rewards: dict[int, Program], terminations: dict[int, Program],
     """The user-term functions of one table and their dispatchers, keyed by table row; the observation terms
     as (first word in the (N, obs_words) user-observation row, program), each twice (owner phase, reset path)."""
     parts = []
-    for r, prog in sorted(rewards.items()):
-        parts.append(f"/* reward row {r} */\n" + function_body(prog, f"gfb_user_r{r}"))
-    for t, prog in sorted(terminations.items()):
-        parts.append(f"/* termination row {t} */\n" + function_body(prog, f"gfb_user_t{t}"))
+    for what, progs, fn in (("reward", rewards, "gfb_user_r"), ("termination", terminations, "gfb_user_t")):
+        for r, prog in sorted(progs.items()):
+            if prog.first is None:
+                parts.append(f"/* {what} row {r} */\n" + function_body(prog, f"{fn}{r}"))
+                continue
+            # lazily initialised state: the first-call program until the host sets the term's p[0]
+            rtype = "bool" if prog.kind == "termination" else "float"
+            parts.append(f"/* {what} row {r}: first call */\n" + function_body(prog.first, f"{fn}{r}_first"))
+            parts.append(f"/* {what} row {r} */\n" + function_body(prog, f"{fn}{r}_steady"))
+            parts.append(f"__device__ __forceinline__ {rtype} {fn}{r}(const UserCtx& c) {{\n"
+                         f"  return c.p[0] != 0.0f ? {fn}{r}_steady(c) : {fn}{r}_first(c);\n}}\n")
     cases_r = "".join(f"    case {r}: return gfb_user_r{r}(c);\n" for r in sorted(rewards))
     cases_t = "".join(f"    case {t}: return gfb_user_t{t}(c);\n" for t in sorted(terminations))
     parts.append("__device__ __forceinline__ float user_reward(int r, const UserCtx& c) {\n  switch (r) {\n"

@@ -42,6 +42,7 @@ except Exception:
 
 _F32 = np.float32
 _log = logging.getLogger(__name__)
+_TORCH_DTYPE = {"f32": torch.float32, "i32": torch.int32, "bool": torch.bool}  # (expr.F32, I32, BOOL)
 
 
 def _f32(x) -> float:
@@ -177,6 +178,8 @@ class FusedStep:
         self._body_acc_started: dict[str, bool] = {}
         self._after_launch_started: list = []
         self._body_acc_terms: set = set()
+        self._lazy_started: dict = {}  # (kind, name) -> the lazily initialised state of a lowered class term exists
+        self._after_launch_lazy: set = set()
         self.entities = list(env.managers["entity"])
         self.entity_manager = self.entities[0] if self.entities else None
         self.secondary_entities = self.entities[1:]
@@ -254,6 +257,10 @@ class FusedStep:
         self.user_term_refusals: dict = {}  # (kind, name) -> why the term stays a host callback
         self._user_code = None
         self._lower_user = bool(getattr(env, "fuse_user_terms", False)) and self._can_specialise_user_terms()
+        # class-style terms (ManagedEnvironment.fuse_stateful_terms): their per-env tensors are bound to the
+        # GFB_B_USER_STATE slots and updated in place by the kernel
+        self._lower_stateful = bool(getattr(env, "fuse_stateful_terms", False)) and self._can_specialise_user_terms()
+        self.stateful: dict = {}  # (kind, name) -> {"inst", "attrs": {attr: (slot, shape, dtype, lazy)}, "tensors"}
         if self.reward is not None:
             for name, item in self.reward.cfg.items():
                 opcode = self._opcode_of(item.fn, "reward")
@@ -424,6 +431,14 @@ class FusedStep:
         self._user_code = None
         self._lower_user = False
         self._lower_obs = False
+        self._lower_stateful = False
+        # the instances already hold their state (updated in place; a lazily initialised attribute is None until
+        # the kernel's first evaluation has filled it): the Python __call__ continues from there
+        for slot in range(K["GFB_B_COUNT"] - K["GFB_B_USER_STATE0"]):
+            self._set(K["GFB_B_USER_STATE0"] + slot, None)
+        self.stateful = {}
+        self._lazy_started = {}
+        self._after_launch_lazy = set()
         self._observation_columns()
         self._set(K["GFB_B_OBS_EXT0"], self.ext_obs)
         self._set(K["GFB_B_OBS_EXT1"], None)
@@ -443,12 +458,16 @@ class FusedStep:
 
     def _lower_user_term(self, kind: str, name: str, item) -> bool:
         """Trace a user-defined term into the expression IR; False (and the reason kept) when it stays a callback."""
-        if not self._lower_user:
-            return False
         from . import expr
 
+        stateful = self._lower_stateful and expr.is_class_term(item.fn)
+        if not (self._lower_user or stateful):
+            return False
         try:
-            prog, live = expr.lower_term(self, kind, name, item)
+            if stateful:
+                prog, live = self._trace_stateful(kind, name, item), False
+            else:
+                prog, live = expr.lower_term(self, kind, name, item)
         except Exception as e:  # noqa: BLE001 - whatever the function does on symbolic inputs, it stays a callback
             why = str(e) if isinstance(e, UnsupportedTermError) else f"{type(e).__name__} while tracing: {e}"
             self.user_term_refusals[(kind, name)] = why
@@ -457,6 +476,74 @@ class FusedStep:
         self.user_terms[(kind, name)] = [prog, live, None if live else dict(item.params or {}),
                                          expr.param_kinds(item.params)]
         return True
+
+    def _trace_stateful(self, kind: str, name: str, item):
+        """
+        Trace a class-style term and bind its state: the instance's own per-env tensors, and for a lazily
+        initialised attribute a zeroed tensor that the instance gets once the kernel has evaluated the term
+        (`_after_report`).  The kernel updates them in place -- the one difference from the host path, where the
+        term rebinds its attributes: a reference kept to a state tensor sees the new values.
+        """
+        from . import expr
+
+        key = (kind, name)
+        old = self.stateful.get(key)
+        own = {a: b[0] for a, b in old["attrs"].items()} if old else {}
+        taken = {slot for k, b in self.stateful.items() if k != key for slot in b["tensors"]}
+        prog = expr.trace_term(self, kind, name, item, live_params=False,
+                               state=expr.StateSlots(own, [s for s in range(expr.MAX_STATE_SLOTS)
+                                                           if s not in taken and s not in own.values()]))
+        inst, tensors = item.fn, {}
+        for attr, (slot, shape, dtype, lazy) in prog.bindings.items():
+            tensors[slot] = (torch.zeros((self.N,) + tuple(shape), device=self.device, dtype=_TORCH_DTYPE[dtype])
+                             if lazy else vars(inst)[attr])
+        others = {t.untyped_storage().data_ptr(): k for k, b in self.stateful.items() if k != key
+                  for t in b["tensors"].values()}
+        for t in tensors.values():
+            if t.untyped_storage().data_ptr() in others:
+                raise UnsupportedTermError(f"{kind} '{name}': a state tensor shares storage with the state of "
+                                           f"{others[t.untyped_storage().data_ptr()][0]} "
+                                           f"'{others[t.untyped_storage().data_ptr()][1]}'")
+        K = nat.K
+        for slot in (old["tensors"] if old else {}):
+            self._set(K["GFB_B_USER_STATE0"] + slot, None)
+        for slot, t in tensors.items():
+            self._set(K["GFB_B_USER_STATE0"] + slot, t)
+        self.stateful[key] = {"inst": inst, "attrs": prog.bindings, "tensors": tensors,
+                              "constants": expr.instance_constants(inst)}
+        if prog.first is not None:
+            self._lazy_started[key] = False
+        else:
+            self._lazy_started.pop(key, None)
+        return prog
+
+    def _check_state(self) -> str | None:
+        """
+        Before a step's first post-physics launch: every state attribute of a lowered class-style term must still
+        be the tensor bound to its slot.  A compatible tensor the user assigned (a manual reset, a direct call of
+        the term) is bound instead; anything else -- another shape, dtype or device, a non-contiguous tensor,
+        None -- is returned as the reason to demote the lowered terms to callbacks.
+        """
+        K = nat.K
+        for key, b in self.stateful.items():
+            d = vars(b["inst"])
+            started = self._lazy_started.get(key, True)
+            for attr, (slot, shape, dtype, lazy) in b["attrs"].items():
+                cur, want = d.get(attr), b["tensors"][slot]
+                if cur is (want if started or not lazy else None):
+                    continue
+                if not (torch.is_tensor(cur) and tuple(cur.shape) == (self.N,) + tuple(shape)
+                        and cur.dtype == _TORCH_DTYPE[dtype] and cur.device == self.device and cur.is_contiguous()):
+                    return (f"{key[0]} '{key[1]}': self.{attr} is no longer a contiguous "
+                            f"{_TORCH_DTYPE[dtype]} tensor of shape {(self.N,) + tuple(shape)} on {self.device}")
+                b["tensors"][slot] = cur
+                self._set(K["GFB_B_USER_STATE0"] + slot, cur)
+                if lazy and not started:  # assigned by the user before the first evaluation: it is the state now
+                    self._lazy_started[key] = started = True
+                    for a, (s2, _, _, lz) in b["attrs"].items():
+                        if lz and a != attr and d.get(a) is None:
+                            d[a] = b["tensors"][s2]
+        return None
 
     @property
     def user_code(self) -> str:
@@ -480,6 +567,15 @@ class FusedStep:
         from . import expr
 
         entry = self.user_terms[(kind, name)]
+        bound = self.stateful.get((kind, name))
+        if bound is not None:
+            # a new instance (params edited: ConfigItem._rebuild) or an edited scalar attribute: traced again,
+            # with the new instance's tensors bound
+            if (item.fn is not bound["inst"] or dict(item.params or {}) != entry[2]
+                    or expr.instance_constants(item.fn) != bound["constants"]):
+                entry[0], entry[2] = self._trace_stateful(kind, name, item), dict(item.params or {})
+                self._user_code = None
+            return entry[0]
         # traced with constant params and they changed, or a live param changed between int and float (its
         # kernel type, int32 or fp32, was fixed by the trace)
         changed = entry[2] is not None and dict(item.params or {}) != entry[2]
@@ -650,7 +746,17 @@ class FusedStep:
             [(i.scale, i.noise) for i in obs_items],
             # lowered user observation terms fold their params in: a change traces them again (pack)
             [repr(sorted(dict(self.observations[g].cfg[n].params or {}).items())) for g, n in self.user_obs],
+            # lowered class-style terms: a new instance or an edited scalar attribute traces them again (pack)
+            self._stateful_fingerprint() if self.stateful else (),
         )
+
+    def _stateful_fingerprint(self) -> list:
+        from .expr import instance_constants
+
+        cfg = {"reward": self.reward.cfg if self.reward is not None else {},
+               "termination": self.termination.term_cfg if self.termination is not None else {}}
+        return [(id(cfg[k][n].fn), instance_constants(cfg[k][n].fn), self._lazy_started.get((k, n)))
+                for k, n in self.stateful]
 
     def _entity_of(self, params: dict):
         """The entity a term's (bound) parameters refer to, or None when the term takes no entity."""
@@ -710,6 +816,8 @@ class FusedStep:
         params = item.params or {}
         for k, pname in enumerate(prog.params):
             t.p[k] = params[pname]  # live: a curriculum may change them without a new kernel
+        if prog.first is not None:  # class-style terms have no live params: p[0] selects the steady program
+            t.p[0] = 1.0 if self._lazy_started.get((kind, name), False) else 0.0
 
     def _tilt_threshold(self, limit_angle: float) -> float:
         key = float(limit_angle)
@@ -1238,6 +1346,7 @@ class FusedStep:
             tuple(m._external_controller is None for m in self.commands),
             self._contact_dims,
             self._obs_user_id,
+            tuple(self.user_terms[k][0].digest() for k in self.stateful if k in self.user_terms),
         )
 
     def spec_stats(self) -> dict:
@@ -1250,6 +1359,9 @@ class FusedStep:
 
     def evaluate_external(self, kind: str):
         """Run the user-defined reward / termination functions; their values become kernel inputs."""
+        mgr = self.reward if kind == "reward" else self.termination
+        if mgr is not None and not mgr.enabled:  # a disabled manager calls no term (a class-style term's state stays)
+            return
         for j, (k, name, item) in enumerate(self.external_rows):
             if k != kind:
                 continue
@@ -1300,6 +1412,12 @@ class FusedStep:
         phases &= self._phase_mask
         first = self.first_launch_of_step
         self.first_launch_of_step = False
+        if first and self.stateful:
+            why = self._check_state()
+            if why is not None:
+                self._demote_user_terms(why)
+                raise UserTermsDemoted(why)
+            self._set_program()  # (a state tensor the user assigned may start a lazily initialised term)
         if first and self.lowered_user_terms and self.split_mode:
             # a later launch of the split step evaluates the lowered terms: check before anything is launched
             why = self._user_terms_blocked()
@@ -1313,6 +1431,10 @@ class FusedStep:
                 name for name in self._body_acc_terms
                 if not self._body_acc_started.get(name, False) and self.reward.cfg[name].weight != 0
             ] if self._body_acc_terms else []
+        for key, started in self._lazy_started.items():  # lowered class terms this launch evaluates
+            if not started and phases & (self._PHASE_REWARD if key[0] == "reward" else nat.K["GFB_PHASE_TERMINATION"]):
+                if key[0] == "termination" or self.reward.cfg[key[1]].weight != 0:
+                    self._after_launch_lazy.add(key)
         stream = self._stream()
         rc = self.lib.gfb_post_physics(self._h, self._buffers_ref, phases, stream)
         if rc:
@@ -1346,6 +1468,14 @@ class FusedStep:
         for name in self._after_launch_started:  # the term now has a previous velocity to difference
             self._body_acc_started[name] = True
         self._after_launch_started = []
+        for key in self._after_launch_lazy:  # the kernel has initialised the state: the instance holds it now
+            if key in self.stateful:
+                b = self.stateful[key]
+                self._lazy_started[key] = True
+                for attr, (slot, _, _, lazy) in b["attrs"].items():
+                    if lazy:
+                        setattr(b["inst"], attr, b["tensors"][slot])
+        self._after_launch_lazy = set()
 
     def observe(self, idx: torch.Tensor | None, n: int):
         self._engine_buffers(post_reset=True)

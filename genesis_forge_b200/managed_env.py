@@ -50,6 +50,11 @@ class ManagedEnvironment(GenesisEnv):
     # kernel instead of the host, and re-observed reset envs by a small kernel of the same library
     # (FusedStep.user_term_refusals[("observation", name)] says why a term stays a host column).
     fuse_user_observations = os.environ.get("GFB_FUSE_USER_OBS", "0") == "1"
+    # Class-style (MdpFnClass) user reward / termination terms, which keep per-env state from one step to the
+    # next (independent of the two switches above, same preconditions): with this set to True -- or
+    # GFB_FUSE_STATEFUL_TERMS=1 in the environment -- the ones that lower are evaluated by the specialised
+    # kernel, which updates the instance's state tensors in place (FusedStep.user_term_refusals says why not).
+    fuse_stateful_terms = os.environ.get("GFB_FUSE_STATEFUL_TERMS", "0") == "1"
 
     def __init__(
         self,

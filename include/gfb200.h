@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define GFB_ABI_VERSION 13
+#define GFB_ABI_VERSION 14
 
 /* ---- limits ------------------------------------------------------------------------------- */
 #define GFB_MAX_DOFS 32
@@ -115,6 +115,10 @@ typedef enum {
   /* values of user-defined (host-evaluated) reward / termination terms: (J, N) fp32, one row per term */
   GFB_B_EXT_VALUES,
   GFB_B_DONES,        /* (N,) bool written: terminated | truncated (what wrappers/rsl_rl.py:57 computes) */
+  /* per-env state of class-style user terms lowered into the specialised kernel: (N, *s) fp32 / int32 / bool,
+     read and updated in place (ABI v14) */
+  GFB_B_USER_STATE0, GFB_B_USER_STATE1, GFB_B_USER_STATE2, GFB_B_USER_STATE3,
+  GFB_B_USER_STATE4, GFB_B_USER_STATE5, GFB_B_USER_STATE6, GFB_B_USER_STATE7,
   GFB_B_COUNT
 } gfb_buf;
 
