@@ -1317,6 +1317,11 @@ int gfb_observe(gfb_handle* h, const gfb_buffers* b, const int64_t* idx, int32_t
       return fail(h, GFB_ERR_UNSUPPORTED,
                   "gfb_observe: the program has GFB_O_USER columns and no specialised kernel generated for them is "
                   "attached (the generic kernel does not evaluate them)");
+    for (int i = 0; i < 8; ++i)  // its class-style observation terms read and write these rows in place
+      if (((user_spec->state_slots >> i) & 1u) && !b->buf[GFB_B_USER_STATE0 + i])
+        return fail(h, GFB_ERR_INVALID,
+                    "buffer USER_STATE" + std::to_string(i) + " is NULL (the attached specialised kernel keeps the "
+                    "state of a lowered class-style term there)");
   }
   rc = upload_table(h, h->observe_slot, table, stream);
   if (rc != GFB_OK) return rc;

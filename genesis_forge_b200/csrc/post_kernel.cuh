@@ -1002,10 +1002,17 @@ __global__ void __launch_bounds__(TILE, GFB_MIN_BLOCKS(TILE)) post_kernel(const 
 
 #if defined(GFB_SPEC) && defined(GFB_SPEC_USER_OBS)
   // lowered user-defined observation terms: from what a stock column of this launch sees (the post-resample
-  // command, the body-frame registers, the staged rows) into the stash words the GFB_O_USER columns read
+  // command, the body-frame registers, the staged rows) into the stash words the GFB_O_USER columns read.
+  // Class-style terms among them (GFB_SPEC_USER_OBS_STATE) store their state once per evaluation: a reset env
+  // of this launch is evaluated again by the reset path (gfb_observe), which stores it, so it does not store here.
   if (ph & GFB_PHASE_OBSERVE)
     user_observations(UserCtx{K.b, (size_t)e, ep_len, max_len, terminated, truncated, iw, iq, lin_b, ang_b, grav_b, S,
-                              tid, st, plan, nullptr, N, active},
+                              tid, st, plan, nullptr, N,
+#ifdef GFB_SPEC_USER_OBS_STATE
+                              active && !reset},
+#else
+                              active},
+#endif
                       st + user_stash_base(SP));
 #endif
 

@@ -27,14 +27,17 @@ unsqueeze, None in an index and reshape / view / flatten of a row.  Their params
 again when they change).  Their device code comes twice: for the owner phase of post_kernel and, reading
 global memory only, for the reset path that re-observes reset envs (spec_kernel.cu).
 
-Class-style reward / termination terms (an MdpFnClass instance, ManagedEnvironment.fuse_stateful_terms) are
-traced through `type(inst).__call__`.  A per-env tensor attribute of the instance -- (N, *s) with at most
-MAX_CONST_VEC elements a row, fp32 / int32 / bool, on the env's device and contiguous -- is a source
+Class-style reward / termination / observation terms (an MdpFnClass instance,
+ManagedEnvironment.fuse_stateful_terms) are traced through `type(inst).__call__` (`trace_stateful`).  A per-env
+tensor attribute of the instance -- (N, *s) with at most MAX_CONST_VEC elements a row, fp32 / int32 / bool,
+on the env's device and contiguous -- is a source
 ("state", slot); rebinding it to a value of the same row shape and dtype, `self.x[:] = v` and `self.x.copy_(v)`
 are state writes (`Program.writes`), stored to the env's row after the result is computed.  An attribute
 that is None and gets a per-env value during the call (lazy initialisation) gives a second, first-call
-program (`Program.first`), which the kernel selects while the term's p[0] is 0.  Python-scalar attributes
-and params are trace constants.
+program (`Program.first`), which the kernel selects while the term's p[0] is 0 (rewards and terminations
+only: an observation term's state exists once the build's dry run has called it).  Python-scalar attributes
+and params are trace constants.  An observation term stores its state only when `UserCtx::active` says so:
+the owner phase passes `active && !reset`, because the reset path evaluates a reset env once more.
 
 Anything outside this subset raises UnsupportedTermError naming the op or source; the term then
 stays a host callback (split execution), with exactly the results it had before.
@@ -920,6 +923,23 @@ def trace_term(fused, kind: str, name: str, item, live_params: bool = True, stat
     if not isinstance(result, Sym):
         raise UnsupportedTermError(f"{what}: the result does not depend on per-env state the kernel holds "
                                    f"({type(result).__name__})")
+    return _term_program(tr, kind, what, result)
+
+
+def trace_stateful(fused, kind: str, name: str, item, state: StateSlots) -> Program:
+    """Trace one class-style reward / termination / observation term, binding its per-env tensors to the
+    `state` slots (raises UnsupportedTermError)."""
+    if isinstance(item.fn, type):
+        raise UnsupportedTermError(f"{kind} '{name}': a class, not an instance of it")
+    return _trace_stateful(fused, kind, f"{kind} '{name}'", item, state)
+
+
+def _term_program(tr: Tracer, kind: str, what: str, result, writes: dict | None = None) -> Program:
+    """The Program of a term's result (and of its state writes {slot: node})."""
+    if not isinstance(result, Sym):
+        raise UnsupportedTermError(f"{what}: the result does not depend on per-env state the kernel holds "
+                                   f"({type(result).__name__})")
+    slots = sorted(writes or {})
     if kind == "observation":
         # flattened row-major into its columns and cast to fp32, as FusedStep.evaluate_external_obs copies it
         if result.weak:
@@ -928,16 +948,8 @@ def trace_term(fused, kind: str, name: str, item, live_params: bool = True, stat
         if width > MAX_CONST_VEC:
             raise UnsupportedTermError(f"{what}: {width} columns (at most {MAX_CONST_VEC} are lowered)")
         out = tr.cast(tr._as_row((width,), result), F32)._id
-        nodes = _live_nodes(tr.nodes, out)
-        return Program(kind, nodes[0], nodes[1], [], [])
-    return _term_program(tr, kind, what, result)
-
-
-def _term_program(tr: Tracer, kind: str, what: str, result, writes: dict | None = None) -> Program:
-    """The Program of a reward / termination's result (and of its state writes {slot: node})."""
-    if not isinstance(result, Sym):
-        raise UnsupportedTermError(f"{what}: the result does not depend on per-env state the kernel holds "
-                                   f"({type(result).__name__})")
+        nodes, out, extra = _live_nodes(tr.nodes, out, [writes[s] for s in slots])
+        return Program(kind, nodes, out, [], [], list(zip(slots, extra)))
     if result.weak or result.shape_ != ():
         raise UnsupportedTermError(f"{what}: the result has shape {tuple(result.shape)}, not (N,)")
     if kind == "termination" and result.dtype_ != BOOL:
@@ -945,7 +957,6 @@ def _term_program(tr: Tracer, kind: str, what: str, result, writes: dict | None 
     out = result._id
     if kind == "reward" and result.dtype_ != F32:
         out = tr.cast(result, F32)._id
-    slots = sorted(writes or {})
     nodes, out, extra = _live_nodes(tr.nodes, out, [writes[s] for s in slots])
     return Program(kind, nodes, out, tr.params, tr.param_types, list(zip(slots, extra)))
 
@@ -970,9 +981,11 @@ def _holds_env_rows(obj, N: int) -> bool:
 
 def _trace_stateful(fused, kind: str, what: str, item, state: StateSlots) -> Program:
     """
-    Trace a class-style term: `type(inst).__call__(inst, env, **params)` with the instance's per-env tensors as
-    ("state", slot) sources.  Attributes that are None and get a per-env value during the call are initialised
-    lazily: the call is traced once with them None (the first-call program) and once more with them as state.
+    Trace a class-style term: `type(inst).__call__(inst, env, **params)` (an observation term: `env=env`) with
+    the instance's per-env tensors as ("state", slot) sources.  Attributes that are None and get a per-env value
+    during the call are initialised lazily: the call is traced once with them None (the first-call program) and
+    once more with them as state.  Observation terms have no first-call program: the build's dry run has
+    already called them, so such an attribute still None is refused.
     """
     env, inst, N = fused.env, item.fn, fused.N
     params = dict(item.params or {})
@@ -1015,7 +1028,10 @@ def _trace_stateful(fused, kind: str, what: str, item, state: StateSlots) -> Pro
             _install_sources(fused, tr, swap, kind)
             env._tracing = ExprMode(tr, fused)
             inst.__dict__.update(syms)
-            result = type(inst).__call__(inst, env, **params)
+            if kind == "observation":
+                result = type(inst).__call__(inst, env=env, **params)
+            else:
+                result = type(inst).__call__(inst, env, **params)
             after = dict(vars(inst))
         finally:
             env._tracing = None
@@ -1033,6 +1049,11 @@ def _trace_stateful(fused, kind: str, what: str, item, state: StateSlots) -> Pro
                                                "row shape and dtype must stay)")
                 if new._id != src[attr]:
                     writes[state.slot(attr)] = new._id
+            elif old is None and isinstance(new, Sym) and kind == "observation":
+                # (the build's dry run has called the term: lazily initialised state exists by now, or the
+                #  term did not initialise it there)
+                raise UnsupportedTermError(f"{what}: self.{attr} is None when the term is traced (an observation "
+                                           "term is lowered with its state initialised)")
             elif old is None and isinstance(new, Sym) and not lazy_rows:  # lazy initialisation (first call)
                 if new.weak or int(np.prod(new.shape_)) > MAX_CONST_VEC:
                     raise UnsupportedTermError(f"{what}: self.{attr} is initialised to a value that is not per-env "
@@ -1388,19 +1409,21 @@ def function_body(prog: Program, fname: str, glob: bool = False) -> str:
             names.append(nm)
         elems.append(names)
     body = "\n".join("  " + ln for ln in lines)
-    if prog.kind == "observation":
-        stores = "\n".join(f"  out[{k}] = {x};" for k, x in enumerate(elems[prog.out]))
-        return f"__device__ __forceinline__ void {fname}(const UserCtx& c, float* out) {{\n{body}\n{stores}\n}}\n"
-    ret = elems[prog.out][0]
-    rtype = "bool" if prog.kind == "termination" else "float"
     stores = []
-    for slot, i in prog.writes:  # after the result; lanes that shadow env N-1 in a tail slab do not store
+    # after the result; lanes that shadow env N-1 in a tail slab do not store, nor (observation terms) a reset
+    # env in the owner phase: the reset path evaluates it again
+    for slot, i in prog.writes:
         ct = _CT[prog.nodes[i].dtype]
         row = elems[i]
         stores.append(f"    {ct}* s{slot} = reinterpret_cast<{ct}*>(c.b.buf[GFB_B_USER_STATE0 + {slot}]) + c.e * "
                       f"{len(row)};")
         stores += [f"    s{slot}[{k}] = {x};" for k, x in enumerate(row)]
     store = ("\n  if (c.active) {\n" + "\n".join(stores) + "\n  }") if stores else ""
+    if prog.kind == "observation":
+        out = "\n".join(f"  out[{k}] = {x};" for k, x in enumerate(elems[prog.out]))
+        return f"__device__ __forceinline__ void {fname}(const UserCtx& c, float* out) {{\n{body}\n{out}{store}\n}}\n"
+    ret = elems[prog.out][0]
+    rtype = "bool" if prog.kind == "termination" else "float"
     return (f"__device__ __forceinline__ {rtype} {fname}(const UserCtx& c) {{\n{body}{store}\n  return {ret};\n}}\n")
 
 
@@ -1464,6 +1487,9 @@ def device_code(rewards: dict[int, Program], terminations: dict[int, Program],
             parts.append(function_body(prog, f"gfb_user_og{j}", glob=True))
             calls += f"  gfb_user_o{j}(c, out + {col0});\n"
             calls_g += f"  gfb_user_og{j}(c, out + {col0});\n"
+        if any(prog.writes for _, prog in observations):
+            # (spec.py defines GFB_SPEC_USER_OBS_STATE for it: the owner phase passes active && !reset)
+            parts.append("/* observation terms store state */\n")
         parts.append(f"constexpr int kUserObsWords = {obs_words};\n")
         parts.append(f"__device__ __forceinline__ void user_observations(const UserCtx& c, float* out) {{\n{calls}}}\n")
         parts.append("__device__ __forceinline__ void user_observations_global(const UserCtx& c, float* out) {\n"

@@ -45,6 +45,13 @@ _log = logging.getLogger(__name__)
 _TORCH_DTYPE = {"f32": torch.float32, "i32": torch.int32, "bool": torch.bool}  # (expr.F32, I32, BOOL)
 
 
+def _check_width(prog, name: str, width: int):
+    """An observation term's traced columns must be the width its dry run returned."""
+    if prog.nodes[prog.out].shape != (width,):
+        raise UnsupportedTermError(f"observation '{name}': traced {prog.nodes[prog.out].shape[0]} columns, "
+                                   f"the function returned {width}")
+
+
 def _f32(x) -> float:
     """Python float -> the fp32 value torch uses when a Python scalar meets a float32 tensor."""
     return float(_F32(x))
@@ -260,7 +267,10 @@ class FusedStep:
         # class-style terms (ManagedEnvironment.fuse_stateful_terms): their per-env tensors are bound to the
         # GFB_B_USER_STATE slots and updated in place by the kernel
         self._lower_stateful = bool(getattr(env, "fuse_stateful_terms", False)) and self._can_specialise_user_terms()
-        self.stateful: dict = {}  # (kind, name) -> {"inst", "attrs": {attr: (slot, shape, dtype, lazy)}, "tensors"}
+        # (kind, name), for an observation term ("observation", name, group) -> {"inst", "attrs": {attr: (slot,
+        # shape, dtype, lazy)}, "tensors", "constants"}
+        self.stateful: dict = {}
+        self._state_refusal = None  # why a class-style observation term could not be traced again (demotes)
         if self.reward is not None:
             for name, item in self.reward.cfg.items():
                 opcode = self._opcode_of(item.fn, "reward")
@@ -323,15 +333,17 @@ class FusedStep:
 
     def _lower_user_obs(self, g: int, name: str, item, width: int) -> bool:
         """Trace a user-defined observation term into the expression IR; False (reason kept) when it stays a host column."""
-        if not self._lower_obs:
-            return False
         from . import expr
 
+        stateful = self._lower_stateful and expr.is_class_term(item.fn)
+        if not (self._lower_obs or stateful):
+            return False
         try:
-            prog, _ = expr.lower_term(self, "observation", name, item)
-            if prog.nodes[prog.out].shape != (width,):
-                raise UnsupportedTermError(f"observation '{name}': traced {prog.nodes[prog.out].shape[0]} columns, "
-                                           f"the function returned {width}")
+            if stateful:
+                prog = self._trace_stateful("observation", name, item, (g, width))
+            else:
+                prog, _ = expr.lower_term(self, "observation", name, item)
+                _check_width(prog, name, width)
         except Exception as e:  # noqa: BLE001 - whatever the function does on symbolic inputs, it stays a host column
             why = str(e) if isinstance(e, UnsupportedTermError) else f"{type(e).__name__} while tracing: {e}"
             self.user_term_refusals[("observation", name)] = why
@@ -345,6 +357,22 @@ class FusedStep:
         from . import expr
 
         entry = self.user_obs[(g, name)]
+        bound = self.stateful.get(("observation", name, g))
+        if bound is not None:
+            # a new instance (params edited) or an edited scalar attribute: traced again.  If that fails, the
+            # table keeps the old program until _check_state demotes the lowered terms (before any launch that
+            # evaluates this one)
+            if self._state_refusal is None and (item.fn is not bound["inst"] or dict(item.params or {}) != entry[1]
+                                                or expr.instance_constants(item.fn) != bound["constants"]):
+                try:
+                    entry[0] = self._trace_stateful("observation", name, item, (g, entry[3]))
+                except Exception as e:  # noqa: BLE001 - as at build: the term becomes a host column
+                    self._state_refusal = str(e) if isinstance(e, UnsupportedTermError) else \
+                        f"{type(e).__name__} while tracing: {e}"
+                    return entry[0]
+                entry[1] = dict(item.params or {})
+                self._user_code = None
+            return entry[0]
         if dict(item.params or {}) != entry[1]:
             prog, _ = expr.lower_term(self, "observation", name, item)
             if prog.nodes[prog.out].shape != (entry[3],):
@@ -437,6 +465,7 @@ class FusedStep:
         for slot in range(K["GFB_B_COUNT"] - K["GFB_B_USER_STATE0"]):
             self._set(K["GFB_B_USER_STATE0"] + slot, None)
         self.stateful = {}
+        self._state_refusal = None
         self._lazy_started = {}
         self._after_launch_lazy = set()
         self._observation_columns()
@@ -477,22 +506,25 @@ class FusedStep:
                                          expr.param_kinds(item.params)]
         return True
 
-    def _trace_stateful(self, kind: str, name: str, item):
+    def _trace_stateful(self, kind: str, name: str, item, obs: tuple | None = None):
         """
         Trace a class-style term and bind its state: the instance's own per-env tensors, and for a lazily
         initialised attribute a zeroed tensor that the instance gets once the kernel has evaluated the term
         (`_after_report`).  The kernel updates them in place -- the one difference from the host path, where the
-        term rebinds its attributes: a reference kept to a state tensor sees the new values.
+        term rebinds its attributes: a reference kept to a state tensor sees the new values.  `obs`: (group,
+        width) of an observation term (keyed by group too: the same class in two groups is two instances).
         """
         from . import expr
 
-        key = (kind, name)
+        key = (kind, name) if obs is None else (kind, name, obs[0])
         old = self.stateful.get(key)
         own = {a: b[0] for a, b in old["attrs"].items()} if old else {}
         taken = {slot for k, b in self.stateful.items() if k != key for slot in b["tensors"]}
-        prog = expr.trace_term(self, kind, name, item, live_params=False,
-                               state=expr.StateSlots(own, [s for s in range(expr.MAX_STATE_SLOTS)
-                                                           if s not in taken and s not in own.values()]))
+        prog = expr.trace_stateful(self, kind, name, item,
+                                   expr.StateSlots(own, [s for s in range(expr.MAX_STATE_SLOTS)
+                                                         if s not in taken and s not in own.values()]))
+        if obs is not None:
+            _check_width(prog, name, obs[1])
         inst, tensors = item.fn, {}
         for attr, (slot, shape, dtype, lazy) in prog.bindings.items():
             tensors[slot] = (torch.zeros((self.N,) + tuple(shape), device=self.device, dtype=_TORCH_DTYPE[dtype])
@@ -519,11 +551,18 @@ class FusedStep:
 
     def _check_state(self) -> str | None:
         """
-        Before a step's first post-physics launch: every state attribute of a lowered class-style term must still
-        be the tensor bound to its slot.  A compatible tensor the user assigned (a manual reset, a direct call of
-        the term) is bound instead; anything else -- another shape, dtype or device, a non-contiguous tensor,
-        None -- is returned as the reason to demote the lowered terms to callbacks.
+        Before a step's first post-physics launch and before the host columns of an observation are evaluated
+        (evaluate_external_obs, which precedes every other launch that evaluates a lowered class-style
+        observation term): every state attribute of a lowered class-style term must still be the tensor bound to
+        its slot.  A compatible tensor the user assigned (a manual reset, a direct call of the term) is bound
+        instead; anything else -- another shape, dtype or device, a non-contiguous tensor, None -- is returned
+        as the reason to demote the lowered terms to callbacks, as is a class-style observation term that
+        could not be traced again after an edit.
         """
+        for key in [k for k in self.stateful if len(k) == 3]:  # (a new instance or constants: traced again)
+            self._user_obs_program(key[2], key[1], self.observations[key[2]].cfg[key[1]])
+        if self._state_refusal is not None:
+            return self._state_refusal
         K = nat.K
         for key, b in self.stateful.items():
             d = vars(b["inst"])
@@ -755,8 +794,11 @@ class FusedStep:
 
         cfg = {"reward": self.reward.cfg if self.reward is not None else {},
                "termination": self.termination.term_cfg if self.termination is not None else {}}
-        return [(id(cfg[k][n].fn), instance_constants(cfg[k][n].fn), self._lazy_started.get((k, n)))
-                for k, n in self.stateful]
+        out = []
+        for key in self.stateful:
+            fn = (self.observations[key[2]].cfg if len(key) == 3 else cfg[key[0]])[key[1]].fn
+            out.append((id(fn), instance_constants(fn), self._lazy_started.get(key)))
+        return out
 
     def _entity_of(self, params: dict):
         """The entity a term's (bound) parameters refer to, or None when the term takes no entity."""
@@ -1371,6 +1413,12 @@ class FusedStep:
             self.ext_values[j].copy_(value.reshape(self.N))
 
     def evaluate_external_obs(self):
+        if any(len(k) == 3 for k in self.stateful):
+            # the lowered class-style observation terms are evaluated next (get_observations, the observation
+            # launch of a split step): their state is checked first; demoted, they are host columns from here on
+            why = self._check_state()
+            if why is not None:
+                self._demote_user_terms(why)
         for om, name, item, col0, width in self.external_obs:
             value = item.fn(env=self.env, **item.params)
             self.ext_obs[:, col0:col0 + width].copy_(value.reshape(self.N, width))

@@ -26,6 +26,7 @@ import torch
 
 from . import _native as nat
 from ._gs import gs
+from .expr import is_class_term
 from .fused import FusedStep, UnsupportedTermError, UserTermsDemoted, combine_logging, make_obs_dict
 from .genesis_env import GenesisEnv
 from .managers.base import BaseManager, ManagerType
@@ -50,8 +51,8 @@ class ManagedEnvironment(GenesisEnv):
     # kernel instead of the host, and re-observed reset envs by a small kernel of the same library
     # (FusedStep.user_term_refusals[("observation", name)] says why a term stays a host column).
     fuse_user_observations = os.environ.get("GFB_FUSE_USER_OBS", "0") == "1"
-    # Class-style (MdpFnClass) user reward / termination terms, which keep per-env state from one step to the
-    # next (independent of the two switches above, same preconditions): with this set to True -- or
+    # Class-style (MdpFnClass) user reward / termination / observation terms, which keep per-env state from one
+    # step to the next (independent of the two switches above, same preconditions): with this set to True -- or
     # GFB_FUSE_STATEFUL_TERMS=1 in the environment -- the ones that lower are evaluated by the specialised
     # kernel, which updates the instance's state tensors in place (FusedStep.user_term_refusals says why not).
     fuse_stateful_terms = os.environ.get("GFB_FUSE_STATEFUL_TERMS", "0") == "1"
@@ -157,8 +158,17 @@ class ManagedEnvironment(GenesisEnv):
     def _trace_term(self, fn, params: dict, what: str):
         """Run an observation term once under tracing and identify which manager value it returns."""
         self._tracing = {}
+        # a class-style term keeps state: this call on placeholders must not advance (or break) it -- the
+        # reference calls the term once at build, the dry run of ObservationManager.resolve_external
+        saved = dict(vars(fn)) if is_class_term(fn) and hasattr(fn, "__dict__") else None
+        data = {k: v.clone() for k, v in saved.items() if torch.is_tensor(v)} if saved is not None else {}
         try:
-            result = fn(env=self, **params)
+            try:
+                result = fn(env=self, **params)
+            except Exception as e:
+                if saved is None or isinstance(e, UnsupportedTermError):
+                    raise
+                raise UnsupportedTermError(f"{what}: a class-style term that does not run on placeholders") from e
             for key, sentinel in self._tracing.items():
                 if result is sentinel:
                     if isinstance(key, str) and key.endswith("_uncached"):
@@ -175,6 +185,11 @@ class ManagedEnvironment(GenesisEnv):
                     return key, sentinel.shape[1]
         finally:
             self._tracing = None
+            if saved is not None:
+                vars(fn).clear()
+                vars(fn).update(saved)
+                for k, t in data.items():
+                    saved[k].copy_(t)
         raise UnsupportedTermError(
             f"{what}: the term function does not return a manager value the fused step recognises "
             "(EntityManager.get_*, action manager getters, CommandManager.observation, "

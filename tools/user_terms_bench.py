@@ -5,14 +5,15 @@ kernel (fuse_user_terms on), at 65,536 and 1,048,576 envs.  `--workload user_obs
 for workload A of configs/user_observations.py (fuse_user_observations), adds the stock `contacts` table
 as a third, reference environment for the post-physics kernel's time, and reports the reset-path kernel
 of the lowered observation terms.  `--workload stateful_terms` compares workload A of configs/stateful_terms.py
-(class-style terms with per-env state) as callbacks and lowered (fuse_stateful_terms).  The two modes are built
-side by side and
+(class-style terms with per-env state) as callbacks and lowered (fuse_stateful_terms), and
+`--workload stateful_observations` workload A of configs/stateful_observations.py (class-style observation
+terms: host columns against lowered, fuse_stateful_terms).  The two modes are built side by side and
 timed alternately in one process (CUDA events around `steps` steps, in-kernel Philox draws as bench.py
 runs them, on bench.py's pool of pre-generated state sets); the post-physics kernel's device time comes
 from the library's own event brackets.  The outputs of one more step of both modes (same states, same
 actions, same draws) are compared.
 
-    python tools/user_terms_bench.py [--workload user_terms|user_observations|stateful_terms]
+    python tools/user_terms_bench.py [--workload user_terms|user_observations|stateful_terms|stateful_observations]
                                      [--sizes 65536 1048576]
                                      [--steps 50] [--warmup 10] [--rounds 3]
 """
@@ -44,17 +45,19 @@ def gpu_info() -> dict:
 
 def make_env(n: int, mode: str, dev, workload: str = "user_terms"):
     import genesis_forge_b200 as gfb
-    from configs import specs, stateful_terms, user_observations, user_terms
+    from configs import specs, stateful_observations, stateful_terms, user_observations, user_terms
     from configs.env_builder import build_env, dropin_namespace
     from genesis_forge_b200.managed_env import ManagedEnvironment
 
-    obs, stateful = workload == "user_observations", workload == "stateful_terms"
+    obs = workload == "user_observations"
+    stateful = workload in ("stateful_terms", "stateful_observations")
     ManagedEnvironment.fuse_user_terms = mode == "fused" and not obs and not stateful
     ManagedEnvironment.fuse_user_observations = mode == "fused" and obs
     ManagedEnvironment.fuse_stateful_terms = mode == "fused" and stateful
     gfb.set_device(dev)
     spec = specs.contacts() if mode == "stock" else (user_observations.user_observations() if obs
-                                                     else stateful_terms.stateful_terms() if stateful
+                                                     else stateful_terms.stateful_terms() if workload == "stateful_terms"
+                                                     else stateful_observations.stateful_observations() if stateful
                                                      else user_terms.user_terms())
     # as bench.py: a pool of pre-generated state sets rotated by scene.step() (the same states for both modes),
     # engine-side reset writes accepted but not applied
@@ -94,7 +97,8 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--rounds", type=int, default=3)
-    ap.add_argument("--workload", choices=["user_terms", "user_observations", "stateful_terms"], default="user_terms")
+    ap.add_argument("--workload", choices=["user_terms", "user_observations", "stateful_terms",
+                                                       "stateful_observations"], default="user_terms")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     print(json.dumps({"gpu": gpu_info()}), flush=True)
@@ -130,7 +134,7 @@ def main():
             result[mode] = {"ms_per_step_median": round(ms, 4), "env_steps_per_s": round(n / ms * 1e3),
                             "post_kernel_ms_per_step_median": round(post, 4), "post_launches_per_step": r[0][2],
                             "ms_per_step_all": [round(x[0], 4) for x in r]}
-            if args.workload == "user_observations" and mode == "fused":
+            if args.workload in ("user_observations", "stateful_observations") and mode == "fused":
                 result[mode]["user_observe_kernel_us_median"] = round(sorted(x[3] for x in r)[len(r) // 2], 2)
                 result[mode]["spec_stats"] = envs[mode]._fused.spec_stats()
         print(json.dumps(result), flush=True)
