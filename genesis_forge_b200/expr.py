@@ -9,8 +9,10 @@ A user term is a plain Python function of the environment, e.g.
 `trace_term` runs it ONCE with symbolic stand-ins for the per-env state it may read (the primary
 entity's getters, the first EntityManager's cache and body-frame vectors, the action manager's
 getters, env.actions / last_actions / episode_length / max_episode_length, the `command` of
-kernel-resampled command managers, contact forces and air-time state, and -- rewards only --
-extras["terminations"] / ["time_outs"]).  Every operation on them is recorded as a node of a small
+kernel-resampled command managers, contact forces and air-time state, the primary entity's link positions /
+velocities (`get_links_pos` / `get_links_vel` with `links_idx_local`, and its link objects' `get_pos` /
+`get_vel`; FusedStep._layout_links binds them as per-launch gathers in free GFB_B_USER_STATE slots) and -- rewards
+only -- extras["terminations"] / ["time_outs"]).  Every operation on them is recorded as a node of a small
 expression IR (`Program`) with torch's shapes and type promotion.  Scalar entries of the term's
 params become LIVE slots (the term's p[4] in the packed table), so a curriculum that edits them keeps
 the same kernel binary; everything else the function captures is a compile-time constant.
@@ -57,6 +59,7 @@ _RANK = {BOOL: 0, I32: 1, F32: 2}
 MAX_CONST_VEC = 32  # GFB_MAX_DOFS: small constant vectors (per-joint limits, gains) are folded in
 MAX_LIVE_PARAMS = 4  # gfb_reward_term.p / gfb_termination_term.p
 MAX_STATE_SLOTS = 8  # GFB_B_USER_STATE0..7
+MAX_LINKS = 10  # links of one per-link array: a (N, |U|, 3) row stays within GFB_MAX_DOFS floats
 # bumped whenever `function_body` emits different code for the same IR: the digest changes with it
 CODEGEN_REVISION = 2
 
@@ -73,11 +76,12 @@ def _f32(x) -> float:
 # IR
 # ------------------------------------------------------------------------------------------------
 class Node:
-    __slots__ = ("op", "args", "attr", "shape", "dtype", "weak")
+    __slots__ = ("op", "args", "attr", "shape", "dtype", "weak", "envless")
 
-    def __init__(self, op, args, attr, shape, dtype, weak=False):
+    def __init__(self, op, args, attr, shape, dtype, weak=False, envless=False):
         self.op, self.args, self.attr = op, tuple(args), attr
         self.shape, self.dtype, self.weak = tuple(shape), dtype, weak
+        self.envless = envless  # a value without the env dim (a constant vector): broadcasting aligns it right
 
     def text(self, i: int) -> str:
         return f"%{i} = {self.op}({', '.join('%' + str(a) for a in self.args)}; {self.attr!r}) : {self.dtype}{list(self.shape)}{' weak' if self.weak else ''}"
@@ -129,8 +133,37 @@ def _bshape(a: "Sym", b: "Sym", what: str) -> tuple:
         return a.shape_
     if not a.shape_:
         return b.shape_
-    raise UnsupportedTermError(f"user term: '{what}' of shapes (N, *{a.shape_}) and (N, *{b.shape_}) does not broadcast "
-                               "row by row")
+    return _broadcast([a, b], what)
+
+
+def _broadcast(xs: list, what: str) -> tuple:
+    """torch's broadcasting of the per-env shapes: per-env values of one rank, trailing dims aligned, size-1 dims
+    expanded; a value without the env dim (a constant vector) aligns with the trailing per-env dims."""
+    shapes = [x.shape_ for x in xs if x.shape_]
+    ranks = {len(x.shape_) for x in xs if x.shape_ and not x._node.envless}
+    rank = max(len(s) for s in shapes)
+    out = []
+    for d in range(1, rank + 1):
+        sizes = {s[-d] for s in shapes if len(s) >= d} - {1}
+        if len(sizes) > 1:
+            break
+        out.append(sizes.pop() if sizes else 1)
+    if len(out) == rank and len(ranks) <= 1 and (not ranks or ranks == {rank}):
+        return tuple(reversed(out))
+    raise UnsupportedTermError(f"user term: '{what}' of shapes {' and '.join(f'(N, *{s})' for s in shapes)} does "
+                               "not broadcast row by row")
+
+
+def _bidx(out_shape: tuple, shape: tuple) -> list[int]:
+    """Per element of `out_shape` (row-major), the flat index into a value of `shape` broadcast to it."""
+    if shape == out_shape:
+        return list(range(int(np.prod(out_shape)) if out_shape else 1))
+    if not shape:
+        return [0] * (int(np.prod(out_shape)) if out_shape else 1)
+    st = _strides(shape)
+    lead = len(out_shape) - len(shape)
+    return [sum(combo[lead + d] * st[d] for d in range(len(shape)) if shape[d] != 1)
+            for combo in np.ndindex(*out_shape)]
 
 
 class Sym:
@@ -353,6 +386,33 @@ _REDUCE_TORCH = {"sum": "sum", "mean": "mean", "any": "any", "all": "all", "amax
 _LAYOUT_SEQ = ("stack", "cat", "concat", "concatenate")  # over a sequence of values (observation terms only)
 
 
+def _const_index(k):
+    """An index list or integer tensor as a list of ints (a 0-d integer tensor: an int), anything else as is."""
+    if isinstance(k, np.ndarray):
+        k = torch.from_numpy(k)
+    if torch.is_tensor(k):
+        if k.dtype is torch.bool:
+            raise UnsupportedTermError("user term: a bool mask index (data-dependent shape)")
+        if k.is_floating_point() or k.is_complex() or k.dim() > 1:
+            raise UnsupportedTermError(f"user term: a {k.dtype} index tensor of shape {tuple(k.shape)} (0-d or 1-D "
+                                       "integer tensors only)")
+        k = k.detach().cpu()
+        if k.dim() == 0:
+            return int(k.item())
+        k = k.tolist()
+    if isinstance(k, (list, tuple)):
+        if any(isinstance(i, Sym) for i in k):
+            next(i for i in k if isinstance(i, Sym))._control("index")
+        if any(isinstance(i, (bool, np.bool_)) for i in k):
+            raise UnsupportedTermError("user term: a bool mask index (data-dependent shape)")
+        if not all(isinstance(i, (int, np.integer)) for i in k):
+            raise UnsupportedTermError(f"user term: index list {k!r} (ints only)")
+        if len(k) > MAX_CONST_VEC:
+            raise UnsupportedTermError(f"user term: an index list of {len(k)} ids (at most {MAX_CONST_VEC})")
+        return [int(i) for i in k]
+    return k
+
+
 # ------------------------------------------------------------------------------------------------
 # tracer
 # ------------------------------------------------------------------------------------------------
@@ -366,12 +426,15 @@ class Tracer:
         self.state_objs: dict = {}  # id(Sym) -> (slot, Sym): the instance's state tensors
         self.viewed: set = set()  # state slots a view was taken of
 
-    def add(self, op, args, attr, shape, dtype, weak=False) -> Sym:
+    def add(self, op, args, attr, shape, dtype, weak=False, envless=None) -> Sym:
         key = (op, tuple(args), repr(attr), tuple(shape), dtype, weak)
         nid = self._cse.get(key)
         if nid is None:
+            if envless is None:  # (derived from constant vectors alone)
+                strong = [self.nodes[i] for i in args if not self.nodes[i].weak]
+                envless = bool(strong) and all(n.envless for n in strong)
             nid = len(self.nodes)
-            self.nodes.append(Node(op, args, attr, shape, dtype, weak))
+            self.nodes.append(Node(op, args, attr, shape, dtype, weak, envless))
             self._cse[key] = nid
         return Sym(self, nid)
 
@@ -432,7 +495,7 @@ class Tracer:
             if t.dim() == 1 and t.shape[0] <= MAX_CONST_VEC and t.shape[0] != self.N:
                 dtype = _dtype_of(t.dtype)
                 vals = tuple(bool(v) if dtype == BOOL else (int(v) if dtype == I32 else _f32(v)) for v in t.tolist())
-                return self.add("constvec", (), vals, (t.shape[0],), dtype)
+                return self.add("constvec", (), vals, (t.shape[0],), dtype, envless=True)
             raise UnsupportedTermError(
                 f"user term: a concrete tensor of shape {tuple(t.shape)} enters the expression (per-env state the "
                 "kernel does not hold: a captured buffer, a further entity, a user-level manager's state)")
@@ -494,10 +557,8 @@ class Tracer:
             dt = a.dtype_ if _RANK[a.dtype_] >= _RANK[b.dtype_] else b.dtype_
         else:
             dt = _promote(a, b)
-        shape = max((c.shape_, a.shape_, b.shape_), key=len)
-        for s in (c.shape_, a.shape_, b.shape_):
-            if s and s != shape:
-                raise UnsupportedTermError("user term: where() operands do not broadcast row by row")
+        shapes = {s for s in (c.shape_, a.shape_, b.shape_) if s}
+        shape = (shapes.pop() if len(shapes) == 1 else _broadcast([c, a, b], "where")) if shapes else ()
         if c.weak:
             raise UnsupportedTermError("user term: where() with a scalar condition")
         return self.add("where", (c._id, self.cast(a, dt)._id, self.cast(b, dt)._id), None, shape, dt)
@@ -660,7 +721,7 @@ class Tracer:
             for k in rest:
                 if k is None:
                     shape.append(1)
-                elif isinstance(k, slice):
+                elif isinstance(k, slice) or isinstance(_const_index(k), list):
                     shape.append(src.pop(0))
             shape += src
             return self._as_row(tuple(shape), out)
@@ -680,11 +741,20 @@ class Tracer:
             raise UnsupportedTermError("user term: too many indices")
         rest += [slice(None)] * (len(shape) - len(rest))
         spec, out_shape = [], []
+        rest = [_const_index(k) for k in rest]
+        if sum(isinstance(k, list) for k in rest) > 1:
+            raise UnsupportedTermError("user term: two advanced (list / tensor) indices in one indexing expression")
         for k, n in zip(rest, shape):
             if isinstance(k, Sym):
                 k._control("index")
+            if isinstance(k, list):  # a constant index list: a gather along the axis, order and duplicates kept
+                if any(not -n <= i < n for i in k):
+                    raise UnsupportedTermError(f"user term: index list {k} out of range for size {n}")
+                spec.append(("list",) + tuple(i % n for i in k))
+                out_shape.append(len(k))
+                continue
             if isinstance(k, bool) or not isinstance(k, (int, slice)):
-                raise UnsupportedTermError(f"user term: index {k!r} (ints and basic slices only)")
+                raise UnsupportedTermError(f"user term: index {k!r} (ints, basic slices and constant index lists only)")
             if isinstance(k, int):
                 if not -n <= k < n:
                     raise UnsupportedTermError(f"user term: index {k} out of range for size {n}")
@@ -766,8 +836,47 @@ class Tracer:
 class _EntityProxy:
     """Stands for the primary entity while a term is traced."""
 
-    def __init__(self, tr: Tracer, dofs_idx, n_dofs: int):
-        self._tr, self._dofs_idx, self._D = tr, dofs_idx, n_dofs
+    def __init__(self, tr: Tracer, dofs_idx, n_dofs: int, robot=None):
+        self._tr, self._dofs_idx, self._D, self._robot = tr, dofs_idx, n_dofs, robot
+
+    # -- links: the real link objects (their get_pos / get_vel are swapped for the trace) --------------
+    @property
+    def links(self):
+        return self._robot_or_refuse("links").links
+
+    def get_link(self, name=None, *args, **kwargs):
+        return self._robot_or_refuse("get_link").get_link(name, *args, **kwargs)
+
+    def get_links_pos(self, links_idx_local=None, envs_idx=None):
+        return self._links("pos", links_idx_local, envs_idx)
+
+    def get_links_vel(self, links_idx_local=None, envs_idx=None):
+        return self._links("vel", links_idx_local, envs_idx)
+
+    def _robot_or_refuse(self, what):
+        if self._robot is None:
+            raise UnsupportedTermError(f"user term: robot.{what} without a primary entity")
+        return self._robot
+
+    def _links(self, what, links_idx_local, envs_idx):
+        if envs_idx is not None:
+            raise UnsupportedTermError(f"user term: robot.get_links_{what}(envs_idx=...)")
+        if links_idx_local is None:
+            raise UnsupportedTermError(f"user term: robot.get_links_{what}() without links_idx_local (every link of "
+                                       "the entity; name the links the term reads)")
+        if isinstance(links_idx_local, range):
+            links_idx_local = list(links_idx_local)
+        ids = _const_index(links_idx_local)
+        if not isinstance(ids, list):
+            raise UnsupportedTermError(f"user term: robot.get_links_{what}(links_idx_local={links_idx_local!r}) (a "
+                                       "list, tuple, range or 1-D integer tensor of local link ids)")
+        n = len(self._robot_or_refuse(f"get_links_{what}").links)
+        if not ids or any(not 0 <= i < n for i in ids):
+            raise UnsupportedTermError(f"user term: robot.get_links_{what}: local link ids {ids} (the entity has {n})")
+        if len(set(ids)) > MAX_LINKS:
+            raise UnsupportedTermError(f"user term: robot.get_links_{what} of {len(set(ids))} links (at most "
+                                       f"{MAX_LINKS})")
+        return self._tr.source((f"link_{what}", tuple(ids)), (len(ids), 3), F32)
 
     def get_pos(self, envs_idx=None):
         return self._plain("pos", 3, envs_idx)
@@ -1121,11 +1230,15 @@ def _install_sources(fused, tr: Tracer, swap: _Swap, kind: str):
     env = fused.env
     robot = fused.primary_entity
     dofs_idx = fused.action.dofs_idx if fused.action is not None else None
-    proxy = _EntityProxy(tr, dofs_idx, fused.D)
+    proxy = _EntityProxy(tr, dofs_idx, fused.D, robot)
     if robot is not None:
         for attr, value in list(vars(env).items()):
             if value is robot:
                 swap.set(env, attr, proxy)
+        # the primary entity's link objects, also those a term captured at build time: (N, 3) sources
+        for link in getattr(robot, "links", ()):
+            for what in ("pos", "vel"):
+                swap.set(link, f"get_{what}", _link_getter(tr, what, int(link.idx_local)))
     if fused.entity_manager is not None:
         em = fused.entity_manager
         swap.set(em, "entity", proxy)
@@ -1157,6 +1270,38 @@ def _install_sources(fused, tr: Tracer, swap: _Swap, kind: str):
             swap.set_item(extras, key, tr.source((src,), (), BOOL))
         else:
             swap.set_item(extras, key, _Refused(f"extras['{key}'] inside a {kind} term"))
+
+
+def _link_getter(tr: Tracer, what: str, local: int):
+    def get(envs_idx=None):
+        if envs_idx is not None:
+            raise UnsupportedTermError(f"user term: link.get_{what}(envs_idx=...)")
+        return tr.source((f"link_{what}", (local,)), (3,), F32)
+    return get
+
+
+def link_union(progs) -> dict:
+    """{"pos" / "vel": local link ids in first-use order} read by the link sources of `progs` (and their
+    first-call programs)."""
+    out: dict = {}
+    for prog in progs:
+        for p in (prog, prog.first):
+            for n in (p.nodes if p is not None else ()):
+                if n.op == "src" and n.attr[0] in ("link_pos", "link_vel"):
+                    ids = out.setdefault(n.attr[0][5:], [])
+                    ids += [i for i in n.attr[1] if i not in ids]
+    return {k: out[k] for k in ("pos", "vel") if k in out}
+
+
+def place_links(progs, layout: dict):
+    """Write the table's link layout {"pos" / "vel": (slot, U)} into the link sources of `progs`: the attr
+    (kind, ids, slot, U) is part of the program's text, so of its identity and of the header."""
+    for prog in progs:
+        for p in (prog, prog.first):
+            for n in (p.nodes if p is not None else ()):
+                if n.op == "src" and n.attr[0] in ("link_pos", "link_vel"):
+                    slot, U = layout[n.attr[0][5:]]
+                    n.attr = (n.attr[0], n.attr[1], slot, tuple(U))
 
 
 class _Refused:
@@ -1258,6 +1403,14 @@ def _src_elems(key: tuple, shape: tuple, lines: list, v: str, glob: bool = False
         else:
             lines.append(f"const V3 {v}r = (c.plan.needs & {need}) ? c.{reg} : rotate({vec}, c.iw, c.iq);")
         return [f"{v}r.x", f"{v}r.y", f"{v}r.z"]
+    if name in ("link_pos", "link_vel"):
+        # a per-launch (N, |U|, 3) gather of the engine's link array, bound to a free GFB_B_USER_STATE slot
+        if len(key) != 4:
+            raise UnsupportedTermError(f"user term: source {key!r} has no link layout")
+        ids, slot, U = key[1], key[2], key[3]
+        lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[GFB_B_USER_STATE0 + {slot}]) + "
+                     f"(size_t)c.e * {len(U) * 3};")
+        return [f"{v}p[{U.index(i) * 3 + k}]" for i in ids for k in range(3)]
     if name == "episode_length":
         return ["c.ep_len"]
     if name == "max_episode_length":
@@ -1369,13 +1522,14 @@ def function_body(prog: Program, fname: str, glob: bool = False) -> str:
             exprs = [_unop(n.op, x, n.dtype) for x in elems[n.args[0]]]
         elif n.op == "where":
             c, a, b = (elems[j] for j in n.args)
-            exprs = [f"({c[k if len(c) > 1 else 0]} ? {a[k if len(a) > 1 else 0]} : {b[k if len(b) > 1 else 0]})"
-                     for k in range(size)]
+            ic, ia, ib = (_bidx(n.shape, prog.nodes[j].shape) for j in n.args)
+            exprs = [f"({c[ic[k]]} ? {a[ia[k]]} : {b[ib[k]]})" for k in range(size)]
         elif n.op == "index":
             src_shape = prog.nodes[n.args[0]].shape
             a = elems[n.args[0]]
             st = _strides(src_shape)
-            ranges = [[s] if isinstance(s, int) else list(range(s[0], s[1])) for s in n.attr]
+            ranges = [[s] if isinstance(s, int) else list(s[1:]) if s[0] == "list" else list(range(s[0], s[1]))
+                      for s in n.attr]
             exprs = []
             for combo in np.ndindex(*[len(r) for r in ranges]) if ranges else [()]:
                 flat = sum(ranges[d][combo[d]] * st[d] for d in range(len(ranges)))
@@ -1398,8 +1552,8 @@ def function_body(prog: Program, fname: str, glob: bool = False) -> str:
         else:
             a = elems[n.args[0]]
             b = elems[n.args[1]]
-            exprs = [_binop(n.op, a[k if len(a) > 1 else 0], b[k if len(b) > 1 else 0], prog.nodes[n.args[0]].dtype,
-                            n.attr) for k in range(size)]
+            ia, ib = (_bidx(n.shape, prog.nodes[j].shape) for j in n.args)
+            exprs = [_binop(n.op, a[ia[k]], b[ib[k]], prog.nodes[n.args[0]].dtype, n.attr) for k in range(size)]
         # every element is materialised once, in node order (torch's operation order)
         names = []
         for k, x in enumerate(exprs):

@@ -90,6 +90,10 @@ def asin_tilt_threshold(limit_angle_deg: float) -> float:
 from .managers.observation import UnsupportedTermError  # noqa: E402  (one class, importable from here too)
 
 
+class _LinkLimit(UnsupportedTermError):
+    """A term's link reads would take the table past the links of an array or the slots of the ABI."""
+
+
 class UserTermsDemoted(Exception):
     """Raised before a step's first post-physics launch when its lowered user terms became host callbacks."""
 
@@ -262,6 +266,8 @@ class FusedStep:
         self.external_rows: list[tuple[str, str, object]] = []  # (kind, name, config item)
         self.user_terms: dict = {}  # (kind, name) -> [Program, params live, params traced as constants]
         self.user_term_refusals: dict = {}  # (kind, name) -> why the term stays a host callback
+        # user-defined observation terms lowered below (_observation_columns)
+        self.user_obs: dict = {}  # (group, name) -> [Program, params it was traced with, first word, width]
         self._user_code = None
         self._lower_user = bool(getattr(env, "fuse_user_terms", False)) and self._can_specialise_user_terms()
         # class-style terms (ManagedEnvironment.fuse_stateful_terms): their per-env tensors are bound to the
@@ -270,7 +276,14 @@ class FusedStep:
         # (kind, name), for an observation term ("observation", name, group) -> {"inst", "attrs": {attr: (slot,
         # shape, dtype, lazy)}, "tensors", "constants"}
         self.stateful: dict = {}
-        self._state_refusal = None  # why a class-style observation term could not be traced again (demotes)
+        self._state_refusal = None  # why a lowered term could not be traced again after an edit (demotes)
+        # per-link arrays the lowered terms read ({"pos" / "vel": (GFB_B_USER_STATE slot, local link ids U)}):
+        # gathered once per launch that evaluates them, from the entity the layout was built for, and bound to a
+        # state slot no class-style term uses
+        self._link_layout: dict = {}
+        self._link_entity = self.primary_entity
+        self._link_phases = 0  # phases whose lowered terms read the arrays
+        self._link_placeholder = None  # bound to the slots of a launch that does not read them (never read)
         if self.reward is not None:
             for name, item in self.reward.cfg.items():
                 opcode = self._opcode_of(item.fn, "reward")
@@ -297,9 +310,9 @@ class FusedStep:
         self._has_command_override = False  # set by CommandManager.use_external_controller / use_gamepad
         # user-defined observation terms: one (N, W) array filled on the host; with
         # ManagedEnvironment.fuse_user_observations the ones that lower are evaluated in the kernel instead
-        self.user_obs: dict = {}  # (group, name) -> [Program, params it was traced with, first word, width]
         self._lower_obs = bool(getattr(env, "fuse_user_observations", False)) and self._can_specialise_user_terms()
         self._observation_columns()
+        self._layout_links()
         self._plan_launches()
         self._static_buffers()
 
@@ -344,6 +357,7 @@ class FusedStep:
             else:
                 prog, _ = expr.lower_term(self, "observation", name, item)
                 _check_width(prog, name, width)
+                self._check_links(("observation", name, g), prog)
         except Exception as e:  # noqa: BLE001 - whatever the function does on symbolic inputs, it stays a host column
             why = str(e) if isinstance(e, UnsupportedTermError) else f"{type(e).__name__} while tracing: {e}"
             self.user_term_refusals[("observation", name)] = why
@@ -377,6 +391,10 @@ class FusedStep:
             prog, _ = expr.lower_term(self, "observation", name, item)
             if prog.nodes[prog.out].shape != (entry[3],):
                 raise UnsupportedTermError(f"observation '{name}': its width changed with its params")
+            try:
+                self._check_links(("observation", name, g), prog)
+            except _LinkLimit as e:
+                return self._retrace_refused("observation", name, e, entry[0])
             entry[0], entry[1] = prog, dict(item.params or {})
             self._user_code = None
         return entry[0]
@@ -468,6 +486,7 @@ class FusedStep:
         self._state_refusal = None
         self._lazy_started = {}
         self._after_launch_lazy = set()
+        self._link_layout, self._link_phases, self._obs_reads_links = {}, 0, False
         self._observation_columns()
         self._set(K["GFB_B_OBS_EXT0"], self.ext_obs)
         self._set(K["GFB_B_OBS_EXT1"], None)
@@ -497,6 +516,7 @@ class FusedStep:
                 prog, live = self._trace_stateful(kind, name, item), False
             else:
                 prog, live = expr.lower_term(self, kind, name, item)
+                self._check_links((kind, name), prog)
         except Exception as e:  # noqa: BLE001 - whatever the function does on symbolic inputs, it stays a callback
             why = str(e) if isinstance(e, UnsupportedTermError) else f"{type(e).__name__} while tracing: {e}"
             self.user_term_refusals[(kind, name)] = why
@@ -520,11 +540,13 @@ class FusedStep:
         old = self.stateful.get(key)
         own = {a: b[0] for a, b in old["attrs"].items()} if old else {}
         taken = {slot for k, b in self.stateful.items() if k != key for slot in b["tensors"]}
+        taken |= {slot for slot, _ in self._link_layout.values()}
         prog = expr.trace_stateful(self, kind, name, item,
                                    expr.StateSlots(own, [s for s in range(expr.MAX_STATE_SLOTS)
                                                          if s not in taken and s not in own.values()]))
         if obs is not None:
             _check_width(prog, name, obs[1])
+        self._check_links(key, prog, {slot for slot, *_ in prog.bindings.values()})
         inst, tensors = item.fn, {}
         for attr, (slot, shape, dtype, lazy) in prog.bindings.items():
             tensors[slot] = (torch.zeros((self.N,) + tuple(shape), device=self.device, dtype=_TORCH_DTYPE[dtype])
@@ -547,6 +569,69 @@ class FusedStep:
             self._lazy_started[key] = False
         else:
             self._lazy_started.pop(key, None)
+        return prog
+
+    def _user_programs(self, skip=None) -> list:
+        """The Programs of the lowered terms (`skip`: a (kind, name) / (kind, name, group) key left out)."""
+        progs = [e[0] for k, e in self.user_terms.items() if k != skip]
+        return progs + [e[0] for (g, n), e in self.user_obs.items() if ("observation", n, g) != skip]
+
+    def _check_links(self, key, prog, state_slots=frozenset()):
+        """A term whose link reads would take the table past MAX_LINKS links an array, or past the 8
+        GFB_B_USER_STATE slots that per-link arrays share with class-style state, stays a callback."""
+        from . import expr
+
+        union = expr.link_union(self._user_programs(skip=key) + [prog])
+        if not union:
+            return None
+        for what, ids in union.items():
+            if len(ids) > expr.MAX_LINKS:
+                raise _LinkLimit(f"user term: the lowered terms would read {len(ids)} links with "
+                                           f"get_links_{what} (at most {expr.MAX_LINKS} an array)")
+        state = {slot for k, b in self.stateful.items() if k != key for slot in b["tensors"]} | set(state_slots)
+        if len(state) + len(union) > expr.MAX_STATE_SLOTS:
+            raise _LinkLimit(f"user term: {len(state)} state tensors and {len(union)} per-link arrays need "
+                                       f"more than the {expr.MAX_STATE_SLOTS} slots GFB_B_USER_STATE0..7")
+
+    def _layout_links(self):
+        """Give every per-link array the lowered terms read its slot and link list, and write that layout into
+        their programs (it is part of their identity).  After tracing the table, and after every re-trace."""
+        from . import expr
+
+        progs = self._user_programs()
+        union = expr.link_union(progs)
+        state = {slot for b in self.stateful.values() for slot in b["tensors"]}
+        old = self._link_layout
+        free = [s for s in reversed(range(expr.MAX_STATE_SLOTS)) if s not in state]
+        layout = {}
+        for what, ids in union.items():
+            prev = old.get(what)
+            slot = prev[0] if prev is not None and prev[0] in free else free[0]
+            free.remove(slot)
+            layout[what] = (slot, tuple(ids))
+        K = nat.K
+        for what, (slot, _) in old.items():
+            if slot not in {s for s, _ in layout.values()} and slot not in state:
+                self._set(K["GFB_B_USER_STATE0"] + slot, None)
+        expr.place_links(progs, layout)
+        reads = lambda prog: bool(expr.link_union([prog]))  # noqa: E731
+        self._link_phases = 0
+        for (kind, _), (prog, *_) in self.user_terms.items():
+            if reads(prog):
+                self._link_phases |= K["GFB_PHASE_REWARD" if kind == "reward" else "GFB_PHASE_TERMINATION"]
+        self._obs_reads_links = any(reads(prog) for prog, *_ in self.user_obs.values())
+        if self._obs_reads_links:
+            self._link_phases |= K["GFB_PHASE_OBSERVE"]
+        if layout and self._link_placeholder is None:
+            self._link_placeholder = torch.zeros(1, device=self.device)
+        if layout != old:
+            self._link_layout = layout
+            self._user_code = None
+
+    def _retrace_refused(self, kind: str, name: str, why, prog):
+        """A term traced again after an edit no longer fits the link arrays or the slots: the table keeps its
+        program (consistent with its layout and binary) until the step's first launch demotes the lowered terms."""
+        self._state_refusal = f"{kind} '{name}' traced again after an edit: {why}"
         return prog
 
     def _check_state(self) -> str | None:
@@ -590,6 +675,7 @@ class FusedStep:
         if self._user_code is None:
             from . import expr
 
+            self._layout_links()  # (a class-style observation term traced again since the last pack)
             rows = {"reward": {}, "termination": {}}
             for kind, terms in (("reward", self.reward_terms), ("termination", self.termination_terms)):
                 for row, (name, _, _) in enumerate(terms):
@@ -612,14 +698,22 @@ class FusedStep:
             # with the new instance's tensors bound
             if (item.fn is not bound["inst"] or dict(item.params or {}) != entry[2]
                     or expr.instance_constants(item.fn) != bound["constants"]):
-                entry[0], entry[2] = self._trace_stateful(kind, name, item), dict(item.params or {})
+                try:
+                    entry[0], entry[2] = self._trace_stateful(kind, name, item), dict(item.params or {})
+                except _LinkLimit as e:
+                    return self._retrace_refused(kind, name, e, entry[0])
                 self._user_code = None
             return entry[0]
         # traced with constant params and they changed, or a live param changed between int and float (its
         # kernel type, int32 or fp32, was fixed by the trace)
         changed = entry[2] is not None and dict(item.params or {}) != entry[2]
         if changed or expr.param_kinds(item.params) != entry[3]:
-            entry[0], live = expr.lower_term(self, kind, name, item)
+            prog, live = expr.lower_term(self, kind, name, item)
+            try:
+                self._check_links((kind, name), prog)
+            except _LinkLimit as e:
+                return self._retrace_refused(kind, name, e, entry[0])
+            entry[0] = prog
             entry[2] = None if live else dict(item.params or {})
             entry[3] = expr.param_kinds(item.params)
             self._user_code = None
@@ -872,6 +966,14 @@ class FusedStep:
         if fp == self._fingerprint:
             return
         self._spec_checked = set()  # the structure may have changed with the values
+        if self._link_layout or any(k[0] in ("link_pos", "link_vel") for p in self._user_programs()
+                                    for k in p.sources()):
+            # (a re-trace may change the links the table reads: every term's identity follows the layout)
+            for kind, name in list(self.user_terms):
+                self._user_program(kind, name, (self.reward.cfg if kind == "reward" else self.termination.term_cfg)[name])
+            for g, name in list(self.user_obs):
+                self._user_obs_program(g, name, self.observations[g].cfg[name])
+            self._layout_links()
         env, K, P = self.env, nat.K, self.program.head
         C.memset(C.byref(self.program), 0, C.sizeof(self.program))
         P.num_envs, P.num_dofs = self.N, self.D
@@ -1167,6 +1269,24 @@ class FusedStep:
         if self._fixed_command_parts:
             s(K["GFB_B_FIXED_COMMAND"], self._resolve_fixed_command(), f32)
 
+    def _bind_links(self, gather: bool):
+        """
+        The per-link arrays of the lowered terms, bound right before a launch (after any re-pack, so with the
+        layout the launch's table was generated for).  `gather`: the launch evaluates lowered terms that read
+        them -- one getter call per array, always on the entity the layout was built for (a one-term evaluation
+        points `primary_entity` at another entity), kept alive until the next launch's pointers are bound.  A
+        launch that reads none binds a placeholder that nothing reads: the library refuses a specialised launch
+        with a slot of its table unbound.
+        """
+        K = nat.K
+        for what, (slot, ids) in self._link_layout.items():
+            if gather:
+                entity = self._link_entity
+                getter = entity.get_links_pos if what == "pos" else entity.get_links_vel
+                self._set(K["GFB_B_USER_STATE0"] + slot, getter(links_idx_local=list(ids)), torch.float32, keep=True)
+            else:
+                self._set(K["GFB_B_USER_STATE0"] + slot, self._link_placeholder)
+
     def _resolve_fixed_command(self) -> torch.Tensor:
         """(N,3) tensor [cmd_x, cmd_y, cmd_yaw] for tracking terms configured with fixed tensors."""
         parts = self._fixed_command_parts
@@ -1296,6 +1416,7 @@ class FusedStep:
         """Entity phase alone (EntityManager.build() caches the pose before the first reset)."""
         self._engine_buffers()
         self._set_program()
+        self._bind_links(False)
         self.handle.check(
             self.lib.gfb_post_physics(self.handle.ptr, C.byref(self.buffers), nat.K["GFB_PHASE_ENTITY"], self._stream()),
             "gfb_post_physics(entity)",
@@ -1352,6 +1473,7 @@ class FusedStep:
         self._obs_buffers()
         self._injection_buffers()
         self._set_program(force=True)
+        self._bind_links(False)
 
     def _maybe_specialise(self, phases: int):
         """Attach the specialised kernel for the current table structure (once per structure)."""
@@ -1389,6 +1511,7 @@ class FusedStep:
             self._contact_dims,
             self._obs_user_id,
             tuple(self.user_terms[k][0].digest() for k in self.stateful if k in self.user_terms),
+            tuple(sorted(self._link_layout.items())),
         )
 
     def spec_stats(self) -> dict:
@@ -1460,7 +1583,7 @@ class FusedStep:
         phases &= self._phase_mask
         first = self.first_launch_of_step
         self.first_launch_of_step = False
-        if first and self.stateful:
+        if first and (self.stateful or self._state_refusal is not None):
             why = self._check_state()
             if why is not None:
                 self._demote_user_terms(why)
@@ -1483,6 +1606,8 @@ class FusedStep:
             if not started and phases & (self._PHASE_REWARD if key[0] == "reward" else nat.K["GFB_PHASE_TERMINATION"]):
                 if key[0] == "termination" or self.reward.cfg[key[1]].weight != 0:
                     self._after_launch_lazy.add(key)
+        if self._link_layout:
+            self._bind_links(bool(phases & self._link_phases))
         stream = self._stream()
         rc = self.lib.gfb_post_physics(self._h, self._buffers_ref, phases, stream)
         if rc:
@@ -1533,6 +1658,8 @@ class FusedStep:
         if self.user_obs:  # the lowered observation terms' reset path is a kernel of the table's specialised library
             K = nat.K
             self._maybe_specialise(K["GFB_PHASE_OBSERVE"] if self.split_mode else self.step_phases & self._phase_mask)
+        if self._link_layout:
+            self._bind_links(self._obs_reads_links)  # (from post-reset engine state)
         rc = self.lib.gfb_observe(self._h, self._buffers_ref, idx.data_ptr() if idx is not None else None, n, self._stream())
         if rc == nat.K["GFB_ERR_UNSUPPORTED"] and self.user_obs:
             # no specialised library for the lowered terms: they become host columns (split execution from now on)

@@ -116,7 +116,8 @@ typedef enum {
   GFB_B_EXT_VALUES,
   GFB_B_DONES,        /* (N,) bool written: terminated | truncated (what wrappers/rsl_rl.py:57 computes) */
   /* per-env state of class-style user terms lowered into the specialised kernel: (N, *s) fp32 / int32 / bool,
-     read and updated in place (ABI v14) */
+     read and updated in place (ABI v14); a free slot may instead hold a per-launch (N, |U|, 3) fp32 gather of
+     the engine's link positions / velocities that lowered terms read (read only) */
   GFB_B_USER_STATE0, GFB_B_USER_STATE1, GFB_B_USER_STATE2, GFB_B_USER_STATE3,
   GFB_B_USER_STATE4, GFB_B_USER_STATE5, GFB_B_USER_STATE6, GFB_B_USER_STATE7,
   GFB_B_COUNT
