@@ -549,6 +549,12 @@ class Tracer:
             return self.add(op, (ca._id, cb._id), None, shape, BOOL)
         return self.add(op, (ca._id, cb._id), None, shape, dt)
 
+    def nan_dropping(self, op: str, a, b) -> Sym:
+        """fmaxf / fminf ("fmax" / "fmin") of fp32 values: a NaN operand gives the other one.  Internal: the
+        restated stock terms use them where their kernel case does."""
+        a, b = self.cast(self.lift(a), F32), self.cast(self.lift(b), F32)
+        return self.add(op, (a._id, b._id), None, _bshape(a, b, op), F32)
+
     def where(self, c, a, b) -> Sym:
         c, a, b = self.lift(c), self.lift(a), self.lift(b)
         if c.dtype_ != BOOL:
@@ -976,6 +982,265 @@ class ExprMode:
         if isinstance(key, str) and key.endswith("_uncached"):
             raise UnsupportedTermError("user term: a body-frame term without an entity_manager")
         return compute()
+
+    def stock_call(self, kind: str, fn, params: dict) -> Sym:
+        """A stock reward / termination descriptor called inside the traced term (ManagedEnvironment.fuse_stock_calls):
+        the unweighted term as IR, `params` normalised as FusedStep.pack normalises a table row."""
+        name = getattr(fn, "__name__", type(fn).__name__)
+        what = f"user term: stock term {name}"
+        if self.tr.kind == "observation":
+            raise UnsupportedTermError(f"{what} inside an observation term (stock calls are inlined in rewards and "
+                                       "terminations only)")
+        restate = _STOCK.get((kind, fn.gfb_opcode))
+        if restate is None:
+            raise UnsupportedTermError(f"{what}: keeps per-term state in the kernel and is not inlined")
+        return restate(_Stock(self, what), params)
+
+
+class _Stock:
+    """What the restatement of one stock term reads: its sources, its managers (checked as FusedStep.pack checks
+    a table row's) and the row's fp32 constants."""
+
+    def __init__(self, mode: ExprMode, what: str):
+        self.tr, self.fused, self.what = mode.tr, mode.fused, what
+
+    def refuse(self, why: str):
+        raise UnsupportedTermError(f"{self.what}: {why}")
+
+    def src(self, key: tuple, shape: tuple = (), dtype: str = F32) -> Sym:
+        return self.tr.source(key, shape, dtype)
+
+    def entity(self, p: dict):
+        """FusedStep._entity_ok, with the trace's stand-in for the primary entity."""
+        fused, em = self.fused, p.get("entity_manager")
+        if em is not None:
+            if em is not fused.entity_manager:
+                self.refuse("the entity_manager is a further EntityManager (the kernel holds the first one's pose)")
+            return
+        attr = p.get("entity_attr", "robot")
+        if not isinstance(getattr(fused.env, attr, None), _EntityProxy):
+            self.refuse(f"entity_attr '{attr}' is not the fused step's entity")
+
+    def command(self, mgr) -> Sym:
+        fused = self.fused
+        k = next((k for k, m in enumerate(fused.commands) if m is mgr), None)
+        if k is None:
+            self.refuse("its command manager is not registered with this environment")
+        if mgr in fused.python_commands or mgr._external_controller is not None:
+            self.refuse("its command manager is a user-level or externally controlled one")
+        return self.src(("command", k), (int(mgr._command.shape[1]),))
+
+    def contact_norm(self, mgr) -> tuple[int, Sym]:
+        """(index, (N, L) force norms of the tracked links): the kernel's st_cnorm."""
+        m = next((m for m, c in enumerate(self.fused.contacts) if c is mgr), None)
+        if m is None:
+            self.refuse("its contact manager is not registered with this environment")
+        return m, self.src(("contacts", m), (int(mgr._link_ids.shape[0]), 3)).norm(dim=-1)
+
+    def scalar(self, v, what: str) -> Sym:
+        """A row's fp32 p[k]: a live param of the user term stays live, a Python or one-element value is a constant."""
+        if isinstance(v, Sym):
+            if not v.weak:
+                self.refuse(f"a per-env {what}")
+            return v
+        if torch.is_tensor(v) or isinstance(v, np.ndarray):
+            t = torch.as_tensor(v)
+            if t.numel() != 1:
+                self.refuse(f"a {what} tensor of shape {tuple(t.shape)} (a per-env value the kernel does not hold)")
+            v = t.item()
+        if isinstance(v, bool) or not isinstance(v, (int, float, np.generic)):
+            self.refuse(f"{what} {v!r}")
+        return self.tr.lift(_f32(v))
+
+    def dof_deviation(self) -> Sym:
+        """sum_d |q_d - default_d| (P.default_dof_pos folded in as a constant vector)."""
+        fused = self.fused
+        if fused.D == 0:
+            self.refuse("no action manager")
+        default = tuple(_f32(x) for x in fused.action.kernel_params()["default"].detach().cpu().tolist())
+        q = self.src(("dof_pos",), (fused.D,))
+        return (q - self.tr.add("constvec", (), default, (fused.D,), F32, envless=True)).abs().sum(dim=1)
+
+    def episode_length(self) -> Sym:
+        return self.src(("episode_length",), (), I32)
+
+    def terminated(self) -> Sym:
+        if self.tr.kind != "reward":
+            self.refuse("reads extras['terminations'], which a termination term does not see")
+        return self.src(("terminated",), (), BOOL)
+
+
+# The stock terms as IR, op for op as their cases in post_kernel.cuh (same operands, same order, the same
+# fp32 helpers), so an inlined call has the bits of the stock row evaluated in the same launch.
+def _r_base_height(s: _Stock, p):
+    s.entity(p)
+    off = 0.0
+    tm = p["terrain_manager"]
+    if tm is not None:
+        if tm.height_field is not None:
+            s.refuse("a height-field terrain")
+        off = float(tm._origin[2])
+    if p["height_command"] is not None:
+        target = s.command(p["height_command"])[:, 0]
+    else:
+        target = s.scalar(p["target_height"], "target_height")
+    z = s.src(("pos",), (3,))[:, 2]
+    return ((z - off) - target).square()
+
+
+def _r_action_rate(s: _Stock, p):
+    # the sum the action kernel wrote for this step (GFB_B_ACTION_RATE): the stock row's value by construction
+    if s.tr.kind != "reward":
+        s.refuse("reads the action-rate sum, which only the reward phase reads")
+    return s.src(("action_rate",))
+
+
+def _r_stand_still(s: _Stock, p):
+    if p["vel_cmd_manager"] is None:
+        s.refuse("no vel_cmd_manager")
+    c = s.command(p["vel_cmd_manager"])
+    return s.dof_deviation() * (c[:, :2].norm(dim=1) < s.scalar(p["command_threshold"], "command_threshold")).float()
+
+
+def _r_body_sq(key: str, dims: tuple):
+    def restate(s: _Stock, p):
+        s.entity(p)
+        v = s.src((key,), (3,))
+        out = v[:, dims[0]].square()
+        return out + v[:, dims[1]].square() if len(dims) > 1 else out
+    return restate
+
+
+def _fixed_command(s: _Stock, value, lin: bool) -> list:
+    """A command tensor of at most MAX_CONST_VEC elements that is the same for every env: its x, y (lin) or its
+    yaw rate, folded in as constants."""
+    if isinstance(value, Sym):
+        s.refuse("a per-env command")
+    t = torch.as_tensor(value, dtype=torch.float32).detach().cpu()
+    if t.numel() > MAX_CONST_VEC:
+        s.refuse(f"a command tensor of shape {tuple(t.shape)} (a per-env command the kernel does not hold)")
+    try:
+        t = torch.broadcast_to(t, (1, 2) if lin else (1,)).reshape(-1)
+    except RuntimeError:
+        s.refuse(f"a command tensor of shape {tuple(t.shape)}")
+    return [s.tr.lift(_f32(x)) for x in t.tolist()]
+
+
+def _r_track(lin: bool):
+    def restate(s: _Stock, p):
+        s.entity(p)
+        if p["vel_cmd_manager"] is not None:
+            c = s.command(p["vel_cmd_manager"])
+            cmd = [c[:, 0], c[:, 1]] if lin else [c[:, 2]]
+        else:
+            cmd = _fixed_command(s, p["command"] if lin else p["commanded_ang_vel"], lin)
+        if lin:
+            v = s.src(("lin_vel_b",), (3,))
+            err = (cmd[0] - v[:, 0]).square() + (cmd[1] - v[:, 1]).square()
+        else:
+            err = (cmd[0] - s.src(("ang_vel_b",), (3,))[:, 2]).square()
+        return (-err / s.scalar(p["sensitivity"], "sensitivity")).exp()
+    return restate
+
+
+def _r_feet_air_time(s: _Stock, p):
+    mgr = p["contact_manager"]
+    m, _ = s.contact_norm(mgr)
+    if not mgr._track_air_time:
+        s.refuse("its contact manager does not track air time")
+    L = int(mgr._link_ids.shape[0])
+    last_air, cur_contact = s.src(("air", m, 0), (L,)), s.src(("air", m, 3), (L,))
+    made = (cur_contact > 0.0) & (cur_contact < _f32(s.fused.env.dt + 1.0e-8))  # has_made_contact(env.dt)
+    a = (last_air - s.scalar(p["time_threshold"], "time_threshold")) * made.float()
+    if p["time_threshold_max"] is not None:
+        span = p["time_threshold_max"] - p["time_threshold"]  # (a live param here is traced as a constant)
+        a = s.tr.nan_dropping("fmin", a, s.scalar(span, "time_threshold_max"))
+    v = a.sum(dim=1)
+    if p["vel_cmd_manager"] is not None:
+        c = s.command(p["vel_cmd_manager"])
+        v = v * (c[:, :2].norm(dim=1) > 0.1).float()
+    return v
+
+
+def _r_feet_slide(s: _Stock, p):
+    mgr = p["contact_manager"]
+    _, cn = s.contact_norm(mgr)
+    s.entity({"entity_attr": p["entity_attr"]})
+    ids = [int(i) for i in mgr.local_link_ids.tolist()]
+    speed = _EntityProxy(s.tr, None, 0, s.fused.primary_entity).get_links_vel(links_idx_local=ids).norm(dim=-1)
+    return (speed * (cn > 1.0).float()).sum(dim=1)
+
+
+def _t_bad_orientation(s: _Stock, p):
+    s.entity(p)
+    threshold = s.fused._tilt_threshold(p["limit_angle"])  # (a live limit_angle: traced as a constant)
+    g = s.src(("gravity_b",), (3,))
+    tilt = g[:, :2].norm(dim=1)
+    after_grace = ~(s.episode_length() <= int(p["grace_steps"]))
+    return after_grace & (tilt == tilt) & (s.tr.nan_dropping("fmin", tilt, 0.99) >= s.scalar(threshold, "limit_angle"))
+
+
+def _t_base_height_min(s: _Stock, p):
+    s.entity(p)
+    return s.src(("pos",), (3,))[:, 2] < s.scalar(p["minimum_height"], "minimum_height")
+
+
+def _t_out_of_bounds(s: _Stock, p):
+    s.entity(p)
+    if p["terrain_manager"] is None:
+        s.refuse("no terrain_manager")
+    x_min, x_max, y_min, y_max = p["terrain_manager"].get_bounds(p["subterrain"])
+    margin = p["border_margin"]
+    lo_x, hi_x = s.scalar(x_min + margin, "bound"), s.scalar(x_max - margin, "bound")
+    lo_y, hi_y = s.scalar(y_min + margin, "bound"), s.scalar(y_max - margin, "bound")
+    pos = s.src(("pos",), (3,))
+    x, y = pos[:, 0], pos[:, 1]
+    return (x < lo_x) | (x > hi_x) | (y < lo_y) | (y > hi_y)
+
+
+def _has_contact(s: _Stock, p):
+    _, cn = s.contact_norm(p["contact_manager"])
+    return (cn > s.scalar(p["threshold"], "threshold")).sum(dim=1) >= int(p["min_contacts"])
+
+
+def _contact_force_any(s: _Stock, p):
+    _, cn = s.contact_norm(p["contact_manager"])
+    return (cn > s.scalar(p["threshold"], "threshold")).any(dim=1)
+
+
+def _t_timeout(s: _Stock, p):
+    ep = s.episode_length()
+    if not s.fused.env._base_max_episode_length:
+        return s.tr.full(ep, False, torch.bool)
+    return ep > s.src(("max_episode_length",), (), I32)
+
+
+_STOCK = {
+    ("reward", "GFB_R_IS_ALIVE"): lambda s, p: (~s.terminated()).float(),
+    ("reward", "GFB_R_TERMINATED"): lambda s, p: s.terminated().float(),
+    ("reward", "GFB_R_BASE_HEIGHT"): _r_base_height,
+    ("reward", "GFB_R_DOF_SIMILAR"): lambda s, p: s.dof_deviation(),
+    ("reward", "GFB_R_STAND_STILL"): _r_stand_still,
+    ("reward", "GFB_R_LIN_VEL_Z"): _r_body_sq("lin_vel_b", (2,)),
+    ("reward", "GFB_R_ANG_VEL_XY"): _r_body_sq("ang_vel_b", (0, 1)),
+    ("reward", "GFB_R_FLAT_ORIENTATION"): _r_body_sq("gravity_b", (0, 1)),
+    ("reward", "GFB_R_ACTION_RATE"): _r_action_rate,
+    ("reward", "GFB_R_TRACK_LIN_VEL"): _r_track(True),
+    ("reward", "GFB_R_TRACK_ANG_VEL"): _r_track(False),
+    ("reward", "GFB_R_HAS_CONTACT"): lambda s, p: _has_contact(s, p).float(),
+    ("reward", "GFB_R_CONTACT_FORCE"): lambda s, p: s.tr.nan_dropping(
+        "fmax", s.contact_norm(p["contact_manager"])[1] - s.scalar(p["threshold"], "threshold"), 0.0).sum(dim=1),
+    ("reward", "GFB_R_FEET_AIR_TIME"): _r_feet_air_time,
+    ("reward", "GFB_R_FEET_SLIDE"): _r_feet_slide,
+    ("termination", "GFB_T_TIMEOUT"): _t_timeout,
+    ("termination", "GFB_T_BAD_ORIENTATION"): _t_bad_orientation,
+    ("termination", "GFB_T_BASE_HEIGHT_MIN"): _t_base_height_min,
+    ("termination", "GFB_T_OUT_OF_BOUNDS"): _t_out_of_bounds,
+    ("termination", "GFB_T_HAS_CONTACT"): _has_contact,
+    ("termination", "GFB_T_CONTACT_FORCE"): _contact_force_any,
+    ("termination", "GFB_T_CONTACT_FORCE_GRACE"): lambda s, p: (
+        _contact_force_any(s, p) & ~(s.episode_length() <= int(p["grace_steps"]))),
+}
 
 
 def param_kinds(params) -> tuple:
@@ -1411,6 +1676,8 @@ def _src_elems(key: tuple, shape: tuple, lines: list, v: str, glob: bool = False
         lines.append(f"const float* {v}p = reinterpret_cast<const float*>(c.b.buf[GFB_B_USER_STATE0 + {slot}]) + "
                      f"(size_t)c.e * {len(U) * 3};")
         return [f"{v}p[{U.index(i) * 3 + k}]" for i in ids for k in range(3)]
+    if name == "action_rate":  # rewards only: the action kernel's sum for this step, as the stock row reads it
+        return ["reinterpret_cast<const float*>(c.b.buf[GFB_B_ACTION_RATE])[c.e]"]
     if name == "episode_length":
         return ["c.ep_len"]
     if name == "max_episode_length":
@@ -1439,6 +1706,8 @@ def _binop(op, a, b, dtype, attr=None):
         return arith[op]
     if op == "mod":
         return f"gfb_user_mod({a}, {b})"
+    if op in ("fmax", "fmin"):
+        return f"{op}f({a}, {b})"
     if op in ("clamp_lo", "clamp_hi") and dtype == F32:
         return f"gfb_user_{op}{'_scalar' if attr == 'scalar' else ''}({a}, {b})"
     if op in ("minimum", "clamp_hi"):

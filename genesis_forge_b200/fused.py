@@ -273,6 +273,9 @@ class FusedStep:
         # class-style terms (ManagedEnvironment.fuse_stateful_terms): their per-env tensors are bound to the
         # GFB_B_USER_STATE slots and updated in place by the kernel
         self._lower_stateful = bool(getattr(env, "fuse_stateful_terms", False)) and self._can_specialise_user_terms()
+        # stock reward / termination calls inside the terms lowered under any of the switches above
+        # (ManagedEnvironment.fuse_stock_calls): inlined as IR (expr.ExprMode.stock_call) instead of refused
+        self._lower_stock_calls = bool(getattr(env, "fuse_stock_calls", False))
         # (kind, name), for an observation term ("observation", name, group) -> {"inst", "attrs": {attr: (slot,
         # shape, dtype, lazy)}, "tensors", "constants"}
         self.stateful: dict = {}
@@ -1732,10 +1735,17 @@ class FusedStep:
         unweighted term, as in the reference (reward_manager.py:185, termination_manager.py:168);
         terms given an `entity_manager` use the base pose cached by the last step, the others the
         entity's current pose; contact terms read the last step's net forces.
+
+        While a user term is traced (ExprMode), the call is refused -- the term stays a host callback -- unless
+        ManagedEnvironment.fuse_stock_calls is set: then the term's arithmetic is returned as IR
+        (`ExprMode.stock_call`), evaluated in the specialised kernel with the bits of the stock row of the same
+        launch, and this path does not launch anything during lowered steps.
         """
         from .expr import ExprMode
 
         if isinstance(self.env._tracing, ExprMode):
+            if self._lower_stock_calls:
+                return self.env._tracing.stock_call(kind, fn, params)
             raise UnsupportedTermError(f"user term: a direct call of the stock term {fn.__name__} is not inlined")
         if self.dry_run:
             raise nat.NativeLibraryError("direct evaluation of mdp terms needs a CUDA device (dry-run handle)")

@@ -56,6 +56,11 @@ class ManagedEnvironment(GenesisEnv):
     # GFB_FUSE_STATEFUL_TERMS=1 in the environment -- the ones that lower are evaluated by the specialised
     # kernel, which updates the instance's state tensors in place (FusedStep.user_term_refusals says why not).
     fuse_stateful_terms = os.environ.get("GFB_FUSE_STATEFUL_TERMS", "0") == "1"
+    # A stock reward / termination term called inside a user term (`rewards.lin_vel_z_l2(env, ...) * gate`) stops
+    # the trace of that term: it stays a host callback and the call is a launch of its own.  With this set to
+    # True -- or GFB_FUSE_STOCK_CALLS=1 in the environment -- the call is inlined into the term lowered under any
+    # of the switches above, with the bits of the stock term evaluated in the same launch (DESIGN.md §1).
+    fuse_stock_calls = os.environ.get("GFB_FUSE_STOCK_CALLS", "0") == "1"
 
     def __init__(
         self,

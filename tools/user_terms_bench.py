@@ -8,14 +8,16 @@ of the lowered observation terms.  `--workload stateful_terms` compares workload
 (class-style terms with per-env state) as callbacks and lowered (fuse_stateful_terms), and
 `--workload stateful_observations` workload A of configs/stateful_observations.py (class-style observation
 terms: host columns against lowered, fuse_stateful_terms), and `--workload link_terms` configs/link_terms.py (user
-terms that read per-link state: callbacks / host columns against lowered, every lowering switch on).  The two modes are built side by side and
+terms that read per-link state: callbacks / host columns against lowered, every lowering switch on), and
+`--workload stock_calls` both workloads of configs/stock_calls.py (user terms that call stock mdp terms: callbacks
+against lowered with fuse_user_terms, fuse_stateful_terms and fuse_stock_calls on).  The two modes are built side by side and
 timed alternately in one process (CUDA events around `steps` steps, in-kernel Philox draws as bench.py
 runs them, on bench.py's pool of pre-generated state sets); the post-physics kernel's device time comes
 from the library's own event brackets.  The outputs of one more step of both modes (same states, same
 actions, same draws) are compared.
 
     python tools/user_terms_bench.py [--workload user_terms|user_observations|stateful_terms|stateful_observations|
-                                                 link_terms]
+                                                 link_terms|stock_calls]
                                      [--sizes 65536 1048576]
                                      [--steps 50] [--warmup 10] [--rounds 3]
 """
@@ -47,18 +49,22 @@ def gpu_info() -> dict:
 
 def make_env(n: int, mode: str, dev, workload: str = "user_terms"):
     import genesis_forge_b200 as gfb
-    from configs import link_terms, specs, stateful_observations, stateful_terms, user_observations, user_terms
+    from configs import (link_terms, specs, stateful_observations, stateful_terms, stock_calls, user_observations,
+                         user_terms)
     from configs.env_builder import build_env, dropin_namespace
     from genesis_forge_b200.managed_env import ManagedEnvironment
 
     obs = workload == "user_observations"
     stateful = workload in ("stateful_terms", "stateful_observations")
     links = workload == "link_terms"
-    ManagedEnvironment.fuse_user_terms = mode == "fused" and (links or not (obs or stateful))
+    calls = workload.startswith("stock_calls")
+    ManagedEnvironment.fuse_user_terms = mode == "fused" and (links or calls or not (obs or stateful))
     ManagedEnvironment.fuse_user_observations = mode == "fused" and (obs or links)
-    ManagedEnvironment.fuse_stateful_terms = mode == "fused" and (stateful or links)
+    ManagedEnvironment.fuse_stateful_terms = mode == "fused" and (stateful or links or calls)
+    ManagedEnvironment.fuse_stock_calls = mode == "fused" and calls
     gfb.set_device(dev)
     spec = specs.contacts() if mode == "stock" else (link_terms.link_terms() if links
+                                                     else getattr(stock_calls, workload)() if calls
                                                      else user_observations.user_observations() if obs
                                                      else stateful_terms.stateful_terms() if workload == "stateful_terms"
                                                      else stateful_observations.stateful_observations() if stateful
@@ -102,13 +108,15 @@ def main():
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--workload", choices=["user_terms", "user_observations", "stateful_terms",
-                                                       "stateful_observations", "link_terms"], default="user_terms")
+                                                       "stateful_observations", "link_terms", "stock_calls"],
+                    default="user_terms")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     print(json.dumps({"gpu": gpu_info()}), flush=True)
-    for n in args.sizes:
-        modes = ("split", "fused") + (("stock",) if args.workload == "user_observations" else ())
-        envs = {mode: make_env(n, mode, dev, args.workload) for mode in modes}
+    workloads = ["stock_calls_a", "stock_calls_b"] if args.workload == "stock_calls" else [args.workload]
+    for n, workload in ((n, w) for n in args.sizes for w in workloads):
+        modes = ("split", "fused") + (("stock",) if workload == "user_observations" else ())
+        envs = {mode: make_env(n, mode, dev, workload) for mode in modes}
         print(f"# N={n}: both environments built", flush=True)
         assert envs["split"]._fused.split_mode and not envs["fused"]._fused.split_mode
         gen = torch.Generator(device=dev).manual_seed(5)
@@ -130,7 +138,7 @@ def main():
             "truncated_equal": bool(torch.equal(a[3], b[3])),
             "obs_max_abs": float((a[0] - b[0]).abs().max()),
         }
-        result = {"workload": args.workload, "num_envs": n, "steps": args.steps, "rounds": args.rounds,
+        result = {"workload": workload, "num_envs": n, "steps": args.steps, "rounds": args.rounds,
                   "compare": diff}
         for mode, r in rows.items():
             ms = sorted(x[0] for x in r)[len(r) // 2]
@@ -138,7 +146,8 @@ def main():
             result[mode] = {"ms_per_step_median": round(ms, 4), "env_steps_per_s": round(n / ms * 1e3),
                             "post_kernel_ms_per_step_median": round(post, 4), "post_launches_per_step": r[0][2],
                             "ms_per_step_all": [round(x[0], 4) for x in r]}
-            if args.workload in ("user_observations", "stateful_observations", "link_terms") and mode == "fused":
+            if workload in ("user_observations", "stateful_observations", "link_terms", "stock_calls_a",
+                            "stock_calls_b") and mode == "fused":
                 result[mode]["user_observe_kernel_us_median"] = round(sorted(x[3] for x in r)[len(r) // 2], 2)
                 result[mode]["spec_stats"] = envs[mode]._fused.spec_stats()
         print(json.dumps(result), flush=True)
